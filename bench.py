@@ -58,7 +58,35 @@ def parse():
     ap.add_argument("--placeholder-supports", action="store_true", help="N(0,1) edge features instead of SpectralDesign supports")
     ap.add_argument("--no-cuda-graph", action="store_true", help="enqueue every step's ~120 launches from the host instead of replaying "
                                                                   "the captured step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the loss of the last timed step, the gradients "
+                                                          "it computed and the parameters it left as DIR/<name>.npy (float32), to "
+                                                          "compare two builds on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "spectconv_sweep"):
+        ap.error("--dump-outputs applies to the training workloads of --impl b200")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, model, loss):
+    """What a caller of the timed training step holds after its last step: the loss (loss.npy), every parameter's gradient
+    (grad.<name>.npy) and every parameter after the Adam update (param.<name>.npy)."""
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        if p.grad is not None:
+            arrays["grad." + name] = p.grad
+        arrays["param." + name] = p
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -608,6 +636,8 @@ def main():
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, loss_t)       # before the steps below train the same model further
     final_loss = float(loss_t.item())
     sampler.stop_flag = True
     sampler.join()

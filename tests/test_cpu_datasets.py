@@ -49,10 +49,10 @@ def test_read_graph6_known_encodings_and_edge_cases():
         read_graph6(b"A\x1f")                                                        # byte below the 63 offset
 
 
-def test_read_exp_pickle_without_torch_geometric():
-    """A pickle of objects whose class lives in `torch_geometric.data.data` is read with the class mapped to a plain record:
-    torch_geometric is never imported (it is not installable here, and the GPU box has no copy either)."""
-    from gnn_matlang_b200.datasets import read_exp_pickle
+def _pyg_pickle(graphs):
+    """Pickle of a list of PyG 1.x ``Data`` objects (the layout of the EXP dataset's GRAPHSAT.pkl) holding the tensors of
+    ``graphs`` = [(x, edge_index, y), ...], made without torch_geometric: a class is registered under the module path PyG
+    pickles ``Data`` with, and unregistered again."""
     assert not any(m.startswith("torch_geometric") for m in sys.modules)
     names = ["torch_geometric", "torch_geometric.data", "torch_geometric.data.data"]
     mods = {n: types.ModuleType(n) for n in names}
@@ -65,37 +65,46 @@ def test_read_exp_pickle_without_torch_geometric():
     sys.modules.update(mods)
     try:
         objs = []
-        for i, (n, e) in enumerate([(4, 6), (1, 0), (7, 10)]):
+        for x, ei, y in graphs:
             d = Data()
-            d.x = torch.arange(n).reshape(n, 1) % 2
-            d.edge_index = torch.randint(0, n, (2, e), generator=torch.Generator().manual_seed(i))
-            d.y = torch.tensor([i % 2])
+            d.x, d.edge_index, d.edge_attr, d.y, d.pos, d.normal, d.face = x, ei, None, y, None, None, None
             objs.append(d)
-        blob = pickle.dumps(objs)
+        return pickle.dumps(objs)
     finally:
         for n in names:
             sys.modules.pop(n, None)
-    out = read_exp_pickle(blob)
+
+
+def test_read_exp_pickle_without_torch_geometric():
+    """A pickle of objects whose class lives in `torch_geometric.data.data` is read with the class mapped to a plain record:
+    torch_geometric is never imported (the product does not depend on it)."""
+    from gnn_matlang_b200.datasets import read_exp_pickle
+    graphs = []
+    for i, (n, e) in enumerate([(4, 6), (1, 0), (7, 10)]):
+        graphs.append((torch.arange(n).reshape(n, 1) % 2, torch.randint(0, n, (2, e), generator=torch.Generator().manual_seed(i)),
+                       torch.tensor([i % 2])))
+    out = read_exp_pickle(_pyg_pickle(graphs))
     assert not any(m.startswith("torch_geometric") for m in sys.modules)
     assert len(out) == 3
-    for d, o in zip(objs, out):
-        assert o["x"].dtype == np.int64 and np.array_equal(o["x"], d.x.numpy())
-        assert o["edge_index"].dtype == np.int64 and np.array_equal(o["edge_index"], d.edge_index.numpy())
-        assert o["y"] == int(d.y)
+    for (x, ei, y), o in zip(graphs, out):
+        assert o["x"].dtype == np.int64 and np.array_equal(o["x"], x.numpy())
+        assert o["edge_index"].dtype == np.int64 and np.array_equal(o["edge_index"], ei.numpy())
+        assert o["y"] == int(y)
 
 
 def test_read_exp_pickle_matches_the_committed_fixture():
-    """First 200 graphs of the real GRAPHSAT.pkl against tests/golden/exp_first200.npz (written by oracle/make_golden.py through
-    the PyG stand-in).  Needs the reference checkout, which only exists in the build container."""
+    """The first 200 graphs of the EXP dataset (tests/golden/exp_first200.npz, taken from the reference's GRAPHSAT.pkl by
+    oracle/make_golden.py), pickled as the dataset file stores them (int64 tensors: x [n, 1] node types, edge_index [2, e],
+    y [1]), are read back exactly and in file order."""
     from gnn_matlang_b200.datasets import read_exp_pickle
-    raw = "/root/reference/dataset/EXP/raw/GRAPHSAT.pkl"
-    if not os.path.exists(raw):
-        pytest.skip("reference checkout not present")
-    e = read_exp_pickle(raw)
-    assert len(e) == 1200
     z = np.load(os.path.join(GOLDEN, "exp_first200.npz"))
     xo, eo = np.cumsum(np.r_[0, z["n"]]), np.cumsum(np.r_[0, z["ne"]])
+    t = lambda a: torch.from_numpy(a.astype(np.int64))
+    e = read_exp_pickle(_pyg_pickle([(t(z["x"][xo[i]:xo[i + 1]]).reshape(-1, 1), t(z["edge_index"][:, eo[i]:eo[i + 1]]), t(z["y"][i:i + 1]))
+                                     for i in range(200)]))
+    assert len(e) == 200
     for i in range(200):
+        assert e[i]["x"].shape == (z["n"][i], 1)
         assert np.array_equal(e[i]["x"].reshape(-1), z["x"][xo[i]:xo[i + 1]])
         assert np.array_equal(e[i]["edge_index"], z["edge_index"][:, eo[i]:eo[i + 1]])
         assert e[i]["y"] == int(z["y"][i])
@@ -153,15 +162,40 @@ def test_read_mat_zinc_and_counting_schemas(tmp_path):
         assert np.array_equal(r["edge_index"], np.vstack(np.where(a > 0)))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/dataset/enzymes/raw/enzymes.mat"), reason="reference checkout not present")
+def _write_tu_mat(path, kind, count):
+    """A file in the schema of the reference's TU file ``kind``, with ``count`` seeded random graphs: ``A`` and ``F`` are
+    1 x count cells of sparse adjacencies and node feature matrices; the labels are ``Y`` (1 x count, ENZYMES' classes 1..6),
+    ``Y`` (count x 1, PROTEINS / PTC) or ``y`` (count x 1 in {-1, 1}, MUTAG)."""
+    import scipy.io as sio
+    import scipy.sparse as sp
+    rng = np.random.default_rng(count)
+    width = dict(enzymes=21, proteins=4, ptc=18, mutag=7)[kind]
+    A = np.empty((1, count), dtype=object)
+    F = np.empty((1, count), dtype=object)
+    for i in range(count):
+        n = int(rng.integers(1, 30))
+        up = np.triu(rng.random((n, n)) < 3.0 / n, 1)
+        A[0, i] = sp.csc_matrix((up | up.T).astype(np.float64))
+        F[0, i] = rng.integers(0, 2, (n, width)).astype(np.float64)
+    if kind == "enzymes":
+        labels = {"Y": rng.integers(1, 7, (1, count))}
+    elif kind == "mutag":
+        labels = {"y": rng.choice([-1, 1], (count, 1))}
+    else:
+        labels = {"Y": rng.integers(0, 2, (count, 1))}
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    sio.savemat(path, dict(A=A, F=F, **labels))
+
+
 @pytest.mark.parametrize("kind,rel,count,nfeat", [("enzymes", "enzymes/raw/enzymes.mat", 600, 3), ("proteins", "proteins/raw/proteins.mat", 1113, 3),
                                                   ("ptc", "PTC/raw/ptc.mat", 344, None), ("mutag", "mutag/raw/mutag.mat", 188, None)])
-def test_read_mat_tu_files_shipped_with_the_reference(kind, rel, count, nfeat):
-    """The TU files that ship with the reference, against a restatement of the dataset classes' process() lines
-    (libs/utils.py:46-61, 93-112, 146-165, 195-211)."""
+def test_read_mat_tu_files_shipped_with_the_reference(kind, rel, count, nfeat, tmp_path):
+    """Files in the schema of the TU files that ship with the reference (as many graphs as each of them holds), against a
+    restatement of the dataset classes' process() lines (libs/utils.py:46-61, 93-112, 146-165, 195-211)."""
     import scipy.io as sio
     from gnn_matlang_b200.datasets import read_mat
-    path = os.path.join("/root/reference/dataset", rel)
+    path = str(tmp_path / rel)
+    _write_tu_mat(path, kind, count)
     recs = read_mat(path, kind)
     a = sio.loadmat(path)
     assert len(recs) == count
