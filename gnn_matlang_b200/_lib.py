@@ -73,7 +73,13 @@ SIGNATURES = {
                                      _i64, _p, _p, _i64, _p, _sz, _p]),
     "gnnml3_ml3layer_backward": (_i, [_p, _p, _p, _p, _p, _p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p, _i, _p, _p, _i,
                                       _p, _i64, _p, _p, _i64, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _sz, _p]),
-    "gnnml3_segment_pool_fwd": (_i, [_p, _i64, _p, _i, _i, _i, _p, _p]),
+    "gnnml3_ml1layer_supported": (_i, [_i, _i, _i]),
+    "gnnml3_ml1layer_workspace_bytes": (_sz, [_i64, _i, _i, _i]),
+    "gnnml3_ml1layer_forward": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64,
+                                     _p, _i64, _p, _sz, _p]),
+    "gnnml3_ml1layer_backward": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64, _p, _i64, _i,
+                                      _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "gnnml3_segment_pool_fwd":(_i, [_p, _i64, _p, _i, _i, _i, _p, _p]),
     "gnnml3_segment_pool_bwd": (_i, [_p, _p, _i, _i, _i, _p, _i64, _p]),
     "gnnml3_segment_max_fwd": (_i, [_p, _i64, _p, _i, _i, _p, _p, _p]),
     "gnnml3_segment_max_bwd": (_i, [_p, _p, _p, _i, _i, _p, _i64, _p]),

@@ -48,9 +48,11 @@ class Batch(object):
         return sum(v.numel() * v.element_size() for v in self.__dict__.values() if isinstance(v, torch.Tensor))
 
 
-def collate(graphs):
+def collate(graphs, adjacency=False):
     """``graphs``: sequence of dicts / objects with ``x [n,f]``, ``edge_index2 [2,e]``, ``edge_attr2 [e,K]``
-    and optionally ``y``.  Returns a host ``Batch``."""
+    and optionally ``y``.  Returns a host ``Batch``.  ``adjacency=True``: the records also carry the graph's plain
+    ``edge_index [2, m]`` (what GNNML1 reads), concatenated and shifted by the running node count like ``edge_index2``; records
+    without ``edge_index2`` (GNNML1 needs no SpectralDesign supports) then give a batch without ``edge_index2`` / ``edge_attr2``."""
     def get(g, k):
         return g.get(k) if isinstance(g, dict) else getattr(g, k, None)
 
@@ -58,15 +60,20 @@ def collate(graphs):
     off = np.zeros(len(graphs) + 1, dtype=np.int64)
     np.cumsum(ns, out=off[1:])
     x = torch.cat([torch.as_tensor(get(g, "x"), dtype=torch.float32) for g in graphs], 0)
-    ei = torch.cat([torch.as_tensor(get(g, "edge_index2"), dtype=torch.int64) + int(o) for g, o in zip(graphs, off[:-1])], 1)
-    ea = torch.cat([torch.as_tensor(get(g, "edge_attr2"), dtype=torch.float32) for g in graphs], 0)
+    kw = dict(x=x)
+    if not adjacency or all(get(g, "edge_index2") is not None for g in graphs):
+        kw["edge_index2"] = torch.cat([torch.as_tensor(get(g, "edge_index2"), dtype=torch.int64) + int(o) for g, o in zip(graphs, off[:-1])], 1)
+        kw["edge_attr2"] = torch.cat([torch.as_tensor(get(g, "edge_attr2"), dtype=torch.float32) for g in graphs], 0)
     batch = torch.from_numpy(np.repeat(np.arange(len(graphs), dtype=np.int64), ns))
-    out = Batch(x=x, edge_index2=ei, edge_attr2=ea, batch=batch, num_graphs=len(graphs),
-                graph_ptr=torch.from_numpy(off.astype(np.int32)))
+    kw.update(batch=batch, num_graphs=len(graphs), graph_ptr=torch.from_numpy(off.astype(np.int32)))
+    out = Batch(**kw)
     ys = [get(g, "y") for g in graphs]
     if all(y is not None for y in ys) and len(ys) > 0:
         ys = [torch.as_tensor(y) for y in ys]
         out.y = torch.cat([y.reshape(1, -1) if y.dim() < 2 else y for y in ys], 0)
+    if adjacency:
+        out.edge_index = torch.cat([torch.as_tensor(get(g, "edge_index"), dtype=torch.int64).reshape(2, -1) + int(o)
+                                    for g, o in zip(graphs, off[:-1])], 1)
     return out
 
 

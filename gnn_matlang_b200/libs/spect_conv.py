@@ -6,6 +6,8 @@ constructor / forward signatures, parameter names, shapes, initialisation and ``
 * ``SpectConv(in_channels, out_channels, K=1, selfconn=True, depthwise=False, bias=True)``
   -- reference libs/spect_conv.py:23-103 (a PyG ``MessagePassing`` module there).
 * ``ML3Layer(learnedge, nedgeinput, nedgeoutput, ninp, nout1, nout2)`` -- reference libs/spect_conv.py:182-212.
+* ``ML1Layer(ninp, nout, concat=False)`` -- the GNNML1 layer the reference's experiment scripts define next to GNNML3
+  (``SpectConv`` K=1 on all-ones edge weights + three ``nn.Linear``), as one fused library call per direction.
 
 What runs underneath is different: instead of K x (index_select, mul, scatter_add, matmul, add) the batch's
 edge list is turned once into a dst-sorted CSR (``graph.GraphPlan``), one segmented-reduction kernel applies
@@ -641,3 +643,96 @@ class ML3Layer(torch.nn.Module):
         w = (self.fc1_1.weight, self.fc1_2.weight, self.fc1_3.weight, self.fc1_4.weight) if fused_edge else (None,) * 4
         g = (self.fc11.weight, self.fc11.bias, self.fc12.weight, self.fc12.bias) if self.nout2 > 0 else (None,) * 4
         return _ML3LayerFn.apply(x, ea, *w, c.weight, c.bias, *g, plan, fused_edge, prec)
+
+
+# paths taken by ML1Layer since import (tests and benchmarks read it): "fused" = one library call per direction, "composed" =
+# the layer composed from the aggregation kernel and the tensor-core GEMMs (shapes outside gnnml3_ml1layer_supported)
+ML1_PATH_COUNTS = {"fused": 0, "composed": 0}
+
+
+class _ML1LayerFn(torch.autograd.Function):
+    """Whole GNNML1 layer as one autograd node (gnnml3_ml1layer_forward / _backward):
+
+        p0 = x WA^T + bA + (A x) Wc + bc,   p1 = x WB^T + bB,   p2 = x WC^T + bC
+        y  = relu(p0 + p1 * p2)   or, concatenated,   [relu(x WA^T + bA) | relu((A x) Wc + bc) | relu(p1 * p2)]
+
+    Backward: G = [gA | gP p2 | gP p1] from the masks of y; dx = (A^T gc) Wc^T + G [WA ; WB ; WC] (one fused kernel over the
+    transposed CSR); [dWA^T | dWB^T | dWC^T | dWc] = x^T [G | A^T gc] (one contraction); biases = column sums of G and gc."""
+
+    @staticmethod
+    def forward(ctx, x, wconv, bconv, wA, bA, wB, bB, wC, bC, plan, concat):
+        xa = ops.aligned_rows(x)
+        ws = [w.contiguous() for w in (wconv, wA, wB, wC)]
+        bs = [b.contiguous() if b is not None else None for b in (bconv, bA, bB, bC)]
+        y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat)
+        ctx.plan, ctx.concat = plan, concat
+        ctx.has_bias = tuple(b is not None for b in (bconv, bA, bB, bC))
+        ctx.save_for_backward(xa, *ws, y, aux)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        xa, wconv, wA, wB, wC, y, aux = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        N, Fi = xa.shape
+        if N == 0:
+            z = torch.zeros_like
+            bz = [torch.zeros(wconv.size(2), device=xa.device) if h else None for h in ctx.has_bias]
+            return z(xa), z(wconv), bz[0], z(wA), bz[1], z(wB), bz[2], z(wC), bz[3], None, None
+        gy = gy if gy.stride(1) == 1 else gy.contiguous()
+        dx, dwc, dbc, dwA, dbA, dwB, dbB, dwC, dbC = ops.ml1layer_backward(ctx.plan, xa, wconv, wA, wB, wC, y, aux, gy, need[0],
+                                                                          concat=ctx.concat)
+        hb = ctx.has_bias
+        return (dx, dwc, dbc if hb[0] else None, dwA, dbA if hb[1] else None, dwB, dbB if hb[2] else None, dwC,
+                dbC if hb[3] else None, None, None)
+
+
+class ML1Layer(torch.nn.Module):
+    """GNNML1 layer, the paper's 1-WL model (the GNNML1 classes of the reference's experiment scripts):
+    ``relu(fc11(x) + conv1(x, edge_index, ones) + fc12(x) * fc13(x))`` or, with ``concat=True``,
+    ``[relu(fc11(x)) | relu(conv1(x, edge_index, ones)) | relu(fc12(x) * fc13(x))]``.
+
+    ``conv1`` is a ``SpectConv(ninp, nout, K=1, selfconn=False)`` on the graph's plain ``edge_index`` with every edge weight
+    one; ``fc11``, ``fc12``, ``fc13`` are ``nn.Linear(ninp, nout)``.  ``forward(x, edge_index)`` -> [N, nout] (or [N, 3 nout]).
+    Shapes with ninp, nout <= 64 run as one fused library call per direction; larger ones are composed from the aggregation
+    kernel and the tensor-core GEMMs of this library, with the same result."""
+
+    def __init__(self, ninp, nout, concat=False):
+        super(ML1Layer, self).__init__()
+        self.concat = bool(concat)
+        self.conv1 = SpectConv(ninp, nout, 1, selfconn=False)
+        self.fc11 = torch.nn.Linear(ninp, nout)
+        self.fc12 = torch.nn.Linear(ninp, nout)
+        self.fc13 = torch.nn.Linear(ninp, nout)
+
+    @property
+    def out_features(self):
+        return self.conv1.out_channels * (3 if self.concat else 1)
+
+    def forward(self, x, edge_index):
+        return ml1_layer(x, edge_index, self.conv1, self.fc11, self.fc12, self.fc13, self.concat)
+
+
+def ml1_layer(x, edge_index, conv, fcA, fcB, fcC, concat=False):
+    """The GNNML1 layer on given modules (``conv`` a SpectConv(K=1, selfconn=False), ``fcA``/``fcB``/``fcC`` nn.Linear):
+    what ``ML1Layer.forward`` and ``models.GNNML1`` run."""
+    if not (x.is_cuda and edge_index.is_cuda):
+        raise RuntimeError("gnn_matlang_b200: x and edge_index must be CUDA tensors (the B200 hot path has no CPU fallback)")
+    if x.dim() != 2 or x.dtype != torch.float32:
+        raise RuntimeError("gnn_matlang_b200: x [N, F] must be float32")
+    plan = get_plan(edge_index, x.size(0))
+    Fi, Fo = conv.in_channels, conv.out_channels
+    if ops.ml1layer_supported(Fi, Fo, concat):
+        ML1_PATH_COUNTS["fused"] += 1
+        return _ML1LayerFn.apply(x, conv.weight, conv.bias, fcA.weight, fcA.bias, fcB.weight, fcB.bias, fcC.weight, fcC.bias, plan,
+                                 bool(concat))
+    ML1_PATH_COUNTS["composed"] += 1
+    prec = _lib.PREC_3XTF32
+    ones = torch.ones(plan.E, 1, dtype=torch.float32, device=x.device)
+    ax = _AggregateFn.apply(x, ones, plan)
+    pa = _LinearFn.apply(x, fcA.weight.t(), fcA.bias, prec)
+    pc = _LinearFn.apply(ax, conv.weight[0], conv.bias, prec)
+    pp = _LinearFn.apply(x, fcB.weight.t(), fcB.bias, prec) * _LinearFn.apply(x, fcC.weight.t(), fcC.bias, prec)
+    if concat:
+        return torch.cat([torch.relu(pa), torch.relu(pc), torch.relu(pp)], 1)
+    return torch.relu(pa + pc + pp)

@@ -18,11 +18,15 @@ concatenated read-outs, log-softmax heads:
 
 The same (unlearned) ``edge_attr2`` feeds every layer; the graph plan (CSR) is built once per batch.  BatchNorm, dropout and
 log-softmax are torch modules (statistics / elementwise work on [N, F] and [B, F], outside the hot path of SURVEY.md 8a).
+
+``GNNML1`` is the paper's 1-WL model, defined next to GNNML3 in every experiment script of the reference: ``nlayer`` GNNML1
+layers (``libs.spect_conv.ML1Layer``) on the graph's plain ``edge_index``, then the pool and head of the same-named GNNML3
+preset (``graph8c``, ``zinc``, ``exp``, ``counting``).
 """
 import torch
 import torch.nn as nn
 
-from .libs.spect_conv import ML3Layer, _LinearFn, _PRECISIONS
+from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _PRECISIONS, ml1_layer
 import torch.nn.functional as F
 
 from .pool import global_add_pool, global_max_pool, global_mean_pool
@@ -88,4 +92,49 @@ class GNNML3(nn.Module):
                 return torch.tanh(x)
             return F.log_softmax(x, dim=1) if c["final"] == "log_softmax" else x
         x = _LinearFn.apply(x, self.fc1.weight.t(), self.fc1.bias, prec)
+        return _LinearFn.apply(torch.relu(x), self.fc2.weight.t(), self.fc2.bias, prec)
+
+
+GNNML1_PRESETS = ("graph8c", "zinc", "exp", "counting")
+
+
+class GNNML1(nn.Module):
+    """GNNML1: ``nlayer`` x [relu(fc{l}1(x) + conv{l}1(x, edge_index, ones) + fc{l}2(x) * fc{l}3(x))] (or the concatenated
+    form with ``concat=True``: layer width 3 * nout), then the read-out and head of ``MODEL_CONFIGS[config]``.  Parameters keep
+    the reference's names: ``conv{l}1`` (SpectConv(K=1, selfconn=False)), ``fc{l}1``, ``fc{l}2``, ``fc{l}3`` (nn.Linear) for
+    l = 1..nlayer, then the head (``fc1``, ``fc2``).  ``forward(data)`` reads ``data.x``, ``data.edge_index``, ``data.batch``
+    (``batch.collate(graphs, adjacency=True)`` provides ``edge_index``)."""
+
+    def __init__(self, config, ninp, nlayer=3, nout=64, concat=False):
+        super().__init__()
+        if isinstance(config, str) and config not in GNNML1_PRESETS:
+            raise ValueError("GNNML1 presets: %s" % (GNNML1_PRESETS,))
+        c = dict(MODEL_CONFIGS[config]) if isinstance(config, str) else dict(config)
+        self.cfg = c
+        self.nlayer, self.concat = int(nlayer), bool(concat)
+        width = nout * (3 if concat else 1)
+        for l in range(1, self.nlayer + 1):
+            nin = ninp if l == 1 else width
+            setattr(self, "conv%d1" % l, SpectConv(nin, nout, 1, selfconn=False))
+            setattr(self, "fc%d1" % l, nn.Linear(nin, nout))
+            setattr(self, "fc%d2" % l, nn.Linear(nin, nout))
+            setattr(self, "fc%d3" % l, nn.Linear(nin, nout))
+        self.fc1 = nn.Linear(width, c["head"][0])
+        if len(c["head"]) > 1:
+            self.fc2 = nn.Linear(c["head"][0], c["head"][1])
+
+    def forward(self, data):
+        x = data.x
+        edge_index = data.edge_index
+        for l in range(1, self.nlayer + 1):
+            x = ml1_layer(x, edge_index, getattr(self, "conv%d1" % l), getattr(self, "fc%d1" % l), getattr(self, "fc%d2" % l),
+                          getattr(self, "fc%d3" % l), self.concat)
+        c = self.cfg
+        B = getattr(data, "num_graphs", None)
+        pool = {"add": global_add_pool, "mean": global_mean_pool}[c["pool"]]
+        x = pool(x, data.batch, B)
+        prec = _PRECISIONS["fp32"]
+        x = _LinearFn.apply(x, self.fc1.weight.t(), self.fc1.bias, prec)
+        if len(c["head"]) == 1:
+            return torch.tanh(x) if c["final"] == "tanh" else x
         return _LinearFn.apply(torch.relu(x), self.fc2.weight.t(), self.fc2.bias, prec)

@@ -558,6 +558,55 @@ def ml3layer_backward(plan, x, ea_s, ea2, ws4, wconv, gates_w, y, aux, gy, need_
     return (dx[:, :Fi] if need_dx else None), dea, dws, dwc, dbc, dw11, db11, dw12, db12
 
 
+def ml1layer_supported(Fi, Fo, concat=False):
+    return bool(_lib.load().gnnml3_ml1layer_supported(int(Fi), int(Fo), int(bool(concat))))
+
+
+def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False, keep_aggregate=False):
+    """Whole GNNML1 layer forward in one library call (gnnml3_ml1layer_forward) over the plan of the plain ``edge_index``.
+    x [N, Fi] must satisfy ``aligned_rows``; wconv [1, Fi, Fo]; wA/wB/wC [Fo, Fi].  -> (y [N, Fo] or [N, 3 Fo],
+    aux [N, 2 Fo] = [p1 | p2], A x [N, Fi] if ``keep_aggregate`` else None)"""
+    lib = _lib.load()
+    N, Fi = x.shape
+    Fo = wconv.size(2)
+    dev = x.device
+    W = 3 * Fo if concat else Fo
+    y = _padded_rows(N, W, dev)
+    aux = torch.empty(N, 2 * Fo, dtype=torch.float32, device=dev)
+    hside = _padded_rows(N, Fi, dev) if keep_aggregate else None
+    ws = _ws(dev, lib.gnnml3_ml1layer_workspace_bytes(N, Fi, Fo, int(bool(concat))), tag="ml1")
+    p = _lib.ptr
+    with _on(dev):
+        _lib.check(lib.gnnml3_ml1layer_forward(p(plan.rowptr), p(plan.col), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(bconv), p(wA), p(bA),
+                                               p(wB), p(bB), p(wC), p(bC), Fo, int(bool(concat)), p(y), _ld(y) if N > 1 else (W + 3) // 4 * 4,
+                                               p(aux), 2 * Fo, p(hside), (Fi + 3) // 4 * 4, p(ws), ws.numel(), _lib.stream_ptr()),
+                   "gnnml3_ml1layer_forward")
+    return y, aux, hside
+
+
+def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=False):
+    """Whole GNNML1 layer backward in one library call (gnnml3_ml1layer_backward).
+    -> dx (None unless need_dx), dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC"""
+    lib = _lib.load()
+    N, Fi = x.shape
+    Fo = wconv.size(2)
+    dev = x.device
+    f32 = dict(dtype=torch.float32, device=dev)
+    lddx = (Fi + 3) // 4 * 4
+    dx = torch.empty(N, lddx, **f32) if need_dx else None
+    dwc = torch.empty_like(wconv)
+    dwA, dwB, dwC = torch.empty_like(wA), torch.empty_like(wB), torch.empty_like(wC)
+    dbs = torch.empty(4, Fo, **f32)                      # conv | fcA | fcB | fcC
+    ws = _ws(dev, lib.gnnml3_ml1layer_workspace_bytes(N, Fi, Fo, int(bool(concat))), tag="ml1")
+    p = _lib.ptr
+    with _on(dev):
+        _lib.check(lib.gnnml3_ml1layer_backward(
+            p(plan.rowptrT), p(plan.colT), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(wA), p(wB), p(wC), Fo, int(bool(concat)),
+            p(y), _ld(y) if N > 1 else y.size(1), p(aux), 2 * Fo, p(gy), _ld(gy), int(bool(need_dx)), p(dx), lddx, p(dwc), p(dbs[0]),
+            p(dwA), p(dbs[1]), p(dwB), p(dbs[2]), p(dwC), p(dbs[3]), p(ws), ws.numel(), _lib.stream_ptr()), "gnnml3_ml1layer_backward")
+    return (dx[:, :Fi] if need_dx else None), dwc, dbs[0], dwA, dbs[1], dwB, dbs[2], dwC, dbs[3]
+
+
 def collate_device(n, e, el, ea, B, out, idx=None, node_off=None, edge_off=None, xc=None, widths=None, x=None):
     """Batch B per-graph records on the device (gnnml3_collate) into the tensors of ``out`` (a ``Batch`` whose ``x [Np, F]``,
     ``edge_index2 [2, Ep]`` int64, ``edge_attr2 [Ep, K]``, ``batch [Np]`` int64 and ``graph_ptr`` int32 are preallocated; rows

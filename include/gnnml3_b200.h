@@ -250,6 +250,35 @@ GNNML3_API int gnnml3_ml3layer_backward(const int32_t* rowptr, const int32_t* co
                              void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
+ * Whole-layer entry points of GNNML1, the paper's 1-WL model (ml1_layer.cu).  With A the adjacency of the plain edge_index
+ * ((A x)[t] = sum of x[s] over the edges s -> t; every edge weight is one and none is read), wconv [1, Fi, Fo] / bconv [Fo]
+ * (SpectConv(Fi, Fo, K=1, selfconn=False)) and the nn.Linear(Fi, Fo) weights wA, wB, wC [Fo, Fi] with biases bA, bB, bC:
+ *   p0 = x wA^T + bA + (A x) wconv[0] + bconv,   p1 = x wB^T + bB,   p2 = x wC^T + bC
+ *   concat = 0: y = relu(p0 + p1 * p2)                                                        [N, Fo]
+ *   concat = 1: y = [relu(x wA^T + bA) | relu((A x) wconv[0] + bconv) | relu(p1 * p2)]         [N, 3 Fo]
+ * One fused kernel per direction: the aggregate and the four projections meet in tensor memory (tcgen05, 3xTF32, FP32-grade).
+ *   forward : rowptr / col = the dst-sorted CSR of edge_index (gnnml3_csr_build); outputs y [N, ldy] and aux [N, ldaux >= 2 Fo]
+ *             = [p1 | p2] (saved for the backward); hside (nullable, [N, ldh >= Fi]) receives A x.  Biases are nullable.
+ *   backward: rowptrT / colT = the transposed CSR; gy [N, ldgy]; dx [N, lddx] if need_dx (else dx may be NULL: the aggregate
+ *             A^T gc is still formed for d wconv); outputs the eight parameter gradients (dw* overwritten; db* nullable).
+ * Supported: 1 <= Fi <= 64, 1 <= Fo <= 64 (gnnml3_ml1layer_supported), E = 0 allowed; x rows 16-byte aligned (ldx % 4 == 0).
+ * Deterministic (fixed summation order, no atomics), no host sync; caller-provided workspace.
+ * --------------------------------------------------------------------------------------------------- */
+GNNML3_API int gnnml3_ml1layer_supported(int Fi, int Fo, int concat);
+GNNML3_API size_t gnnml3_ml1layer_workspace_bytes(int64_t N, int Fi, int Fo, int concat);
+GNNML3_API int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x, int64_t ldx,
+                            int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA, const float* wB,
+                            const float* bB, const float* wC, const float* bC, int Fo, int concat, float* y, int64_t ldy,
+                            float* aux, int64_t ldaux, float* hside, int64_t ldh, void* workspace, size_t workspace_bytes,
+                            void* stream);
+GNNML3_API int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
+                             int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
+                             const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
+                             int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
+                             float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
+                             void* stream);
+
+/* ---------------------------------------------------------------------------------------------------
  * Readout: PyG global_add_pool (mean = 0) / global_mean_pool (mean = 1) over contiguous node ranges
  * graph_ptr [B+1] (graph b owns nodes graph_ptr[b] .. graph_ptr[b+1]-1, as produced by batching).
  * --------------------------------------------------------------------------------------------------- */

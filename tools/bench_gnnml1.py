@@ -1,0 +1,226 @@
+#!/usr/bin/env python
+"""bench_gnnml1.py -- GNNML1 (the paper's 1-WL model) on one B200.  Prints ONE JSON line with
+
+* the training step (forward, L1-sum loss, backward, Adam) of the GNNML1 ``zinc`` preset on a batch of ZINC-shaped graphs
+  (``synthetic.zinc_graph``; 8192 by default), with the fused GNNML1 layers of this library;
+* in the same process, alternating with it, the same model as a user would compose it today: this package's
+  ``SpectConv(K=1, selfconn=False)`` on a ``ones[E, 1]`` edge weight plus three ``torch.nn.Linear`` and torch elementwise ops;
+* the largest deviation between the two paths' losses and gradients on that batch (same weights);
+* CUDA-event times of one ``gnnml3_ml1layer_forward`` / ``_backward`` call at the layer-2 shape (64 -> 64) and, from a separate
+  ``torch.profiler`` pass, the device time of the fused kernel in the forward and in the dx pass, with the algorithmic bytes of
+  each launch (every operand once) and their share of the 7.7 TB/s HBM3e bandwidth of one B200 (NVIDIA HGX B200 data sheet);
+* the time to embed all 11,117 graph8c graphs (one batch, eval mode);
+* the card's name and power limit, read in the same run.
+
+    python tools/bench_gnnml1.py [--batch 8192] [--steps 20] [--warmup 5] [--rounds 3] [--out FILE]
+
+Nothing is written unless --out is given.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+import torch
+import torch.nn as nn
+import torch.nn.functional as F
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+HBM_PEAK = 7.7e12        # bytes/s, one B200 (HGX B200 data sheet)
+
+
+def card():
+    name = torch.cuda.get_device_name(0)
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception as e:                                   # pragma: no cover
+        q = "unavailable (%s)" % e
+    return dict(name=name, power_limit_and_max_sm_clock=q)
+
+
+def zinc_batch(B, seed):
+    from gnn_matlang_b200.batch import collate
+    from gnn_matlang_b200.synthetic import zinc_graph
+    rng = np.random.default_rng(seed)
+    gs = []
+    for _ in range(B):
+        n, ei, x = zinc_graph(rng)
+        gs.append(dict(x=x, edge_index=ei, y=np.float32(rng.standard_normal())))
+    return collate(gs, adjacency=True)
+
+
+class ComposedGNNML1(nn.Module):
+    """GNNML1 as a user writes it without the fused layer: SpectConv on ones[E, 1], three nn.Linear (cuBLAS), torch glue.
+    Same parameter names as models.GNNML1, so one state_dict serves both."""
+
+    def __init__(self, ref):
+        super().__init__()
+        from gnn_matlang_b200.libs.spect_conv import SpectConv
+        self.cfg, self.nlayer = ref.cfg, ref.nlayer
+        for l in range(1, ref.nlayer + 1):
+            c = getattr(ref, "conv%d1" % l)
+            setattr(self, "conv%d1" % l, SpectConv(c.in_channels, c.out_channels, 1, selfconn=False))
+            for j in (1, 2, 3):
+                fc = getattr(ref, "fc%d%d" % (l, j))
+                setattr(self, "fc%d%d" % (l, j), nn.Linear(fc.in_features, fc.out_features))
+        self.fc1 = nn.Linear(ref.fc1.in_features, ref.fc1.out_features)
+        self.fc2 = nn.Linear(ref.fc2.in_features, ref.fc2.out_features)
+        self.load_state_dict(ref.state_dict())
+
+    def forward(self, data):
+        from gnn_matlang_b200.pool import global_add_pool
+        x, ei = data.x, data.edge_index
+        ones = torch.ones(ei.size(1), 1, device=x.device)
+        for l in range(1, self.nlayer + 1):
+            x = F.relu(getattr(self, "fc%d1" % l)(x) + getattr(self, "conv%d1" % l)(x, ei, ones)
+                       + getattr(self, "fc%d2" % l)(x) * getattr(self, "fc%d3" % l)(x))
+        x = global_add_pool(x, data.batch, data.num_graphs)
+        return self.fc2(F.relu(self.fc1(x)))
+
+
+def timed_steps(model, opt, b, steps):
+    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    start.record()
+    for _ in range(steps):
+        opt.zero_grad(set_to_none=True)
+        loss = (model(b).view(-1) - b.y.view(-1)).abs().sum()
+        loss.backward()
+        opt.step()
+    end.record()
+    torch.cuda.synchronize()
+    return start.elapsed_time(end) / steps
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--batch", type=int, default=8192)
+    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--out", default=None)
+    a = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_gnnml1.py measures the GPU: no CUDA device")
+    from gnn_matlang_b200 import ops
+    from gnn_matlang_b200.batch import collate
+    from gnn_matlang_b200.datasets import read_graph6
+    from gnn_matlang_b200.graph import get_plan
+    from gnn_matlang_b200.models import GNNML1
+    d = torch.device("cuda:0")
+    res = dict(metric="gnnml1_zinc_train_step", card=card(), batch_graphs=a.batch)
+
+    hb = zinc_batch(a.batch, 0)
+    b = hb.to(d)
+    N, E = int(b.x.shape[0]), int(b.edge_index.shape[1])
+    res.update(nodes=N, edges=E)
+    torch.manual_seed(0)
+    fused = GNNML1("zinc", ninp=25).to(d)
+    comp = ComposedGNNML1(fused).to(d)
+    res["model"] = "GNNML1 zinc preset: %d layers, width %d, sum mode, add-pool, fc2(relu(fc1 -> 32)) -> 1" % (fused.nlayer, 64)
+
+    # deviation of the two paths at this size, identical weights, before any update
+    for m in (fused, comp):
+        m.zero_grad(set_to_none=True)
+    losses = []
+    for m in (fused, comp):
+        loss = (m(b).view(-1) - b.y.view(-1)).abs().sum()
+        loss.backward()
+        losses.append(loss.detach().double())
+    gf, gc = dict(fused.named_parameters()), dict(comp.named_parameters())
+    dev_rel = {k: float((gf[k].grad.double() - gc[k].grad.double()).abs().max() / gc[k].grad.double().abs().max().clamp_min(1e-30))
+               for k in gf}
+    res["loss_fused"], res["loss_composed"] = float(losses[0]), float(losses[1])
+    res["loss_rel_dev"] = float((losses[0] - losses[1]).abs() / losses[1].abs())
+    res["grad_max_rel_dev"] = max(dev_rel.values())
+    res["grad_max_rel_dev_param"] = max(dev_rel, key=dev_rel.get)
+
+    of = torch.optim.Adam(fused.parameters(), lr=1e-3)
+    oc = torch.optim.Adam(comp.parameters(), lr=1e-3)
+    timed_steps(fused, of, b, a.warmup)
+    timed_steps(comp, oc, b, a.warmup)
+    tf, tc = [], []
+    for _ in range(a.rounds):
+        tf.append(timed_steps(fused, of, b, a.steps))
+        tc.append(timed_steps(comp, oc, b, a.steps))
+    res["ms_per_step_fused"] = tf
+    res["ms_per_step_composed"] = tc
+    res["graphs_per_s_fused"] = a.batch / (min(tf) * 1e-3)
+    res["graphs_per_s_composed"] = a.batch / (min(tc) * 1e-3)
+    res["speedup_vs_composed"] = min(tc) / min(tf)
+
+    # the layer entry points at the layer-2 shape (64 -> 64, sum mode)
+    plan = get_plan(b.edge_index, N)
+    g = torch.Generator().manual_seed(1)
+    Fi = Fo = 64
+    x = torch.randn(N, Fi, generator=g).to(d)
+    L = fused.conv21, fused.fc21, fused.fc22, fused.fc23
+    w = [L[0].weight.detach(), L[1].weight.detach(), L[2].weight.detach(), L[3].weight.detach()]
+    bs = [L[0].bias.detach(), L[1].bias.detach(), L[2].bias.detach(), L[3].bias.detach()]
+    fwd = lambda: ops.ml1layer_forward(plan, x, w[0], bs[0], w[1], bs[1], w[2], bs[2], w[3], bs[3])   # noqa: E731
+    y, aux, _ = fwd()
+    gy = torch.randn(N, Fo, generator=g).to(d)
+    bwd = lambda: ops.ml1layer_backward(plan, x, w[0], w[1], w[2], w[3], y, aux, gy, True)            # noqa: E731
+
+    def ev(fn, reps=50):
+        for _ in range(5):
+            fn()
+        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        s.record()
+        for _ in range(reps):
+            fn()
+        e.record()
+        torch.cuda.synchronize()
+        return s.elapsed_time(e) / reps
+
+    res["layer_forward_call_ms"] = ev(fwd)
+    res["layer_backward_call_ms"] = ev(bwd)
+
+    def kernel_us(fn, reps=20):
+        from torch.profiler import ProfilerActivity, profile
+        fn()
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(reps):
+                fn()
+            torch.cuda.synchronize()
+        out = {}
+        for evt in prof.key_averages():
+            if evt.device_type.name == "CUDA" and "ml1" in evt.key:
+                t = getattr(evt, "device_time_total", None) or getattr(evt, "cuda_time_total", 0)
+                out[evt.key.split("(")[0].split("<")[0]] = t / max(evt.count, 1)
+        return out
+
+    kf, kb = kernel_us(fwd), kernel_us(bwd)
+    fk = next(v for k, v in kf.items() if "agg_proj" in k)
+    bk = next(v for k, v in kb.items() if "agg_proj" in k)
+    bytes_f = 4.0 * (N * Fi + E + (N + 1) + 4 * Fi * Fo + 4 * Fo + N * Fo + N * 2 * Fo)
+    bytes_b = 4.0 * (N * 3 * Fo + N * Fo + E + (N + 1) + 4 * Fi * Fo + N * Fi + N * Fo)
+    res["kernels_layer2"] = dict(
+        forward_kernel_us=fk, forward_bytes=bytes_f, forward_hbm_share=bytes_f / (fk * 1e-6) / HBM_PEAK,
+        dx_kernel_us=bk, dx_bytes=bytes_b, dx_hbm_share=bytes_b / (bk * 1e-6) / HBM_PEAK,
+        forward_call_kernels_us=kf, backward_call_kernels_us=kb,
+        hbm_peak="7.7 TB/s HBM3e, one B200 (HGX B200 data sheet)",
+        bytes_rule="every operand once: x, CSR, weights, outputs (forward: y and aux; dx: G, gc, dx and the A^T gc side output)")
+
+    # embedding all of graph8c
+    gs = read_graph6(os.path.join(ROOT, "tests", "golden", "graph8c.g6"))
+    g8 = collate(gs, adjacency=True).to(d)
+    torch.manual_seed(0)
+    m8 = GNNML1("graph8c", ninp=1).to(d).eval()
+    with torch.no_grad():
+        res["graph8c_graphs"] = len(gs)
+        res["graph8c_embed_ms"] = ev(lambda: m8(g8), reps=20)
+    line = json.dumps(res)
+    print(line)
+    if a.out:
+        with open(a.out, "w") as f:
+            f.write(line + "\n")
+
+
+if __name__ == "__main__":
+    main()
