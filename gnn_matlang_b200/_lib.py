@@ -41,6 +41,9 @@ SIGNATURES = {
     "gnnml3_edge_mlp_supported": (_i, [_i, _i]),
     "gnnml3_collate_workspace_bytes": (_sz, [_i]),
     "gnnml3_collate": (_i, [_p, _p, _p, _p, _p, _p, _i, _p, _p, _i, _p, _i, _i64, _p, _i, _i, _i64, _i64, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "gnnml3_collate_graphs_workspace_bytes": (_sz, [_i]),
+    "gnnml3_collate_graphs": (_i, [_p, _p, _p, _p, _i, _p, _p, _i, _p, _p, _p, _i, _i64, _p, _i, _p, _p, _p, _i, _i64, _i, _i64, _i64, _i64,
+                                   _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "gnnml3_edge_mlp_set_tc": (_i, [_i]),
     "gnnml3_edge_mlp_path_counts": (_i, [_p, _i]),
     "gnnml3_edge_mlp_fwd": (_i, [_p, _p, _p, _p, _p, _p, _i64, _i, _i, _p, _p]),

@@ -77,6 +77,20 @@ def collate(graphs, adjacency=False):
     return out
 
 
+def _local_ids(ei, gp, n, name):
+    """Global [2, E] edge ids of a collated batch -> (edges per graph, graph-local ids in the smallest integer dtype that holds
+    the largest graph's ids).  The edges must stay inside their graph and be grouped by graph in batch order."""
+    eg = np.searchsorted(gp, ei[0], side="right") - 1            # graph of every edge (by its source node)
+    cnt = np.bincount(eg, minlength=len(n))
+    loc = ei - gp[eg][None, :]
+    if not (np.all(loc >= 0) and np.all(loc[1] < n[eg])):
+        raise ValueError("%s crosses graph boundaries" % name)
+    if len(eg) and np.any(np.diff(eg) < 0):
+        raise ValueError("%s is not grouped by graph" % name)
+    dt = np.uint8 if (n.max() if len(n) else 0) <= 256 else np.int16 if n.max() <= 32768 else np.int32
+    return cnt, np.ascontiguousarray(loc.astype(dt))
+
+
 class CompactBatch(object):
     """Wire format of a batch for the host -> device link (the reference ships every attribute of the PyG batch as it sits in
     host memory: int64 ``edge_index2``, int64 ``batch``, FP32 one-hot ``x`` -- Zinc12k.py:360 ``data.to(device)``):
@@ -86,9 +100,13 @@ class CompactBatch(object):
     * ``xc [N, C]`` uint8 + ``widths``  class codes of a concatenation of one-hot blocks (ZINC: atom type | degree code),
                                        or ``x [N, F]`` float32 when the features are not one-hot
     * ``ea [E, K]`` float32, ``y``    unchanged
+    * ``m [B]`` int32, ``al [2, M]``  for batches of ``collate(..., adjacency=True)``: plain edges per graph and the plain
+                                       ``edge_index`` (what GNNML1 reads) with graph-local ids, like ``e`` / ``el``
 
-    ``expand(device)`` rebuilds the reference's batch attributes ON THE DEVICE, bit-exact (integer work) -- tested against
-    ``collate``.  For the ZINC-shaped bench batches this is 36 bytes per support entry + 2 per node instead of 48 + 108."""
+    A batch without supports (GNNML1 records) has ``e`` / ``el`` / ``ea`` = None; one without the plain list has ``m`` / ``al``
+    = None.  ``expand(device)`` rebuilds the reference's batch attributes ON THE DEVICE, bit-exact (integer work) -- tested
+    against ``collate``.  For the ZINC-shaped bench batches this is 36 bytes per support entry + 2 per node instead of 48 + 108,
+    and 2 bytes per plain edge instead of 16."""
 
     def __init__(self, **kw):
         self.__dict__.update(kw)
@@ -98,17 +116,16 @@ class CompactBatch(object):
         """Host ``Batch`` -> ``CompactBatch`` (numpy work on the host; exact)."""
         gp = b.graph_ptr.numpy().astype(np.int64)
         n = np.diff(gp)
-        ei = b.edge_index2.numpy()
-        eg = np.searchsorted(gp, ei[0], side="right") - 1            # graph of every entry (by its source node)
-        e = np.bincount(eg, minlength=len(n))
-        loc = ei - gp[eg][None, :]
-        if not (np.all(loc >= 0) and np.all(loc[1] < n[eg])):
-            raise ValueError("edge_index2 crosses graph boundaries")
-        if len(eg) and np.any(np.diff(eg) < 0):
-            raise ValueError("edge_index2 is not grouped by graph")
-        dt = np.uint8 if (n.max() if len(n) else 0) <= 256 else np.int16 if n.max() <= 32768 else np.int32
-        kw = dict(n=torch.from_numpy(n.astype(np.int32)), e=torch.from_numpy(e.astype(np.int32)), el=torch.from_numpy(np.ascontiguousarray(loc.astype(dt))),
-                  ea=b.edge_attr2, y=getattr(b, "y", None), num_graphs=len(n), widths=None, x=None, xc=None)
+        kw = dict(n=torch.from_numpy(n.astype(np.int32)), e=None, el=None, ea=None, m=None, al=None, y=getattr(b, "y", None),
+                  num_graphs=len(n), widths=None, x=None, xc=None)
+        if getattr(b, "edge_index2", None) is not None:
+            e, el = _local_ids(b.edge_index2.numpy(), gp, n, "edge_index2")
+            kw.update(e=torch.from_numpy(e.astype(np.int32)), el=torch.from_numpy(el), ea=b.edge_attr2)
+        if getattr(b, "edge_index", None) is not None:
+            m, al = _local_ids(b.edge_index.numpy(), gp, n, "edge_index")
+            kw.update(m=torch.from_numpy(m.astype(np.int32)), al=torch.from_numpy(al))
+        if kw["el"] is None and kw["al"] is None:
+            raise ValueError("the batch has neither edge_index2 nor edge_index")
         x = b.x.numpy()
         if onehot_widths is not None:
             codes, off = [], 0
@@ -141,30 +158,52 @@ class CompactBatch(object):
             out.__dict__[k] = v.to(device, non_blocking=non_blocking)
         return out
 
-    def _out(self, Np, Ep, padded):
+    def sizes(self):
+        """(nodes, support entries, plain edges) of the batch; None for a list it does not carry."""
+        return ((self.xc if self.xc is not None else self.x).size(0), None if self.el is None else self.el.size(1),
+                None if getattr(self, "al", None) is None else self.al.size(1))
+
+    def _out(self, Np, Ep, padded, Mp=None):
         dev = self.n.device
         F = sum(self.widths) if self.xc is not None else self.x.size(1)
         B = self.num_graphs
-        return Batch(x=torch.empty(Np, F, dtype=torch.float32, device=dev), edge_index2=torch.empty(2, Ep, dtype=torch.int64, device=dev),
-                     edge_attr2=torch.empty(Ep, self.ea.size(1), dtype=torch.float32, device=dev),
-                     batch=torch.empty(Np, dtype=torch.int64, device=dev),
-                     graph_ptr=torch.empty(B + (2 if padded else 1), dtype=torch.int32, device=dev), num_graphs=B)
+        out = Batch(x=torch.empty(Np, F, dtype=torch.float32, device=dev))
+        if self.el is not None:
+            out.edge_index2 = torch.empty(2, Ep, dtype=torch.int64, device=dev)
+            out.edge_attr2 = torch.empty(Ep, self.ea.size(1), dtype=torch.float32, device=dev)
+        out.batch = torch.empty(Np, dtype=torch.int64, device=dev)
+        out.graph_ptr = torch.empty(B + (2 if padded else 1), dtype=torch.int32, device=dev)
+        out.num_graphs = B
+        if Mp is not None:
+            out.edge_index = torch.empty(2, Mp, dtype=torch.int64, device=dev)
+        return out
 
     def expand_into(self, out):
         """Device ``CompactBatch`` -> the preallocated device ``Batch`` ``out`` (its tensors may be larger than the batch: the rest
-        receives the neutral padding of ``train.pad_batch``).  Two library launches (``gnnml3_collate``), no host sync; integer
-        work, bit-exact with host ``collate``."""
+        receives the neutral padding of ``train.pad_batch``).  Two library launches (``gnnml3_collate``, or
+        ``gnnml3_collate_graphs`` with the plain list), no host sync; integer work, bit-exact with host ``collate``.  ``out.edge_index``
+        is filled when both carry the plain list."""
         from . import ops
-        ops.collate_device(self.n, self.e, self.el, self.ea, self.num_graphs, out, xc=self.xc, widths=self.widths, x=self.x)
+        al = getattr(self, "al", None)
+        if al is not None and getattr(out, "edge_index", None) is not None:
+            N, _, M = self.sizes()
+            if out.edge_index.size(1) > M and out.x.size(0) <= N:
+                raise ValueError("expand_into: padding edge_index (%d > %d edges) needs dummy nodes (out.x has %d rows for %d nodes)"
+                                 % (out.edge_index.size(1), M, out.x.size(0), N))
+            ops.collate_device(self.n, self.e, self.el, self.ea, self.num_graphs, out, xc=self.xc, widths=self.widths, x=self.x,
+                               m=self.m, al=al)
+        else:
+            ops.collate_device(self.n, self.e, self.el, self.ea, self.num_graphs, out, xc=self.xc, widths=self.widths, x=self.x)
         if self.y is not None and getattr(out, "y", None) is not None and out.y is not self.y:
             out.y.copy_(self.y.reshape(out.y.shape), non_blocking=True)
         return out
 
     def expand(self):
         """Device ``CompactBatch`` -> device ``Batch`` with the reference's attributes (``x``, ``edge_index2`` int64 global ids,
-        ``edge_attr2``, ``batch`` int64, ``y``) + ``graph_ptr``; integer work, bit-exact with host ``collate``."""
-        N, E = (self.xc if self.xc is not None else self.x).size(0), self.el.size(1)
-        out = self._out(N, E, False)
+        ``edge_attr2``, ``edge_index`` when the batch carries the plain list, ``batch`` int64, ``y``) + ``graph_ptr``; integer work,
+        bit-exact with host ``collate``."""
+        N, E, M = self.sizes()
+        out = self._out(N, E, False, M)
         if self.y is not None:
             out.y = self.y
         self.expand_into(out)

@@ -607,31 +607,50 @@ def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=Fa
     return (dx[:, :Fi] if need_dx else None), dwc, dbs[0], dwA, dbs[1], dwB, dbs[2], dwC, dbs[3]
 
 
-def collate_device(n, e, el, ea, B, out, idx=None, node_off=None, edge_off=None, xc=None, widths=None, x=None):
-    """Batch B per-graph records on the device (gnnml3_collate) into the tensors of ``out`` (a ``Batch`` whose ``x [Np, F]``,
-    ``edge_index2 [2, Ep]`` int64, ``edge_attr2 [Ep, K]``, ``batch [Np]`` int64 and ``graph_ptr`` int32 are preallocated; rows
-    beyond the batch's nodes / entries get the neutral padding of a captured step).  Records: ``n`` / ``e`` int32 sizes,
-    ``el [2, *]`` graph-local ids (uint8 / int16 / int32 / int64), ``ea [*, K]``, features ``x [*, F]`` or uint8 class codes
-    ``xc [*, C]`` + ``widths``; ``idx`` (int64 graph ids) with ``node_off`` / ``edge_off`` (int64) select records of a resident
-    pool, None = the records are the batch itself in order."""
+def collate_device(n, e, el, ea, B, out, idx=None, node_off=None, edge_off=None, xc=None, widths=None, x=None, m=None, al=None,
+                   adj_off=None):
+    """Batch B per-graph records on the device (gnnml3_collate / gnnml3_collate_graphs) into the tensors of ``out`` (a ``Batch``
+    whose ``x [Np, F]``, ``edge_index2 [2, Ep]`` int64, ``edge_attr2 [Ep, K]``, ``batch [Np]`` int64 and ``graph_ptr`` int32 are
+    preallocated; rows beyond the batch's nodes / entries get the neutral padding of a captured step).  Records: ``n`` / ``e``
+    int32 sizes, ``el [2, *]`` graph-local ids (uint8 / int16 / int32 / int64), ``ea [*, K]``, features ``x [*, F]`` or uint8
+    class codes ``xc [*, C]`` + ``widths``; ``idx`` (int64 graph ids) with ``node_off`` / ``edge_off`` (int64) select records of a
+    resident pool, None = the records are the batch itself in order.
+
+    The plain edge list (what GNNML1 reads): ``m`` int32 edges per record, ``al [2, *]`` graph-local ids (same dtypes as ``el``),
+    ``adj_off`` int64 pool offsets (with ``idx``); ``out.edge_index [2, Mp]`` int64 receives it, padded like the supports.
+    ``ea=None``: the records have no supports (``e`` / ``el`` are ignored and ``out`` needs no ``edge_index2`` / ``edge_attr2``)."""
     import ctypes
     lib = _lib.load()
-    dev = ea.device
-    if el.is_cuda and not el.is_contiguous():
+    sup, adj = ea is not None, m is not None
+    if not sup and not adj:
+        raise RuntimeError("collate_device: the records carry neither supports (ea) nor a plain edge list (m, al)")
+    dev = n.device
+    if sup and el.is_cuda and not el.is_contiguous():
         el = el.contiguous()
-    for name, t in (("n", n), ("e", e), ("el", el), ("ea", ea), ("out.x", out.x), ("out.edge_index2", out.edge_index2),
-                    ("out.edge_attr2", out.edge_attr2), ("out.batch", out.batch), ("out.graph_ptr", out.graph_ptr)):
+    if adj and al is not None and al.is_cuda and not al.is_contiguous():
+        al = al.contiguous()
+    checks = [("n", n), ("out.x", out.x), ("out.batch", out.batch), ("out.graph_ptr", out.graph_ptr)]
+    if sup:
+        checks += [("e", e), ("el", el), ("ea", ea), ("out.edge_index2", out.edge_index2), ("out.edge_attr2", out.edge_attr2)]
+    if adj:
+        if al is None or getattr(out, "edge_index", None) is None:
+            raise RuntimeError("collate_device: the plain edge list needs m, al and out.edge_index")
+        checks += [("m", m), ("al", al), ("out.edge_index", out.edge_index)]
+    for name, t in checks:
         if not t.is_cuda or not t.is_contiguous():
             raise RuntimeError("collate_device: %s must be a contiguous CUDA tensor (no CPU fallback)" % name)
-    if n.dtype != torch.int32 or e.dtype != torch.int32 or out.edge_index2.dtype != torch.int64 or out.batch.dtype != torch.int64 \
-            or out.graph_ptr.dtype != torch.int32 or ea.dtype != torch.float32 or out.x.dtype != torch.float32:
+    if n.dtype != torch.int32 or out.batch.dtype != torch.int64 or out.graph_ptr.dtype != torch.int32 or out.x.dtype != torch.float32 \
+            or (sup and (e.dtype != torch.int32 or out.edge_index2.dtype != torch.int64 or ea.dtype != torch.float32)) \
+            or (adj and (m.dtype != torch.int32 or out.edge_index.dtype != torch.int64)):
         raise RuntimeError("collate_device: unexpected dtype")
-    el_bytes = el.element_size()
-    if el.dtype not in (torch.uint8, torch.int16, torch.int32, torch.int64):
-        raise RuntimeError("collate_device: el must be uint8 / int16 / int32 / int64")
+    for t in ((el,) if sup else ()) + ((al,) if adj else ()):
+        if t.dtype not in (torch.uint8, torch.int16, torch.int32, torch.int64) or t.dim() != 2 or t.size(0) != 2:
+            raise RuntimeError("collate_device: el / al must be [2, *] uint8 / int16 / int32 / int64")
     Np, F = out.x.shape
-    Ep, K = out.edge_attr2.shape
-    if out.edge_index2.size(1) != Ep or out.batch.numel() != Np or out.graph_ptr.numel() < B + 1 or ea.size(1) != K:
+    Ep, K = out.edge_attr2.shape if sup else (0, 0)
+    Mp = out.edge_index.size(1) if adj else 0
+    if (sup and (out.edge_index2.size(1) != Ep or ea.size(1) != K)) or (adj and out.edge_index.size(0) != 2) \
+            or out.batch.numel() != Np or out.graph_ptr.numel() < B + 1:
         raise RuntimeError("collate_device: output shapes do not match")
     wh = None
     C = 0
@@ -642,15 +661,27 @@ def collate_device(n, e, el, ea, B, out, idx=None, node_off=None, edge_off=None,
             raise RuntimeError("collate_device: xc must be a contiguous uint8 tensor")
     elif x is None or x.dtype != torch.float32 or not x.is_contiguous() or x.size(1) != F:
         raise RuntimeError("collate_device: x [*, F] float32 or xc + widths must be given")
-    for t in (idx, node_off, edge_off):
+    for t in (idx, node_off, edge_off, adj_off):
         if t is not None and (t.dtype != torch.int64 or not t.is_cuda or not t.is_contiguous()):
-            raise RuntimeError("collate_device: idx / node_off / edge_off must be contiguous int64 CUDA tensors")
-    ws = _ws(dev, lib.gnnml3_collate_workspace_bytes(int(B)), tag="collate")
+            raise RuntimeError("collate_device: idx / node_off / edge_off / adj_off must be contiguous int64 CUDA tensors")
+    P = _lib.ptr
+    if sup and not adj:
+        ws = _ws(dev, lib.gnnml3_collate_workspace_bytes(int(B)), tag="collate")
+        with _on(dev):
+            _lib.check(lib.gnnml3_collate(P(idx), P(n), P(e), P(node_off), P(edge_off), P(xc), C, wh, P(x), F, P(el),
+                                          el.element_size(), el.size(1), P(ea), K, int(B), Np, Ep, P(out.x), P(out.edge_index2),
+                                          P(out.edge_attr2), P(out.batch), P(out.graph_ptr), P(ws), ws.numel(), _lib.stream_ptr()),
+                       "gnnml3_collate")
+        return out
+    ws = _ws(dev, lib.gnnml3_collate_graphs_workspace_bytes(int(B)), tag="collate")
     with _on(dev):
-        _lib.check(lib.gnnml3_collate(_lib.ptr(idx), _lib.ptr(n), _lib.ptr(e), _lib.ptr(node_off), _lib.ptr(edge_off), _lib.ptr(xc), C,
-                                      wh, _lib.ptr(x), F, _lib.ptr(el), el_bytes, el.size(1), _lib.ptr(ea), K, int(B), Np, Ep,
-                                      _lib.ptr(out.x), _lib.ptr(out.edge_index2), _lib.ptr(out.edge_attr2), _lib.ptr(out.batch),
-                                      _lib.ptr(out.graph_ptr), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "gnnml3_collate")
+        _lib.check(lib.gnnml3_collate_graphs(
+            P(idx), P(n), P(node_off), P(xc), C, wh, P(x), F, P(e) if sup else None, P(edge_off) if sup else None,
+            P(el) if sup else None, el.element_size() if sup else 0, el.size(1) if sup else 0, P(ea), K, P(m),
+            P(adj_off) if adj else None, P(al) if adj else None, al.element_size() if adj else 0, al.size(1) if adj else 0, int(B),
+            Np, Ep, Mp, P(out.x), P(out.edge_index2) if sup else None, P(out.edge_attr2) if sup else None,
+            P(out.edge_index) if adj else None, P(out.batch), P(out.graph_ptr), P(ws), ws.numel(), _lib.stream_ptr()),
+            "gnnml3_collate_graphs")
     return out
 
 

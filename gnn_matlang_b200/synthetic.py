@@ -175,7 +175,9 @@ class GraphPool(object):
         idx = rng.integers(0, len(self.n), B)
         return self.collate(idx)
 
-    def collate(self, idx):
+    def collate(self, idx, adjacency=False):
+        """Host ``Batch`` of the pool's graphs ``idx`` (same result as ``batch.collate`` on the records).  ``adjacency=True``:
+        the batch also carries the graphs' plain ``edge_index`` (what GNNML1 reads), as ``batch.collate(..., adjacency=True)``."""
         idx = np.asarray(idx)
         n, e = self.n[idx], self.e[idx]
         goff = np.concatenate([[0], np.cumsum(n)])
@@ -187,8 +189,14 @@ class GraphPool(object):
         ei = torch.from_numpy(self.ei2[:, esel] + np.repeat(goff[:-1], e)[None, :])
         ea = torch.from_numpy(self.ea2[esel])
         batch = torch.from_numpy(np.repeat(np.arange(len(idx), dtype=np.int64), n))
-        return Batch(x=x, edge_index2=ei, edge_attr2=ea, batch=batch, num_graphs=len(idx),
-                     graph_ptr=torch.from_numpy(goff.astype(np.int32)), y=torch.from_numpy(self.y[idx]).reshape(-1, 1))
+        out = Batch(x=x, edge_index2=ei, edge_attr2=ea, batch=batch, num_graphs=len(idx),
+                    graph_ptr=torch.from_numpy(goff.astype(np.int32)), y=torch.from_numpy(self.y[idx]).reshape(-1, 1))
+        if adjacency:
+            m = self.e1[idx]
+            moff = np.concatenate([[0], np.cumsum(m)])
+            msel = np.repeat(self.edge_off1[idx] - moff[:-1], m) + np.arange(moff[-1])
+            out.edge_index = torch.from_numpy(self.ei1[:, msel] + np.repeat(goff[:-1], m)[None, :])
+        return out
 
 
 class ExpPool(object):
@@ -267,24 +275,77 @@ def design_raw(raw, sd, device):
     return dict(design=out, x=x.contiguous(), n32=(npd[1:] - npd[:-1]).to(torch.int32), num_graphs=int(npd.numel() - 1), y=raw["y"])
 
 
+def _id_dtype(nmax):
+    """Smallest integer dtype of graph-local node ids (the kernel reads uint8 / int16 / int32 / int64)."""
+    return np.uint8 if nmax <= 256 else np.int16 if nmax <= 32768 else np.int32
+
+
 class DeviceDataset(object):
     """A ``GraphPool`` resident in HBM + collation ON THE DEVICE (SURVEY.md 8f rank 1): the reference keeps its
     ``InMemoryDataset`` in host memory, collates every batch on the host and copies all attributes host -> device each step
     (Zinc12k.py:20-22, :360).  Here the per-graph records (features, graph-local support coordinates, supports, labels) are
     uploaded once; a step's only host -> device traffic is the list of graph ids, and ``collate`` builds the reference's batch
-    attributes with a handful of index kernels -- bit-exact with ``GraphPool.collate`` / ``batch.collate`` (tested)."""
+    attributes with a handful of index kernels -- bit-exact with ``GraphPool.collate`` / ``batch.collate`` (tested).
 
-    def __init__(self, pool, device):
+    ``adjacency=True`` also keeps the graphs' plain edge lists (graph-local ids, smallest integer dtype) and batches fill
+    ``edge_index`` (what GNNML1 reads); ``supports=False`` leaves the support lists out (GNNML1 needs no SpectralDesign), and
+    batches then carry no ``edge_index2`` / ``edge_attr2``."""
+
+    def __init__(self, pool, device, adjacency=False, supports=True):
+        if not adjacency and not supports:
+            raise ValueError("DeviceDataset: keep the supports, the plain edge lists or both")
         self.device = device
-        self.n_h, self.e_h = pool.n, pool.e                      # host copies: batch sizes are known without a device round trip
+        self.n_h = pool.n                                        # host copies: batch sizes are known without a device round trip
         t = lambda a, dt=None: torch.as_tensor(a if dt is None else a.astype(dt)).to(device)
-        self.n, self.e = t(pool.n), t(pool.e)
-        self.n32, self.e32 = self.n.to(torch.int32), self.e.to(torch.int32)
-        self.node_off, self.edge_off = t(pool.node_off), t(pool.edge_off)
+        self.n = t(pool.n)
+        self.n32 = self.n.to(torch.int32)
+        self.node_off = t(pool.node_off)
         self.x = t(pool.x)
-        self.el = t(pool.ei2)                                    # support coordinates, node ids local to their graph
-        self.ea = t(pool.ea2)
         self.y = t(pool.y)
+        self.e_h = self.e = self.e32 = self.edge_off = self.el = self.ea = None
+        if supports:
+            self.e_h = pool.e
+            self.e = t(pool.e)
+            self.e32 = self.e.to(torch.int32)
+            self.edge_off = t(pool.edge_off)
+            self.el = t(pool.ei2)                                # support coordinates, node ids local to their graph
+            self.ea = t(pool.ea2)
+        self.m_h = self.m32 = self.adj_off = self.al = None
+        if adjacency:
+            self.m_h = pool.e1
+            self.m32 = t(pool.e1, np.int32)
+            self.adj_off = t(pool.edge_off1)
+            self.al = t(np.ascontiguousarray(pool.ei1), _id_dtype(int(pool.n.max()) if len(pool.n) else 0))
+
+    @classmethod
+    def from_graphs(cls, records, device):
+        """Resident dataset straight from per-graph records ``dict(x [n, F], edge_index [2, m] graph-local, y)`` -- what
+        ``datasets.read_graph6``, ``read_exp_pickle`` and ``read_mat`` return: the plain edge lists only (GNNML1), batches
+        carry ``x`` (float32), ``edge_index``, ``batch``, ``graph_ptr`` and ``y`` as ``batch.collate(records, adjacency=True)``."""
+        self = cls.__new__(cls)
+        self.device = device
+        def get(g, k):
+            return g.get(k) if isinstance(g, dict) else getattr(g, k, None)
+        xs = [np.asarray(get(g, "x"), dtype=np.float32).reshape(np.shape(get(g, "x"))[0], -1) for g in records]
+        eis = [np.asarray(get(g, "edge_index"), dtype=np.int64).reshape(2, -1) for g in records]
+        self.n_h = np.array([x.shape[0] for x in xs], dtype=np.int64)
+        self.m_h = np.array([ei.shape[1] for ei in eis], dtype=np.int64)
+        for ei, n in zip(eis, self.n_h):
+            if ei.size and (ei.min() < 0 or ei.max() >= n):
+                raise ValueError("DeviceDataset.from_graphs: edge_index holds ids outside its graph")
+        t = lambda a: torch.as_tensor(a).to(device)
+        self.n = t(self.n_h)
+        self.n32 = self.n.to(torch.int32)
+        self.node_off = t(np.concatenate([[0], np.cumsum(self.n_h)]).astype(np.int64))
+        self.x = t(np.concatenate(xs, 0))
+        self.m32 = t(self.m_h.astype(np.int32))
+        self.adj_off = t(np.concatenate([[0], np.cumsum(self.m_h)]).astype(np.int64))
+        dt = _id_dtype(int(self.n_h.max()) if len(self.n_h) else 0)
+        self.al = t(np.ascontiguousarray(np.concatenate(eis, 1).astype(dt)))
+        ys = [torch.as_tensor(get(g, "y")) for g in records]         # batch.collate's label layout: one row per graph
+        self.y = t(torch.cat([y.reshape(1, -1) if y.dim() < 2 else y for y in ys], 0))
+        self.e_h = self.e = self.e32 = self.edge_off = self.el = self.ea = None
+        return self
 
     @classmethod
     def from_design(cls, design, node_ptr, x, y=None):
@@ -305,6 +366,7 @@ class DeviceDataset(object):
         self.ea = design["edge_attr2"].contiguous()
         B = self.n.numel()
         self.y = (torch.zeros(B, device=dev) if y is None else torch.as_tensor(y).to(dev)).reshape(B, -1)
+        self.m_h = self.m32 = self.adj_off = self.al = None
         return self
 
     def _idx(self, idx_host):
@@ -313,13 +375,30 @@ class DeviceDataset(object):
             self.device, non_blocking=True).long()
         return idx_np, idx
 
+    def _collate(self, idx, idx_np, out):
+        from . import ops
+        B = idx.numel()
+        adj = self.al is not None and getattr(out, "edge_index", None) is not None
+        if self.ea is None and not adj:
+            raise ValueError("DeviceDataset: the output batch has no edge_index and the dataset keeps no supports")
+        N = int(self.n_h[idx_np].sum())
+        E = int(self.e_h[idx_np].sum()) if self.ea is not None else 0
+        M = int(self.m_h[idx_np].sum()) if adj else 0
+        Np, Ep, Mp = out.x.size(0), (out.edge_index2.size(1) if self.ea is not None else 0), (out.edge_index.size(1) if adj else 0)
+        if N > Np or E > Ep or M > Mp or (Np == N and (Ep > E or Mp > M)):
+            raise ValueError("DeviceDataset: the batch (%d nodes, %d entries, %d edges) does not fit the output (%d, %d, %d; padding "
+                             "needs at least one dummy node)" % (N, E, M, Np, Ep, Mp))
+        kw = dict(m=self.m32, al=self.al, adj_off=self.adj_off) if adj else {}
+        ops.collate_device(self.n32, self.e32, self.el, self.ea, B, out, idx=idx, node_off=self.node_off, edge_off=self.edge_off,
+                           x=self.x, **kw)
+        return out
+
     def collate_into(self, idx_host, out):
         """Graph ids (int64 numpy array or pinned CPU tensor) -> the preallocated device ``Batch`` ``out`` (larger tensors get the
-        neutral padding of ``train.pad_batch``): ONE host -> device copy of the id list and two library launches."""
-        from . import ops
-        _, idx = self._idx(idx_host)
-        ops.collate_device(self.n32, self.e32, self.el, self.ea, idx.numel(), out, idx=idx, node_off=self.node_off, edge_off=self.edge_off,
-                           x=self.x)
+        neutral padding of ``train.pad_batch``; ``out.edge_index`` is filled when the dataset keeps the plain lists): ONE host ->
+        device copy of the id list and two library launches."""
+        idx_np, idx = self._idx(idx_host)
+        self._collate(idx, idx_np, out)
         if getattr(out, "y", None) is not None:
             out.y.copy_(self.y[idx].reshape(out.y.shape))
         return out
@@ -327,14 +406,20 @@ class DeviceDataset(object):
     def collate(self, idx_host):
         """``idx_host``: int64/int32 numpy array or pinned CPU tensor of graph ids -> device ``Batch`` (exact sizes)."""
         idx_np, idx = self._idx(idx_host)
-        N, E = int(self.n_h[idx_np].sum()), int(self.e_h[idx_np].sum())
+        N = int(self.n_h[idx_np].sum())
         dev = self.device
         B = idx.numel()
-        out = Batch(x=torch.empty(N, self.x.size(1), dtype=torch.float32, device=dev), edge_index2=torch.empty(2, E, dtype=torch.int64, device=dev),
-                    edge_attr2=torch.empty(E, self.ea.size(1), dtype=torch.float32, device=dev), batch=torch.empty(N, dtype=torch.int64, device=dev),
-                    graph_ptr=torch.empty(B + 1, dtype=torch.int32, device=dev), num_graphs=B)
-        from . import ops
-        ops.collate_device(self.n32, self.e32, self.el, self.ea, B, out, idx=idx, node_off=self.node_off, edge_off=self.edge_off, x=self.x)
-        out.y = self.y[idx].reshape(-1, 1)
+        out = Batch(x=torch.empty(N, self.x.size(1), dtype=torch.float32, device=dev))
+        if self.ea is not None:
+            E = int(self.e_h[idx_np].sum())
+            out.edge_index2 = torch.empty(2, E, dtype=torch.int64, device=dev)
+            out.edge_attr2 = torch.empty(E, self.ea.size(1), dtype=torch.float32, device=dev)
+        out.batch = torch.empty(N, dtype=torch.int64, device=dev)
+        out.graph_ptr = torch.empty(B + 1, dtype=torch.int32, device=dev)
+        out.num_graphs = B
+        if self.al is not None:
+            out.edge_index = torch.empty(2, int(self.m_h[idx_np].sum()), dtype=torch.int64, device=dev)
+        self._collate(idx, idx_np, out)
+        out.y = self.y[idx].reshape(B, -1)
         out.batch._gnnml3_ptr = (out.batch._version, out.graph_ptr)
         return out

@@ -167,40 +167,88 @@ class DesignFeeder(object):
         return b
 
 
-def pad_batch(hb, n_nodes, n_entries):
+def _pad_loops(N, n_nodes, first, total):
+    """[2, total - first] self-loops spread round-robin over the dummy nodes N .. n_nodes - 1."""
+    return (N + torch.arange(total - first) % (n_nodes - N)).unsqueeze(0).expand(2, -1)
+
+
+def pad_batch(hb, n_nodes, n_entries=None, n_edges=None):
     """Host ``Batch`` -> the same batch padded to ``n_nodes`` nodes and ``n_entries`` support entries (static shapes for CUDA
     graph replay).  The padding is exactly neutral: the extra nodes are isolated, carry zero features and form ONE extra
     (dummy) graph at the end whose read-out row the loss never sees (``GraphedTrainer`` slices it off); the extra entries are
     self-loops spread round-robin over the dummy nodes with all-zero supports (a bias-free edge MLP maps them to zero, they
     add 0 to those nodes and receive zero gradients).  ``n_nodes`` must exceed the batch's node count (the dummy graph is
     never empty); ``padded_shapes`` picks shapes that keep the dummy nodes' degree small (a hub row would serialise the
-    row-parallel kernels)."""
+    row-parallel kernels).
+
+    ``n_edges``: the batch's plain ``edge_index`` (``collate(..., adjacency=True)``, what GNNML1 reads) is padded to
+    ``n_edges`` columns with the same round-robin self-loops on the dummy nodes; a batch without supports passes
+    ``n_entries=None``.  Without ``n_edges`` the result has no ``edge_index``.  GNNML1 has no edge weights, so these self-loops
+    DO add a dummy node's features to itself -- still neutral for the real graphs and for training:
+
+    * no edge joins a dummy node to a real one, so the dummy nodes form one extra graph whose activations never reach a real
+      node's;
+    * that graph's read-out row is sliced off before the loss (``out[:real]``), so the gradient of every dummy row is exactly
+      zero at every layer, and so is the dummy rows' contribution to the weight and bias gradients;
+    * this holds while the dummy activations stay finite (0 * inf is NaN): the round-robin spread keeps each dummy node's
+      self-loop count at most ``max_pad_degree`` of ``padded_shapes``, i.e. in the range of a real node's degree."""
     import numpy as np
     from .batch import Batch
-    N, E = hb.x.size(0), hb.edge_index2.size(1)
-    if n_nodes <= N or n_entries < E:
-        raise ValueError("pad_batch: need n_nodes > %d and n_entries >= %d" % (N, E))
+    sup = getattr(hb, "edge_index2", None) is not None
+    N = hb.x.size(0)
+    E = hb.edge_index2.size(1) if sup else 0
+    if sup and n_entries is None:
+        raise ValueError("pad_batch: the batch has supports: give n_entries")
+    if n_edges is not None and getattr(hb, "edge_index", None) is None:
+        raise ValueError("pad_batch: n_edges given but the batch has no edge_index")
+    M = hb.edge_index.size(1) if n_edges is not None else 0
+    if n_nodes <= N or (sup and n_entries < E) or (n_edges is not None and n_edges < M):
+        raise ValueError("pad_batch: need n_nodes > %d, n_entries >= %d and n_edges >= %d" % (N, E, M))
     B = hb.num_graphs
     x = torch.zeros(n_nodes, hb.x.size(1), dtype=hb.x.dtype)
     x[:N] = hb.x
-    ei = torch.empty((2, n_entries), dtype=torch.int64)
-    ei[:, :E] = hb.edge_index2
-    ei[:, E:] = (N + torch.arange(n_entries - E) % (n_nodes - N)).unsqueeze(0)
-    ea = torch.zeros(n_entries, hb.edge_attr2.size(1), dtype=hb.edge_attr2.dtype)
-    ea[:E] = hb.edge_attr2
+    kw = dict(x=x)
+    if sup:
+        ei = torch.empty((2, n_entries), dtype=torch.int64)
+        ei[:, :E] = hb.edge_index2
+        ei[:, E:] = _pad_loops(N, n_nodes, E, n_entries)
+        ea = torch.zeros(n_entries, hb.edge_attr2.size(1), dtype=hb.edge_attr2.dtype)
+        ea[:E] = hb.edge_attr2
+        kw.update(edge_index2=ei, edge_attr2=ea)
     batch = torch.full((n_nodes,), B, dtype=torch.int64)
     batch[:N] = hb.batch
     gp = torch.cat([hb.graph_ptr.to(torch.int32), torch.tensor([n_nodes], dtype=torch.int32)])
-    return Batch(x=x, edge_index2=ei, edge_attr2=ea, batch=batch, num_graphs=B + 1, graph_ptr=gp, y=hb.y, real_graphs=B)
+    out = Batch(**kw, batch=batch, num_graphs=B + 1, graph_ptr=gp, y=hb.y, real_graphs=B)
+    if n_edges is not None:
+        adj = torch.empty((2, n_edges), dtype=torch.int64)
+        adj[:, :M] = hb.edge_index
+        adj[:, M:] = _pad_loops(N, n_nodes, M, n_edges)
+        out.edge_index = adj
+    return out
 
 
-def padded_shapes(batches, max_pad_degree=8):
+def padded_shapes(batches, max_pad_degree=8, adjacency=False):
     """(n_nodes, n_entries) for ``pad_batch`` / ``GraphedTrainer`` covering every batch of the list: the largest entry count,
-    and enough dummy nodes that the padding self-loops of the SMALLEST batch give no dummy node more than ``max_pad_degree``."""
+    and enough dummy nodes that the padding self-loops of the SMALLEST batch give no dummy node more than ``max_pad_degree``.
+
+    ``adjacency=True``: (n_nodes, n_entries, n_edges), sizing the plain ``edge_index`` as well (``n_entries`` is None for batches
+    without supports); the dummy nodes then bound the self-loops a dummy node receives from BOTH lists together."""
     nmax = max(int(b.x.shape[0]) for b in batches)
-    emax = max(int(b.edge_index2.shape[1]) for b in batches)
-    emin = min(int(b.edge_index2.shape[1]) for b in batches)
-    return nmax + 1 + (emax - emin + max_pad_degree - 1) // max_pad_degree, emax
+    if not adjacency:
+        emax = max(int(b.edge_index2.shape[1]) for b in batches)
+        emin = min(int(b.edge_index2.shape[1]) for b in batches)
+        return nmax + 1 + (emax - emin + max_pad_degree - 1) // max_pad_degree, emax
+    sup = getattr(batches[0], "edge_index2", None) is not None
+    es = [int(b.edge_index2.shape[1]) for b in batches] if sup else [0]
+    ms = [int(b.edge_index.shape[1]) for b in batches]
+    pe, pm = max(es) - min(es), max(ms) - min(ms)             # most padding either list can need (smallest batch)
+    if pe and pm and max_pad_degree < 2:
+        raise ValueError("padded_shapes: padding both lists needs max_pad_degree >= 2")
+    # a dummy node gets ceil(pe / nd) + ceil(pm / nd) self-loops at most (both lists start the round-robin at node N)
+    nd = max(1, -(-(pe + pm) // max_pad_degree))
+    while -(-pe // nd) + -(-pm // nd) > max_pad_degree:
+        nd += 1
+    return nmax + nd, (max(es) if sup else None), max(ms)
 
 
 class GraphedTrainer(object):
@@ -221,7 +269,9 @@ class GraphedTrainer(object):
         dev = self.params[0].device
         self.static = example.to(dev, non_blocking=False) if not example.x.is_cuda else example
         self.real = int(getattr(example, "real_graphs", example.num_graphs))
-        self.fields = ("x", "edge_index2", "edge_attr2", "batch", "graph_ptr", "y")
+        # the inputs the example carries: a GNNML3 batch brings the supports, a GNNML1 batch the plain edge list
+        self.fields = tuple(k for k in ("x", "edge_index2", "edge_attr2", "edge_index", "batch", "graph_ptr", "y")
+                            if getattr(example, k, None) is not None)
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(s):
@@ -284,21 +334,29 @@ class GraphedTrainer(object):
             getattr(self.static, k).copy_(getattr(batch, k), non_blocking=True)
 
     def load_unpadded(self, b):
-        """Write a DEVICE batch of any size that fits (N < captured nodes, E <= captured entries, same number of graphs) into the
-        captured input buffers and fill the rest with the neutral padding of ``pad_batch`` (device-side, no host sync)."""
+        """Write a DEVICE batch of any size that fits (N < captured nodes, E <= captured entries, M <= captured plain edges, same
+        number of graphs) into the captured input buffers and fill the rest with the neutral padding of ``pad_batch``
+        (device-side, no host sync)."""
         st = self.static
-        N, E = b.x.size(0), b.edge_index2.size(1)
-        Np, Ep = st.x.size(0), st.edge_index2.size(1)
-        if N >= Np or E > Ep or b.num_graphs != self.real:
-            raise ValueError("batch (%d nodes, %d entries, %d graphs) does not fit the captured shapes (%d, %d, %d)"
-                             % (N, E, b.num_graphs, Np, Ep, self.real))
+        sup, adj = "edge_index2" in self.fields, "edge_index" in self.fields
+        N = b.x.size(0)
+        E, M = (b.edge_index2.size(1) if sup else 0), (b.edge_index.size(1) if adj else 0)
+        Np, Ep, Mp = st.x.size(0), (st.edge_index2.size(1) if sup else 0), (st.edge_index.size(1) if adj else 0)
+        if N >= Np or E > Ep or M > Mp or b.num_graphs != self.real:
+            raise ValueError("batch (%d nodes, %d entries, %d edges, %d graphs) does not fit the captured shapes (%d, %d, %d, %d)"
+                             % (N, E, M, b.num_graphs, Np, Ep, Mp, self.real))
         st.x[:N].copy_(b.x, non_blocking=True)
         st.x[N:].zero_()
-        st.edge_index2[:, :E].copy_(b.edge_index2, non_blocking=True)
-        if Ep > E:
-            st.edge_index2[:, E:].copy_((N + torch.arange(Ep - E, device=st.x.device) % (Np - N)).unsqueeze(0))
-        st.edge_attr2[:E].copy_(b.edge_attr2, non_blocking=True)
-        st.edge_attr2[E:].zero_()
+        if sup:
+            st.edge_index2[:, :E].copy_(b.edge_index2, non_blocking=True)
+            if Ep > E:
+                st.edge_index2[:, E:].copy_((N + torch.arange(Ep - E, device=st.x.device) % (Np - N)).unsqueeze(0))
+            st.edge_attr2[:E].copy_(b.edge_attr2, non_blocking=True)
+            st.edge_attr2[E:].zero_()
+        if adj:
+            st.edge_index[:, :M].copy_(b.edge_index, non_blocking=True)
+            if Mp > M:
+                st.edge_index[:, M:].copy_((N + torch.arange(Mp - M, device=st.x.device) % (Np - N)).unsqueeze(0))
         st.batch[:N].copy_(b.batch, non_blocking=True)
         st.batch[N:].fill_(self.real)
         st.graph_ptr[:self.real + 1].copy_(b.graph_ptr, non_blocking=True)
@@ -307,10 +365,13 @@ class GraphedTrainer(object):
 
     def load_compact(self, cb):
         """Device ``CompactBatch`` (wire format) -> the captured input buffers, padding included: two library launches
-        (``gnnml3_collate``) + the label copy, instead of ~20 index kernels of ``expand`` and ~12 copies of ``load_unpadded``."""
+        (``gnnml3_collate``, or ``gnnml3_collate_graphs`` with the plain edge list) + the label copy, instead of ~20 index kernels
+        of ``expand`` and ~12 copies of ``load_unpadded``."""
         st = self.static
-        N = (cb.xc if cb.xc is not None else cb.x).size(0)
-        if N >= st.x.size(0) or cb.el.size(1) > st.edge_index2.size(1) or cb.num_graphs != self.real:
+        N, E, M = cb.sizes()
+        sup, adj = "edge_index2" in self.fields, "edge_index" in self.fields
+        if N >= st.x.size(0) or cb.num_graphs != self.real or (E is None) == sup or (M is None and adj) \
+                or (sup and E > st.edge_index2.size(1)) or (adj and M > st.edge_index.size(1)):
             raise ValueError("batch does not fit the captured shapes")
         cb.expand_into(st)
 

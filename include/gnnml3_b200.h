@@ -344,6 +344,21 @@ GNNML3_API int gnnml3_collate(const int64_t* idx, const int32_t* n, const int32_
                    int64_t* out_edge_index, float* out_edge_attr, int64_t* out_batch, int32_t* out_graph_ptr,
                    void* workspace, size_t workspace_bytes, void* stream);
 
+/* The general form: records may carry the support list (e / edge_off / el / ea, K >= 1), the graph's plain edge list (what
+ * GNNML1 reads: m = edges per record, adj_off = first edge of a record in al, al [2, al_stride] graph-local ids in al_bytes-wide
+ * integers), or both.  K = 0 with NULL el / ea / out_edge_index2 / out_edge_attr2 (and Ep = 0): no supports.  m = NULL with NULL
+ * al / out_edge_index (and Mp = 0): no plain list.  out_edge_index [2, Mp] receives int64 global ids in record order; columns
+ * beyond the batch's edges get the same padding self-loops as the supports.  Padding a list (Ep > E or Mp > M) needs dummy
+ * nodes (Np > N): the caller checks this, the kernel writes no padding edges without them.  gnnml3_collate is this call without
+ * the plain list.  Workspace: 3 * (B + 1) int64. */
+GNNML3_API size_t gnnml3_collate_graphs_workspace_bytes(int B);
+GNNML3_API int gnnml3_collate_graphs(const int64_t* idx, const int32_t* n, const int64_t* node_off, const uint8_t* xc, int C,
+                   const int32_t* widths_host, const float* x, int F, const int32_t* e, const int64_t* edge_off, const void* el,
+                   int el_bytes, int64_t el_stride, const float* ea, int K, const int32_t* m, const int64_t* adj_off, const void* al,
+                   int al_bytes, int64_t al_stride, int B, int64_t Np, int64_t Ep, int64_t Mp, float* out_x,
+                   int64_t* out_edge_index2, float* out_edge_attr2, int64_t* out_edge_index, int64_t* out_batch,
+                   int32_t* out_graph_ptr, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -10,9 +10,15 @@
   ``torch.profiler`` pass, the device time of the fused kernel in the forward and in the dx pass, with the algorithmic bytes of
   each launch (every operand once) and their share of the 7.7 TB/s HBM3e bandwidth of one B200 (NVIDIA HGX B200 data sheet);
 * the time to embed all 11,117 graph8c graphs (one batch, eval mode);
+* the training data path (key ``train``): the same step captured in one CUDA graph (``GraphedTrainer``), each step collating a
+  new id list on the device from an HBM-resident ``DeviceDataset(supports=False)`` of ``--pool`` graphs (larger than the
+  126 MB L2); the captured step fed end to end by ``HostFeeder`` from pinned wire-format batches with the loss read back; the
+  eager step on fresh batches (so that both arms build the CSR); captured against eager at batch 64; the host's
+  ``collate(adjacency=True)`` (the feed without this data path) at both batch sizes; one ``gnnml3_collate_graphs`` call at the
+  bench batch with its algorithmic bytes;
 * the card's name and power limit, read in the same run.
 
-    python tools/bench_gnnml1.py [--batch 8192] [--steps 20] [--warmup 5] [--rounds 3] [--out FILE]
+    python tools/bench_gnnml1.py [--batch 8192] [--steps 20] [--warmup 5] [--rounds 3] [--pool 65536] [--out FILE]
 
 Nothing is written unless --out is given.
 """
@@ -96,12 +102,129 @@ def timed_steps(model, opt, b, steps):
     return start.elapsed_time(end) / steps
 
 
+def _events(fn, steps):
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record()
+    for i in range(steps):
+        fn(i)
+    e.record()
+    torch.cuda.synchronize()
+    return s.elapsed_time(e) / steps
+
+
+def _strip(hb):
+    return hb.__class__(**{k: v for k, v in hb.__dict__.items() if k not in ("edge_index2", "edge_attr2")})
+
+
+def train_path(a, d):
+    """GNNML1 training through the device data path; every arm alternates with the others in each of ``a.rounds`` rounds."""
+    import time
+    from gnn_matlang_b200 import ops
+    from gnn_matlang_b200.batch import collate
+    from gnn_matlang_b200.models import GNNML1
+    from gnn_matlang_b200.synthetic import DeviceDataset, GraphPool
+    from gnn_matlang_b200.train import GraphedTrainer, HostFeeder, Trainer, pad_batch, padded_shapes
+    out = {}
+    pool = GraphPool("zinc", a.pool, seed=11)
+    dds = DeviceDataset(pool, d, adjacency=True, supports=False)
+    out["pool_graphs"] = a.pool
+    out["pool_resident_bytes"] = int(sum(t.numel() * t.element_size() for t in (dds.x, dds.al, dds.n, dds.m32, dds.node_off,
+                                                                                 dds.adj_off, dds.y)))
+    rng = np.random.default_rng(2)
+    arms = {}
+    for B in (a.batch, 64):
+        nring = 8
+        ids = [rng.integers(0, a.pool, B) for _ in range(nring)]
+        host = [_strip(pool.collate(i, adjacency=True)) for i in ids]
+        Np, _, Mp = padded_shapes(host, adjacency=True)
+        torch.manual_seed(0)
+        gt = GraphedTrainer(GNNML1("zinc", ninp=25).to(d), pad_batch(host[0], Np, None, Mp), loss="l1")
+        pinned = [torch.from_numpy(i).pin_memory() for i in ids]
+        torch.manual_seed(0)
+        eager_model = GNNML1("zinc", ninp=25).to(d)
+        eager = Trainer(eager_model, loss="l1")
+        dev_batches = [hb.to(d) for hb in host]
+        arms["captured_b%d" % B] = lambda i, gt=gt, pinned=pinned: (gt.load_from_dataset(dds, pinned[i % len(pinned)]), gt.step())
+        arms["eager_b%d" % B] = lambda i, eager=eager, dev_batches=dev_batches: eager.step(dev_batches[i % len(dev_batches)].fresh())
+        if B == a.batch:
+            feeder = HostFeeder(d, onehot_widths=(21, 4))
+            out["wire_bytes_per_step"] = int(np.mean([feeder.bytes_per_batch(hb) for hb in host]))
+            out["host_batch_bytes_per_step"] = int(np.mean([hb.nbytes() for hb in host]))
+            state = {"k": 0}
+            feeder.prefetch(host[0])
+
+            def e2e(i, gt=gt, feeder=feeder, host=host, state=state):
+                cb = feeder.get_compact()
+                state["k"] += 1
+                feeder.prefetch(host[state["k"] % len(host)])
+                gt.load_compact(cb)
+                state["loss"] = float(gt.step())             # the loss read back every step
+            arms["end_to_end_b%d" % B] = e2e
+            # one collation call into the captured buffers
+            st = gt.static
+            ix = torch.from_numpy(ids[0]).to(d)
+            Nb, Mb = int(pool.n[ids[0]].sum()), int(pool.e1[ids[0]].sum())
+            call = lambda i, ix=ix, st=st: ops.collate_device(dds.n32, None, None, None, B, st, idx=ix, node_off=dds.node_off, x=dds.x,  # noqa: E731
+                                                              m=dds.m32, al=dds.al, adj_off=dds.adj_off)
+            F = dds.x.size(1)
+            coll_bytes = (B * (8 + 4 + 4 + 8 + 8)                          # ids; n, m; node and edge offsets
+                          + 2 * Nb * F * 4 + Nb * 8                         # features in and out; batch vector
+                          + Mb * 2 * dds.al.element_size() + Mb * 16        # local ids in, int64 global ids out
+                          + (Np - Nb) * (F * 4 + 8) + (Mp - Mb) * 16        # padding
+                          + (B + 2) * 4 + 2 * 3 * (B + 1) * 8)              # graph_ptr; the three scans written and read
+            out["collate_kernel"] = dict(graphs=B, nodes=Nb, edges=Mb, padded_nodes=Np, padded_edges=Mp, bytes=coll_bytes)
+            arms["collate_call_b%d" % B] = call
+    for name, fn in arms.items():                                          # warm-up of every arm and shape
+        for i in range(a.warmup):
+            fn(i)
+    torch.cuda.synchronize()
+    times = {k: [] for k in arms}
+    for _ in range(a.rounds):
+        for name, fn in arms.items():
+            times[name].append(_events(fn, a.steps if not name.startswith("collate") else 50))
+    out["ms_per_step"] = times
+    best = {k: min(v) for k, v in times.items()}
+    Bb = a.batch
+    out["graphs_per_s_captured"] = Bb / (best["captured_b%d" % Bb] * 1e-3)
+    out["graphs_per_s_end_to_end"] = Bb / (best["end_to_end_b%d" % Bb] * 1e-3)
+    out["graphs_per_s_eager_fresh"] = Bb / (best["eager_b%d" % Bb] * 1e-3)
+    out["end_to_end_over_captured"] = best["end_to_end_b%d" % Bb] / best["captured_b%d" % Bb]
+    out["captured_speedup_vs_eager_fresh"] = best["eager_b%d" % Bb] / best["captured_b%d" % Bb]
+    out["captured_speedup_vs_eager_b64"] = best["eager_b64"] / best["captured_b64"]
+    ck = out["collate_kernel"]
+    ck["call_ms"] = best["collate_call_b%d" % Bb]
+    ck["hbm_share"] = ck["bytes"] / (ck["call_ms"] * 1e-3) / HBM_PEAK
+    ck["bytes_rule"] = "every operand once: ids, sizes, offsets, features in and out, local ids in, global ids out, padding, scans"
+    # the feed without this data path: host collation of the records (one process, this host)
+    rec_rng = np.random.default_rng(0)
+    recs = []
+    for _ in range(Bb):
+        from gnn_matlang_b200.synthetic import zinc_graph
+        n, ei, x = zinc_graph(rec_rng)
+        recs.append(dict(x=x, edge_index=ei, y=np.float32(rec_rng.standard_normal())))
+    hc = {}
+    for B, reps in ((Bb, 3), (64, 100)):
+        sub = recs[:B]
+        collate(sub, adjacency=True)
+        t0 = time.perf_counter()
+        for _ in range(reps):
+            collate(sub, adjacency=True)
+        hc["b%d_ms" % B] = (time.perf_counter() - t0) / reps * 1e3
+    hc["host_cpus"] = os.cpu_count()
+    out["host_collate_adjacency"] = hc
+    out["note"] = ("captured: load_from_dataset (id list H2D + gnnml3_collate_graphs) + graph replay; end_to_end: HostFeeder H2D of "
+                   "the wire format + load_compact + replay + loss read back; eager: Trainer.step on a fresh device batch (CSR build "
+                   "included); ms_per_step lists one value per round, arms alternate within every round")
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=8192)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--pool", type=int, default=65536)
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -215,6 +338,7 @@ def main():
     with torch.no_grad():
         res["graph8c_graphs"] = len(gs)
         res["graph8c_embed_ms"] = ev(lambda: m8(g8), reps=20)
+    res["train"] = train_path(a, d)
     line = json.dumps(res)
     print(line)
     if a.out:
