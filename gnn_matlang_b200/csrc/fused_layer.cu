@@ -148,7 +148,8 @@ __device__ __forceinline__ float lds32(uint32_t a) {
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-template <int KT, int BNH, int NAGG, bool RES>
+// AUX = false: the forward-only instantiation of the gated epilogue (aux == NULL), which stores y and not the tanh factors.
+template <int KT, int BNH, int NAGG, bool RES, bool AUX = true>
 __global__ void __launch_bounds__(32 * (FL_CTRL_WARPS + NAGG), 1)
 k_fused_agg_proj(const __grid_constant__ CUtensorMap mapW, const __grid_constant__ FLParams P) {
     constexpr int ROWS = 8 * NAGG;                      // dst rows per tile
@@ -386,8 +387,10 @@ k_fused_agg_proj(const __grid_constant__ CUtensorMap mapW, const __grid_constant
                             }
                             const float t1 = tanh_fast(p1), t2 = tanh_fast(p2);
                             orow[Fo + j] = t1 * t2;
-                            ax[j] = t1;
-                            ax[G + j] = t2;
+                            if constexpr (AUX) {
+                                ax[j] = t1;
+                                ax[G + j] = t2;
+                            }
                         }
                     }
                 }
@@ -911,11 +914,11 @@ extern "C" int gnnml3_fused_profile_fetch(double* out, int max) {
     return n;
 }
 
-template <int KT, int BNH, int NAGG, bool RES>
+template <int KT, int BNH, int NAGG, bool RES, bool AUX>
 static int fl_launch2(const CUtensorMap& mW, FLParams& P, size_t smem, cudaStream_t st) {
     static bool configured[64] = {};
     if (auto once_ = first_use_on_device(configured))
-        GNNML3_CUDA(cudaFuncSetAttribute(k_fused_agg_proj<KT, BNH, NAGG, RES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        GNNML3_CUDA(cudaFuncSetAttribute(k_fused_agg_proj<KT, BNH, NAGG, RES, AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)FL_SMEM_MAX));
     const int grid = P.n_tiles < kNumSMs ? P.n_tiles : kNumSMs;
     FLProfRec rec;
@@ -927,7 +930,7 @@ static int fl_launch2(const CUtensorMap& mW, FLParams& P, size_t smem, cudaStrea
         for (int i = 0; i < 9; ++i) rec.meta[i] = m[i];
         cudaEventRecord(rec.a, st);
     }
-    k_fused_agg_proj<KT, BNH, NAGG, RES><<<grid, 32 * (FL_CTRL_WARPS + NAGG), smem, st>>>(mW, P);
+    k_fused_agg_proj<KT, BNH, NAGG, RES, AUX><<<grid, 32 * (FL_CTRL_WARPS + NAGG), smem, st>>>(mW, P);
     if (g_fl_prof_on) {
         cudaEventRecord(rec.b, st);
         g_fl_prof.push_back(rec);
@@ -973,7 +976,7 @@ static const size_t g_fl_max_stages = [] {
 // Shared-memory plan.  Preferred: per-warp prefetch slots (64 edges each) + as many H-plane stages as fit, weight planes
 // resident if there is still room for 3 stages, otherwise streamed from L2 into the stages.  Without slots (wide feature
 // blocks, odd edge-weight strides): resident weights when 3 stages fit beside them, else streamed.
-template <int KT, int BNH, int NAGG>
+template <int KT, int BNH, int NAGG, bool AUX = true>
 static int fl_launch(const CUtensorMap& mW, FLParams& P, cudaStream_t st) {
     constexpr int ROWS = 8 * NAGG;
     constexpr size_t HP = 2 * ROWS * 128, WPLANE = 2 * BNH * 128;
@@ -991,7 +994,7 @@ static int fl_launch(const CUtensorMap& mW, FLParams& P, cudaStream_t st) {
         if (ns > g_fl_max_stages) ns = g_fl_max_stages;
             P.nstages = (int)ns;
             P.slot_cap = (int)slot_cap;
-            return fl_launch2<KT, BNH, NAGG, true>(mW, P, resident + ns * HP + FL_SMEM_FIXED + slots, st);
+            return fl_launch2<KT, BNH, NAGG, true, AUX>(mW, P, resident + ns * HP + FL_SMEM_FIXED + slots, st);
         }
         if (slots + 2 * (HP + WPLANE) + FL_SMEM_FIXED <= FL_SMEM_MAX) {
             size_t ns = (FL_SMEM_MAX - FL_SMEM_FIXED - slots) / (HP + WPLANE);
@@ -999,7 +1002,7 @@ static int fl_launch(const CUtensorMap& mW, FLParams& P, cudaStream_t st) {
         if (ns > g_fl_max_stages) ns = g_fl_max_stages;
             P.nstages = (int)ns;
             P.slot_cap = (int)slot_cap;
-            return fl_launch2<KT, BNH, NAGG, false>(mW, P, ns * (HP + WPLANE) + FL_SMEM_FIXED + slots, st);
+            return fl_launch2<KT, BNH, NAGG, false, AUX>(mW, P, ns * (HP + WPLANE) + FL_SMEM_FIXED + slots, st);
         }
     }
     if (resident + 3 * HP + FL_SMEM_FIXED <= FL_SMEM_MAX) {
@@ -1007,13 +1010,13 @@ static int fl_launch(const CUtensorMap& mW, FLParams& P, cudaStream_t st) {
         if (ns > FL_MAX_STAGES) ns = FL_MAX_STAGES;
         if (ns > g_fl_max_stages) ns = g_fl_max_stages;
         P.nstages = (int)ns;
-        return fl_launch2<KT, BNH, NAGG, true>(mW, P, resident + ns * HP + FL_SMEM_FIXED, st);
+        return fl_launch2<KT, BNH, NAGG, true, AUX>(mW, P, resident + ns * HP + FL_SMEM_FIXED, st);
     }
     size_t ns = (FL_SMEM_MAX - FL_SMEM_FIXED) / (HP + WPLANE);
     if (ns > FL_MAX_STAGES) ns = FL_MAX_STAGES;
         if (ns > g_fl_max_stages) ns = g_fl_max_stages;
     P.nstages = (int)ns;
-    return fl_launch2<KT, BNH, NAGG, false>(mW, P, ns * (HP + WPLANE) + FL_SMEM_FIXED, st);
+    return fl_launch2<KT, BNH, NAGG, false, AUX>(mW, P, ns * (HP + WPLANE) + FL_SMEM_FIXED, st);
 }
 
 // aggregator warps per CTA by register need: KT x 8 accumulators per lane.  512 threads leave 128 registers per thread
@@ -1031,13 +1034,13 @@ static const bool g_fl_wide = [] {
     return e && e[0] == '1';
 }();
 
-#define FL_DISPATCH_KT(KTV, BNV)                                                                      \
+#define FL_DISPATCH_KT(KTV, BNV, AUXV)                                                                \
     switch (KTV) {                                                                                    \
-        case 4: return (K == 8 && !g_fl_wide) ? fl_launch<4, BNV, 10>(mW, P, st) : fl_launch<4, BNV, 14>(mW, P, st); \
-        case 5: return fl_launch<5, BNV, 14>(mW, P, st);                                              \
-        case 6: return fl_launch<6, BNV, 14>(mW, P, st);                                              \
-        case 7: return fl_launch<7, BNV, 10>(mW, P, st);                                              \
-        case 8: return fl_launch<8, BNV, 10>(mW, P, st);                                              \
+        case 4: return (K == 8 && !g_fl_wide) ? fl_launch<4, BNV, 10, AUXV>(mW, P, st) : fl_launch<4, BNV, 14, AUXV>(mW, P, st); \
+        case 5: return fl_launch<5, BNV, 14, AUXV>(mW, P, st);                                        \
+        case 6: return fl_launch<6, BNV, 14, AUXV>(mW, P, st);                                        \
+        case 7: return fl_launch<7, BNV, 10, AUXV>(mW, P, st);                                        \
+        case 8: return fl_launch<8, BNV, 10, AUXV>(mW, P, st);                                        \
         default: return set_err(GNNML3_ERR_INVALID, "fused_agg_proj: no kernel for K tile %d", KTV);  \
     }
 
@@ -1062,8 +1065,8 @@ extern "C" int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
     GNNML3_REQUIRE(prec_bits == 0 || prec_bits == 0x100 || prec_bits == 0x200, "fused_agg_proj: unknown precision flag");
     GNNML3_REQUIRE(prec_bits == 0 || (gnnml3_fused_ts_supported(K, Kstride, F, Nc, Fs, self_mode, Ns) && g_fl_slot_mode == 0),
                    "fused_agg_proj: the single-pass TF32 / BF16 modes exist in the tensor-memory kernel only (F <= 32, even K)");
-    GNNML3_REQUIRE(self_mode != 1 || (epilogue == 1 && aux && G >= 1 && G <= 16 && Ns == 2 * G),
-                   "fused_agg_proj: gate columns need the ML3 epilogue, aux and Ns == 2G <= 32");
+    GNNML3_REQUIRE(self_mode != 1 || (epilogue == 1 && G >= 1 && G <= 16 && Ns == 2 * G),
+                   "fused_agg_proj: gate columns need the ML3 epilogue and Ns == 2G <= 32");
     GNNML3_REQUIRE(ldo >= Nc + (self_mode == 1 ? G : 0), "fused_agg_proj: ldo too small");
     GNNML3_REQUIRE(hout == nullptr || (ldh % 4 == 0 && (uintptr_t)hout % 16 == 0 && g_fl_slot_mode == 0 &&
                                        ldh >= (int64_t)(K + (self_mode != 0 ? 1 : 0)) * 32 * cdiv(F, 32)),
@@ -1123,10 +1126,13 @@ extern "C" int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
     P.epi = epilogue;
     P.hout = hout; P.ldh = ldh;
     P.dbg = g_fl_dbg;
+    // gated epilogue without aux (inference): the forward-only instantiations; gates exist with BNH == 32 only
+    const bool fwd_only = self_mode == 1 && !aux;
     if (g_fl_nagg16 && K == 8 && Kstride % 4 == 0 && g_fl_no_slot) {     // 16 aggregator warps, 4 supports per pass, 128-row tiles
-        if (BNH == 32) return fl_launch<4, 32, 16>(mW, P, st);
+        if (BNH == 32) return fwd_only ? fl_launch<4, 32, 16, false>(mW, P, st) : fl_launch<4, 32, 16>(mW, P, st);
         return fl_launch<4, 64, 16>(mW, P, st);
     }
-    if (BNH == 32) { FL_DISPATCH_KT(KT, 32) }
-    FL_DISPATCH_KT(KT, 64)
+    if (BNH == 32 && fwd_only) { FL_DISPATCH_KT(KT, 32, false) }
+    if (BNH == 32) { FL_DISPATCH_KT(KT, 32, true) }
+    FL_DISPATCH_KT(KT, 64, true)
 }

@@ -327,7 +327,8 @@ __host__ __device__ constexpr size_t ts_stage_bytes(int cap, int Kstride) {
 // gather the next tile's first pass.
 // Column c of a slot holds feature 16 * (c & 1) + (c >> 1) of the 32-wide block (the store layout gives a thread the even
 // or the odd columns; it gathers features 0-15 or 16-31): the weight planes are permuted the same way (k_ts_prep_weights).
-template <int KT, int BNH>
+// AUX = false: the forward-only instantiation of the gated epilogue (aux == NULL), which stores y and not the tanh factors.
+template <int KT, int BNH, bool AUX = true>
 __global__ void __launch_bounds__(TS_THREADS, 1)
 k_fused_ts(const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapX, const __grid_constant__ TSParams P) {
     constexpr int WPLANE = 2 * BNH * 128;               // bytes of one weight plane: rows [W_hi^T ; W_lo^T] x 32 k-columns
@@ -579,8 +580,10 @@ k_fused_ts(const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUt
                             const float p1 = g1h[j] + g1l[j] + sbias[64 + j], p2 = g2h[j] + g2l[j] + sbias[64 + G + j];
                             const float t1 = tanh_fast(p1), t2 = tanh_fast(p2);
                             orow[Fo + j] = t1 * t2;
-                            ax[j] = t1;
-                            ax[G + j] = t2;
+                            if constexpr (AUX) {
+                                ax[j] = t1;
+                                ax[G + j] = t2;
+                            }
                         }
                     }
                 }
@@ -997,13 +1000,13 @@ struct TSProfHook {
 };
 TSProfHook g_ts_prof = {nullptr, nullptr};
 
-template <int KT, int BNH>
+template <int KT, int BNH, bool AUX = true>
 static int ts_launch(const CUtensorMap& mW, const CUtensorMap& mX, TSParams& P, size_t smem, cudaStream_t st) {
     static bool configured[64] = {};
     if (auto once_ = first_use_on_device(configured))
-        GNNML3_CUDA(cudaFuncSetAttribute(k_fused_ts<KT, BNH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TS_SMEM_MAX));
+        GNNML3_CUDA(cudaFuncSetAttribute(k_fused_ts<KT, BNH, AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TS_SMEM_MAX));
     const int grid = P.n_tiles < kNumSMs ? P.n_tiles : kNumSMs;
-    k_fused_ts<KT, BNH><<<grid, TS_THREADS, smem, st>>>(mW, mX, P);
+    k_fused_ts<KT, BNH, AUX><<<grid, TS_THREADS, smem, st>>>(mW, mX, P);
     GNNML3_LAUNCH_CHECK();
     return GNNML3_OK;
 }
@@ -1056,6 +1059,8 @@ int fused_ts_run(const int32_t* rowptr, const int32_t* col, const int32_t* eperm
     P.hout = hout; P.ldh = ldh; P.dbg = dbg;
     P.edge_cap = tilewin ? ts_edge_cap(K, Kstride, Nc, self_mode) : 0;
     const size_t smem = ts_smem_bytes(K, Kstride, Nc, self_mode, P.edge_cap);
+    if (BNH == 32 && self_mode == 1 && !aux)      // gated epilogue without aux: the forward-only instantiation
+        return KT == 4 ? ts_launch<4, 32, false>(mW, mX, P, smem, st) : ts_launch<2, 32, false>(mW, mX, P, smem, st);
     if (BNH == 32) return KT == 4 ? ts_launch<4, 32>(mW, mX, P, smem, st) : ts_launch<2, 32>(mW, mX, P, smem, st);
     return KT == 4 ? ts_launch<4, 64>(mW, mX, P, smem, st) : ts_launch<2, 64>(mW, mX, P, smem, st);
 }

@@ -69,6 +69,8 @@ __device__ __forceinline__ float4 ml1_load4(const float* __restrict__ row, int f
 
 __device__ __forceinline__ float ml1_lo(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
 
+// AUX = false: the forward-only instantiation of the GNNML1 epilogues (aux == NULL), which stores y and not [p1 | p2].
+template <bool AUX = true>
 __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_constant__ ML1Params P) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -227,8 +229,10 @@ __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_co
                         const float q1 = p1[u] + (P.bB ? __ldg(P.bB + o) : 0.f);
                         const float q2 = p2[u] + (P.bC ? __ldg(P.bC + o) : 0.f);
                         const float ba = P.bA ? __ldg(P.bA + o) : 0.f, bc = P.bc ? __ldg(P.bc + o) : 0.f;
-                        ar[o] = q1;
-                        ar[Fo + o] = q2;
+                        if constexpr (AUX) {
+                            ar[o] = q1;
+                            ar[Fo + o] = q2;
+                        }
                         if (P.epi == 1) {
                             yr[o] = fmaxf(p0[u] + ba + bc + q1 * q2, 0.f);
                         } else {
@@ -410,13 +414,13 @@ static ML1Ws ml1_ws(int64_t N, int Fi, int Fo, int concat) {
     return w;
 }
 
-static bool g_ml1_configured[64];
-
+template <bool AUX = true>
 static int ml1_launch(const ML1Params& P, size_t smem, cudaStream_t st) {
-    if (auto once = first_use_on_device(g_ml1_configured))
-        GNNML3_CUDA(cudaFuncSetAttribute(k_ml1_agg_proj, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    static bool configured[64] = {};
+    if (auto once = first_use_on_device(configured))
+        GNNML3_CUDA(cudaFuncSetAttribute(k_ml1_agg_proj<AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     const int grid = P.n_tiles < kNumSMs ? P.n_tiles : kNumSMs;
-    k_ml1_agg_proj<<<grid, ML1_THREADS, smem, st>>>(P);
+    k_ml1_agg_proj<AUX><<<grid, ML1_THREADS, smem, st>>>(P);
     GNNML3_LAUNCH_CHECK();
     return GNNML3_OK;
 }
@@ -440,10 +444,10 @@ extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col
                                        float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh,
                                        void* workspace, size_t workspace_bytes, void* stream) {
     GNNML3_REQUIRE(gnnml3_ml1layer_supported(Fi, Fo, concat), "ml1layer_forward: unsupported shape Fi=%d Fo=%d", Fi, Fo);
-    GNNML3_REQUIRE(N >= 0 && E >= 0 && rowptr && x && wconv && wA && wB && wC && y && aux, "ml1layer_forward: NULL pointer");
+    GNNML3_REQUIRE(N >= 0 && E >= 0 && rowptr && x && wconv && wA && wB && wC && y, "ml1layer_forward: NULL pointer");
     GNNML3_REQUIRE(E == 0 || col, "ml1layer_forward: NULL col");
     GNNML3_REQUIRE(ldx >= Fi && ldx % 4 == 0 && ((uintptr_t)x & 15) == 0, "ml1layer_forward: x rows must be 16-byte aligned");
-    GNNML3_REQUIRE(ldy >= (concat ? 3 : 1) * Fo && ldaux >= 2 * Fo, "ml1layer_forward: output leading dimensions too small");
+    GNNML3_REQUIRE(ldy >= (concat ? 3 : 1) * Fo && (!aux || ldaux >= 2 * Fo), "ml1layer_forward: output leading dimensions too small");
     GNNML3_REQUIRE(hside == nullptr || (ldh >= Fi && ldh % 4 == 0 && ((uintptr_t)hside & 15) == 0),
                    "ml1layer_forward: hside rows must be 16-byte aligned and hold Fi floats");
     const ML1Ws w = ml1_ws(N, Fi, Fo, concat);
@@ -463,7 +467,7 @@ extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col
     P.project = 1; P.epi = concat ? 2 : 1; P.Fo = Fo; P.Fop = s.Fop;
     P.bA = bA; P.bB = bB; P.bC = bC; P.bc = bconv;
     P.out = y; P.ldo = ldy; P.aux = aux; P.ldaux = ldaux; P.hout = hside; P.ldh = ldh;
-    return ml1_launch(P, s.smem, st);
+    return aux ? ml1_launch<true>(P, s.smem, st) : ml1_launch<false>(P, s.smem, st);     // no aux: the forward-only instantiation
 }
 
 extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,

@@ -300,10 +300,14 @@ class _ML3LayerFn(torch.autograd.Function):
 
     Backward (atomic-free): d pre from the activation kernel; G' = [S_0^T gc .. S_{K-1}^T gc | gp1 | gp2];
     dx = G' [Wc'^T ; W11 ; W12];  [dWc | dW11^T | dW12^T] = x^T G';  biases = column sums of d pre;
-    d ea' = SDDMM(x, gc Wc^T) and then through the edge MLP (activations recomputed)."""
+    d ea' = SDDMM(x, gc Wc^T) and then through the edge MLP (activations recomputed).
+
+    ``save`` (decided by the caller: inside ``forward`` grad mode is always off): False for a forward nobody differentiates
+    (``no_grad``, ``inference_mode``, frozen parameters) -- the fused kernels then store y alone (no tanh factors, no aggregate
+    side output) and nothing is saved for a backward."""
 
     @staticmethod
-    def forward(ctx, x, ea_s, w1, w2, w3, w4, wconv, bconv, w11, b11, w12, b12, plan, fused_edge, precision):
+    def forward(ctx, x, ea_s, w1, w2, w3, w4, wconv, bconv, w11, b11, w12, b12, plan, fused_edge, precision, save=True):
         if x.stride(1) != 1:        # row-strided views (padded layer outputs) are consumed as they are
             x = x.contiguous()
         ea_s = ea_s.contiguous()
@@ -321,11 +325,16 @@ class _ML3LayerFn(torch.autograd.Function):
             # first layer of a model (x carries no gradient, the weights do): the forward also leaves the aggregate behind and the
             # backward takes dW_k = H_k^T gc from it instead of aggregating S_k^T gc over the transposed CSR
             keep = (not ctx.needs_input_grad[0]) and ctx.needs_input_grad[6] and Fi <= 32 and KEEP_FIRST_LAYER_AGGREGATE
-            y, aux, ea2, hside = ops.ml3layer_forward(plan, xa, ea_s, ws4, wconv, bconv.contiguous() if bconv is not None else None, gates,
-                                                      keep_aggregate=keep)
+            if save:
+                y, aux, ea2, hside = ops.ml3layer_forward(plan, xa, ea_s, ws4, wconv, bconv.contiguous() if bconv is not None else None,
+                                                          gates, keep_aggregate=keep)
+            else:
+                y, aux, ea2, hside = ops.ml3layer_forward(plan, xa, ea_s, ws4, wconv, bconv.contiguous() if bconv is not None else None,
+                                                          gates, keep_aggregate=False, aux=False)
             ctx.plan, ctx.fused_edge, ctx.precision, ctx.G = plan, fused_edge, precision, G
             ctx.has_bias, ctx.fused, ctx.composite = bconv is not None, True, True
-            ctx.save_for_backward(xa, ea_s, ea2, y, aux, w1, w2, w3, w4, wconv, w11, w12, hside)
+            if save:
+                ctx.save_for_backward(xa, ea_s, ea2, y, aux, w1, w2, w3, w4, wconv, w11, w12, hside)
             return y
         if fused_edge:
             w1, w2, w3, w4 = w1.contiguous(), w2.contiguous(), w3.contiguous(), w4.contiguous()
@@ -343,10 +352,15 @@ class _ML3LayerFn(torch.autograd.Function):
             xa = ops.aligned_rows(x)
             wg = torch.cat([w11.t(), w12.t()], 1).contiguous() if G > 0 else None
             bg = torch.cat([b11, b12]) if G > 0 else None
-            y, aux = ops.fused_agg_proj(plan.rowptr, plan.col, None, ea2, xa, wconv.view(K * Fi, Fo), bias=bconv,
-                                        S=xa if G > 0 else None, self_mode=1 if G > 0 else 0, Bself=wg, bias_s=bg, G=G,
-                                        epilogue=1, win=plan.win, precision=precision)
-            ctx.save_for_backward(xa, ea_s, ea2 if fused_edge else None, y, aux, w1, w2, w3, w4, wconv, w11, w12, None)
+            if save:
+                y, aux = ops.fused_agg_proj(plan.rowptr, plan.col, None, ea2, xa, wconv.view(K * Fi, Fo), bias=bconv,
+                                            S=xa if G > 0 else None, self_mode=1 if G > 0 else 0, Bself=wg, bias_s=bg, G=G,
+                                            epilogue=1, win=plan.win, precision=precision)
+                ctx.save_for_backward(xa, ea_s, ea2 if fused_edge else None, y, aux, w1, w2, w3, w4, wconv, w11, w12, None)
+            else:
+                y, _ = ops.fused_agg_proj(plan.rowptr, plan.col, None, ea2, xa, wconv.view(K * Fi, Fo), bias=bconv,
+                                          S=xa if G > 0 else None, self_mode=1 if G > 0 else 0, Bself=wg, bias_s=bg, G=G,
+                                          epilogue=1, win=plan.win, precision=precision, aux=False)
             return y
         H = _aggregate(plan, ea2, x, K)
         # rows padded to a multiple of 4 floats so that the GEMM epilogues can store 128-bit vectors
@@ -357,7 +371,8 @@ class _ML3LayerFn(torch.autograd.Function):
                 wg = torch.cat([w11.t(), w12.t()], 1).contiguous()
                 ops.gemm_nn(x, wg, torch.cat([b11, b12]), precision=precision, out=pre[:, Fo:])
         y = ops.ml3_act_fwd(pre, Fo, G)
-        ctx.save_for_backward(x, ea_s, ea2 if fused_edge else None, pre, None, w1, w2, w3, w4, wconv, w11, w12, None)
+        if save:
+            ctx.save_for_backward(x, ea_s, ea2 if fused_edge else None, pre, None, w1, w2, w3, w4, wconv, w11, w12, None)
         return y
 
     @staticmethod
@@ -374,7 +389,7 @@ class _ML3LayerFn(torch.autograd.Function):
             ws4 = (w1, w2, w3, w4) if ctx.fused_edge else None
             dx, dea, dws, dwc, dbc, dw11, db11, dw12, db12 = ops.ml3layer_backward(
                 plan, x, ea_s, ea2, ws4, wconv, (w11, w12) if G > 0 else None, pre, aux, gy, need[0], need[1], ctx.has_bias, hside=hside)
-            return (dx, dea, dws[0], dws[1], dws[2], dws[3], dwc, dbc, dw11, db11, dw12, db12, None, None, None)
+            return (dx, dea, dws[0], dws[1], dws[2], dws[3], dwc, dbc, dw11, db11, dw12, db12, None, None, None, None)
         gy = gy.contiguous()
         Gp = torch.empty(N, K * Fo + 2 * G, dtype=torch.float32, device=x.device)
         if ctx.fused:
@@ -394,7 +409,7 @@ class _ML3LayerFn(torch.autograd.Function):
             return (z(x), z(ea_s), *(z(w) if w is not None else None for w in (w1, w2, w3, w4)), z(wconv),
                     torch.zeros(Fo, device=x.device) if ctx.has_bias else None,
                     z(w11) if G else None, torch.zeros(G, device=x.device) if G else None,
-                    z(w12) if G else None, torch.zeros(G, device=x.device) if G else None, None, None, None)
+                    z(w12) if G else None, torch.zeros(G, device=x.device) if G else None, None, None, None, None)
         if plan.E == 0:
             Gp[:, :K * Fo].zero_()
         else:
@@ -435,7 +450,14 @@ class _ML3LayerFn(torch.autograd.Function):
                 dea, dws = ops.edge_mlp_bwd(ea_s, None, dea2, w1, w2, w3, w4, need_dea=need[1])
             else:
                 dea = dea2
-        return (dx, dea, dws[0], dws[1], dws[2], dws[3], dwc, dbc, dw11, db11, dw12, db12, None, None, None)
+        return (dx, dea, dws[0], dws[1], dws[2], dws[3], dwc, dbc, dw11, db11, dw12, db12, None, None, None, None)
+
+
+def _needs_save(*tensors):
+    """Whether a layer's forward must keep what its backward reads: grad mode is on and some input or parameter requires a
+    gradient.  Decided before the autograd Function runs -- inside its ``forward`` grad mode is always off, and
+    ``ctx.needs_input_grad`` reports ``requires_grad`` whatever the grad mode."""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
 
 
 def _check_inputs(x, edge_index, edge_attr):
@@ -642,7 +664,7 @@ class ML3Layer(torch.nn.Module):
             ea = torch.relu(_LinearFn.apply(tmp, self.fc1_4.weight.t(), None, prec))
         w = (self.fc1_1.weight, self.fc1_2.weight, self.fc1_3.weight, self.fc1_4.weight) if fused_edge else (None,) * 4
         g = (self.fc11.weight, self.fc11.bias, self.fc12.weight, self.fc12.bias) if self.nout2 > 0 else (None,) * 4
-        return _ML3LayerFn.apply(x, ea, *w, c.weight, c.bias, *g, plan, fused_edge, prec)
+        return _ML3LayerFn.apply(x, ea, *w, c.weight, c.bias, *g, plan, fused_edge, prec, _needs_save(x, ea, *w, c.weight, c.bias, *g))
 
 
 # paths taken by ML1Layer since import (tests and benchmarks read it): "fused" = one library call per direction, "composed" =
@@ -657,17 +679,23 @@ class _ML1LayerFn(torch.autograd.Function):
         y  = relu(p0 + p1 * p2)   or, concatenated,   [relu(x WA^T + bA) | relu((A x) Wc + bc) | relu(p1 * p2)]
 
     Backward: G = [gA | gP p2 | gP p1] from the masks of y; dx = (A^T gc) Wc^T + G [WA ; WB ; WC] (one fused kernel over the
-    transposed CSR); [dWA^T | dWB^T | dWC^T | dWc] = x^T [G | A^T gc] (one contraction); biases = column sums of G and gc."""
+    transposed CSR); [dWA^T | dWB^T | dWC^T | dWc] = x^T [G | A^T gc] (one contraction); biases = column sums of G and gc.
+
+    ``save`` False (a forward nobody differentiates): the kernel stores y alone, without [p1 | p2], and nothing is saved."""
 
     @staticmethod
-    def forward(ctx, x, wconv, bconv, wA, bA, wB, bB, wC, bC, plan, concat):
+    def forward(ctx, x, wconv, bconv, wA, bA, wB, bB, wC, bC, plan, concat, save=True):
         xa = ops.aligned_rows(x)
         ws = [w.contiguous() for w in (wconv, wA, wB, wC)]
         bs = [b.contiguous() if b is not None else None for b in (bconv, bA, bB, bC)]
-        y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat)
+        if save:
+            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat)
+        else:
+            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat, aux=False)
         ctx.plan, ctx.concat = plan, concat
         ctx.has_bias = tuple(b is not None for b in (bconv, bA, bB, bC))
-        ctx.save_for_backward(xa, *ws, y, aux)
+        if save:
+            ctx.save_for_backward(xa, *ws, y, aux)
         return y
 
     @staticmethod
@@ -678,13 +706,13 @@ class _ML1LayerFn(torch.autograd.Function):
         if N == 0:
             z = torch.zeros_like
             bz = [torch.zeros(wconv.size(2), device=xa.device) if h else None for h in ctx.has_bias]
-            return z(xa), z(wconv), bz[0], z(wA), bz[1], z(wB), bz[2], z(wC), bz[3], None, None
+            return z(xa), z(wconv), bz[0], z(wA), bz[1], z(wB), bz[2], z(wC), bz[3], None, None, None
         gy = gy if gy.stride(1) == 1 else gy.contiguous()
         dx, dwc, dbc, dwA, dbA, dwB, dbB, dwC, dbC = ops.ml1layer_backward(ctx.plan, xa, wconv, wA, wB, wC, y, aux, gy, need[0],
                                                                           concat=ctx.concat)
         hb = ctx.has_bias
         return (dx, dwc, dbc if hb[0] else None, dwA, dbA if hb[1] else None, dwB, dbB if hb[2] else None, dwC,
-                dbC if hb[3] else None, None, None)
+                dbC if hb[3] else None, None, None, None)
 
 
 class ML1Layer(torch.nn.Module):
@@ -724,8 +752,8 @@ def ml1_layer(x, edge_index, conv, fcA, fcB, fcC, concat=False):
     Fi, Fo = conv.in_channels, conv.out_channels
     if ops.ml1layer_supported(Fi, Fo, concat):
         ML1_PATH_COUNTS["fused"] += 1
-        return _ML1LayerFn.apply(x, conv.weight, conv.bias, fcA.weight, fcA.bias, fcB.weight, fcB.bias, fcC.weight, fcC.bias, plan,
-                                 bool(concat))
+        ps = (conv.weight, conv.bias, fcA.weight, fcA.bias, fcB.weight, fcB.bias, fcC.weight, fcC.bias)
+        return _ML1LayerFn.apply(x, *ps, plan, bool(concat), _needs_save(x, *ps))
     ML1_PATH_COUNTS["composed"] += 1
     prec = _lib.PREC_3XTF32
     ones = torch.ones(plan.E, 1, dtype=torch.float32, device=x.device)

@@ -385,9 +385,10 @@ def fused_ts_supported(K, Kstride, F, Nc, Fs=0, self_mode=0, Ns=0):
 
 
 def fused_agg_proj(rowptr, col, eperm, ea, x, Bmain, bias=None, S=None, self_mode=0, Bself=None, bias_s=None, G=0,
-                   epilogue=0, hout=None, win=None, precision=_lib.PREC_3XTF32):
+                   epilogue=0, hout=None, win=None, precision=_lib.PREC_3XTF32, aux=True):
     """Fused aggregate + project (gnnml3_fused_agg_proj).  x [*, F] and S [N, Fs] must satisfy ``aligned_rows``.
-    epilogue 0 -> out [N, Nc];  epilogue 1 -> (y [N, Nc + G], aux [N, 2G]) = the ML3Layer node branch."""
+    epilogue 0 -> out [N, Nc];  epilogue 1 -> (y [N, Nc + G], aux [N, 2G]) = the ML3Layer node branch.
+    ``aux=False`` (a forward nobody differentiates): the kernel stores y alone and the returned aux is None."""
     lib = _lib.load()
     ea = _f32c(ea, "edge_attr")
     Bmain = _f32c(Bmain, "Bmain")
@@ -405,7 +406,8 @@ def fused_agg_proj(rowptr, col, eperm, ea, x, Bmain, bias=None, S=None, self_mod
     dev = x.device
     W = Nc + (G if self_mode == 1 else 0)
     out = _padded_rows(N, W, dev)
-    aux = torch.empty(N, 2 * G, dtype=torch.float32, device=dev) if self_mode == 1 else None
+    save_aux = self_mode == 1 and aux
+    aux = torch.empty(N, 2 * G, dtype=torch.float32, device=dev) if save_aux else None
     if bias is not None:
         bias = _f32c(bias, "bias")
     if bias_s is not None:
@@ -413,7 +415,7 @@ def fused_agg_proj(rowptr, col, eperm, ea, x, Bmain, bias=None, S=None, self_mod
     # algorithmic HBM bytes of this launch (SURVEY.md 8d: every operand once, the [N, K*F] aggregate never counted)
     E = ea.size(0)
     _prof["last_bytes"] = 4.0 * (N * F + (N * Fs if (self_mode and S.data_ptr() != x.data_ptr()) else 0) + E * K + E * (2 if eperm is not None else 1)
-                                 + (N + 1) + K * F * Nc + Fs * Ns + Nc + N * W + (N * 2 * G if self_mode == 1 else 0))
+                                 + (N + 1) + K * F * Nc + Fs * Ns + Nc + N * W + (N * 2 * G if save_aux else 0))
     ws = _ws(dev, lib.gnnml3_fused_workspace_bytes(K, F, Nc, self_mode), tag="fused")
     with _on(dev):
         _lib.check(lib.gnnml3_fused_agg_proj(
@@ -495,11 +497,12 @@ def ml3layer_supported(K, Fi, Fo, G, learnedge):
     return bool(_lib.load().gnnml3_ml3layer_supported(int(K), int(Fi), int(Fo), int(G), int(bool(learnedge))))
 
 
-def ml3layer_forward(plan, x, ea_s, ws4, wconv, bconv, gates, keep_aggregate=False):
+def ml3layer_forward(plan, x, ea_s, ws4, wconv, bconv, gates, keep_aggregate=False, aux=True):
     """Whole ML3Layer forward in one library call (gnnml3_ml3layer_forward).  ``ws4`` = (w1, w2, w3, w4) or None,
     ``gates`` = (w11, b11, w12, b12) or None.  -> (y [N, Fo+G], aux [N, 2G] | None, ea2 [E, K] | None, hside | None)
     ``keep_aggregate``: also leave H = [S_0 x .. S_{K-1} x] behind ([N, (K [+1]) * 32]) for a backward that needs the weight
-    gradient but no dx (first layer): dW_k = H_k^T gc then needs no aggregation over the transposed CSR."""
+    gradient but no dx (first layer): dW_k = H_k^T gc then needs no aggregation over the transposed CSR.
+    ``aux=False`` (a forward nobody differentiates): the tanh factors are not stored and the returned aux is None."""
     lib = _lib.load()
     N, Fi = x.shape
     E, K = ea_s.shape
@@ -509,7 +512,7 @@ def ml3layer_forward(plan, x, ea_s, ws4, wconv, bconv, gates, keep_aggregate=Fal
     W = Fo + G
     y = _padded_rows(N, W, dev)
     ldy = (W + 3) // 4 * 4
-    aux = torch.empty(N, 2 * G, dtype=torch.float32, device=dev) if G > 0 else None
+    aux = torch.empty(N, 2 * G, dtype=torch.float32, device=dev) if (G > 0 and aux) else None
     ea2 = torch.empty(E, K, dtype=torch.float32, device=dev) if ws4 is not None else None
     ldh = (K + (1 if G > 0 else 0)) * 32
     hside = torch.empty(N, ldh, dtype=torch.float32, device=dev) if (keep_aggregate and Fi <= 32) else None
@@ -562,17 +565,18 @@ def ml1layer_supported(Fi, Fo, concat=False):
     return bool(_lib.load().gnnml3_ml1layer_supported(int(Fi), int(Fo), int(bool(concat))))
 
 
-def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False, keep_aggregate=False):
+def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False, keep_aggregate=False, aux=True):
     """Whole GNNML1 layer forward in one library call (gnnml3_ml1layer_forward) over the plan of the plain ``edge_index``.
     x [N, Fi] must satisfy ``aligned_rows``; wconv [1, Fi, Fo]; wA/wB/wC [Fo, Fi].  -> (y [N, Fo] or [N, 3 Fo],
-    aux [N, 2 Fo] = [p1 | p2], A x [N, Fi] if ``keep_aggregate`` else None)"""
+    aux [N, 2 Fo] = [p1 | p2] (None with ``aux=False``: a forward nobody differentiates stores y alone),
+    A x [N, Fi] if ``keep_aggregate`` else None)"""
     lib = _lib.load()
     N, Fi = x.shape
     Fo = wconv.size(2)
     dev = x.device
     W = 3 * Fo if concat else Fo
     y = _padded_rows(N, W, dev)
-    aux = torch.empty(N, 2 * Fo, dtype=torch.float32, device=dev)
+    aux = torch.empty(N, 2 * Fo, dtype=torch.float32, device=dev) if aux else None
     hside = _padded_rows(N, Fi, dev) if keep_aggregate else None
     ws = _ws(dev, lib.gnnml3_ml1layer_workspace_bytes(N, Fi, Fo, int(bool(concat))), tag="ml1")
     p = _lib.ptr

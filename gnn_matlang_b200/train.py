@@ -233,14 +233,25 @@ def padded_shapes(batches, max_pad_degree=8, adjacency=False):
 
     ``adjacency=True``: (n_nodes, n_entries, n_edges), sizing the plain ``edge_index`` as well (``n_entries`` is None for batches
     without supports); the dummy nodes then bound the self-loops a dummy node receives from BOTH lists together."""
-    nmax = max(int(b.x.shape[0]) for b in batches)
+    nodes = [int(b.x.shape[0]) for b in batches]
     if not adjacency:
-        emax = max(int(b.edge_index2.shape[1]) for b in batches)
-        emin = min(int(b.edge_index2.shape[1]) for b in batches)
-        return nmax + 1 + (emax - emin + max_pad_degree - 1) // max_pad_degree, emax
+        return padded_shapes_from_sizes(nodes, [int(b.edge_index2.shape[1]) for b in batches], max_pad_degree=max_pad_degree)
     sup = getattr(batches[0], "edge_index2", None) is not None
-    es = [int(b.edge_index2.shape[1]) for b in batches] if sup else [0]
-    ms = [int(b.edge_index.shape[1]) for b in batches]
+    return padded_shapes_from_sizes(nodes, [int(b.edge_index2.shape[1]) for b in batches] if sup else None,
+                                    [int(b.edge_index.shape[1]) for b in batches], max_pad_degree=max_pad_degree)
+
+
+def padded_shapes_from_sizes(nodes, entries=None, edges=None, max_pad_degree=8):
+    """The rule of ``padded_shapes`` on per-batch totals (nodes, support entries, plain edges of every batch) instead of
+    collated batches, so that shapes can be fixed from a dataset's size arrays alone.  ``edges=None``: (n_nodes, n_entries);
+    otherwise (n_nodes, n_entries or None when ``entries`` is None, n_edges)."""
+    nmax = max(int(n) for n in nodes)
+    if edges is None:
+        emax, emin = max(int(e) for e in entries), min(int(e) for e in entries)
+        return nmax + 1 + (emax - emin + max_pad_degree - 1) // max_pad_degree, emax
+    sup = entries is not None
+    es = [int(e) for e in entries] if sup else [0]
+    ms = [int(m) for m in edges]
     pe, pm = max(es) - min(es), max(ms) - min(ms)             # most padding either list can need (smallest batch)
     if pe and pm and max_pad_degree < 2:
         raise ValueError("padded_shapes: padding both lists needs max_pad_degree >= 2")
@@ -398,3 +409,163 @@ class GraphedTrainer(object):
             dist.all_reduce(self.flat, op=dist.ReduceOp.SUM)
             self.graph2.replay()
         return self.static_loss
+
+
+EVAL_METRICS = ("l1", "mse", "bce", None)
+
+
+def eval_terms(metric, out, y):
+    """Per-graph terms of ``loss_fn(metric, out, y)`` (its SUM over graphs is the loss): out [B, d], labels y (any shape with
+    B * d elements) -> (term [B], correct [B] or None).  ``correct`` = [(o > 0) == (y > 0.5)] for a single-output "bce" head (the
+    accuracy of exp_classify.py's test loop); None for the other metrics and for wider heads."""
+    y = y.to(out.dtype).reshape(out.shape)
+    if metric == "l1":
+        return (out - y).abs().sum(1), None
+    if metric == "mse":
+        return torch.square(out - y).sum(1), None
+    if metric == "bce":
+        term = F.binary_cross_entropy(torch.sigmoid(out), y, reduction="none").sum(1)
+        correct = ((out[:, 0] > 0) == (y[:, 0] > 0.5)).to(out.dtype) if out.size(1) == 1 else None
+        return term, correct
+    raise ValueError(metric)
+
+
+def eval_chunks(ids, batch_size, n_nodes):
+    """The batches of an evaluation pass over the split ``ids``: consecutive chunks of ``batch_size`` ids (clipped to len(ids)),
+    in order, as the reference's ``DataLoader(shuffle=False)``; a short last chunk is filled up to ``batch_size`` with copies of
+    the split's smallest graph (fewest nodes, first such id).  ``n_nodes``: the dataset's node count per graph.
+    -> (chunks [n_chunks, B] int64, weights [n_chunks, B] float32: 1 for the split's graphs, 0 for the fillers)."""
+    import numpy as np
+    ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+    B = min(int(batch_size), len(ids))
+    nc = -(-len(ids) // B)
+    filler = ids[int(np.argmin(np.asarray(n_nodes)[ids]))]
+    chunks = np.full(nc * B, filler, dtype=np.int64)
+    chunks[:len(ids)] = ids
+    w = np.zeros(nc * B, dtype=np.float32)
+    w[:len(ids)] = 1.0
+    return chunks.reshape(nc, B), w.reshape(nc, B)
+
+
+def eval_shapes(dataset, chunks, max_pad_degree=8):
+    """Padded shapes of the captured evaluation batch from the dataset's host size arrays (``n_h``, ``e_h``, ``m_h``) and the
+    chunks of ``eval_chunks``, with the rule of ``padded_shapes``: (n_nodes, n_entries or None, n_edges or None).  The batch
+    carries the lists the dataset keeps: supports (``e_h``) and / or plain edges (``m_h``)."""
+    nodes = dataset.n_h[chunks].sum(1)
+    entries = dataset.e_h[chunks].sum(1) if dataset.e_h is not None else None
+    if dataset.m_h is None:
+        Np, Ep = padded_shapes_from_sizes(nodes, entries, max_pad_degree=max_pad_degree)
+        return Np, Ep, None
+    return padded_shapes_from_sizes(nodes, entries, dataset.m_h[chunks].sum(1), max_pad_degree=max_pad_degree)
+
+
+class GraphedEvaluator(object):
+    """The test loop of the reference's scripts (``test()``: MAE on ZINC, MSE on counting, accuracy on EXP, the embeddings of the
+    isomorphism scripts) over a split of a resident ``synthetic.DeviceDataset``, captured ONCE into a CUDA graph and replayed per
+    batch: device collation into static buffers, the model's forward under ``no_grad`` (the forward-only kernels: nothing is saved
+    for a backward) and the metric accumulated on the device in float64.
+
+        ev = GraphedEvaluator(model, dataset, ids, batch_size, metric="l1")
+        res = ev.run()                  # {"graphs": n, "sum": s, "mean": s / n} (+ "correct", "accuracy" for "bce")
+        res = ev.run(outputs=True)      # also res["outputs"]: [len(ids), out] device tensor in id order
+
+    Batches are consecutive chunks of ``ids`` (``eval_chunks``); a short last chunk is filled with copies of the split's smallest
+    graph, which a per-graph weight (0 for fillers) keeps out of the metric and the outputs.  Shapes come from the dataset's host
+    size arrays (``eval_shapes``), so nothing is collated on the host.  The model runs in eval mode (BatchNorm running statistics,
+    no dropout) during warm-up and capture; its previous mode is restored afterwards.  The graph reads parameters and buffers in
+    place: a trainer stepping the same model between two ``run()`` calls is seen by the second.  ``run()`` reads the device once,
+    at the end.  ``distributed=True``: every rank passes its own ids and ``run()`` SUM-all-reduces the metric once (outputs stay per
+    rank).  ``metric``: "l1", "mse", "bce" (the per-graph terms of ``loss_fn``) or None (outputs only)."""
+
+    def __init__(self, model, dataset, ids, batch_size, metric="l1", max_pad_degree=8, distributed=False, warmup=2):
+        import numpy as np
+        from .batch import Batch
+        from .graph import set_range_check
+        if metric not in EVAL_METRICS:
+            raise ValueError("GraphedEvaluator: metric must be one of %s, got %r" % (EVAL_METRICS, metric))
+        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+        if len(ids) == 0:
+            raise ValueError("GraphedEvaluator: ids is empty")
+        if ids.min() < 0 or ids.max() >= len(dataset.n_h):
+            raise ValueError("GraphedEvaluator: ids outside the dataset's %d graphs" % len(dataset.n_h))
+        if int(batch_size) < 1:
+            raise ValueError("GraphedEvaluator: batch_size must be positive")
+        self.model, self.dataset, self.metric = model, dataset, metric
+        self.n = len(ids)
+        self.chunks, weights = eval_chunks(ids, batch_size, dataset.n_h)
+        self.B = B = self.chunks.shape[1]
+        Np, Ep, Mp = eval_shapes(dataset, self.chunks, max_pad_degree)
+        self.shapes = (Np, Ep, Mp)
+        self.distributed = distributed and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+        set_range_check(False)                         # the range check reads a flag back from the device
+        dev = dataset.x.device
+        self._ids = [torch.from_numpy(c).pin_memory() for c in self.chunks]
+        self._w_all = torch.from_numpy(weights).to(dev)
+        f32 = dict(dtype=torch.float32, device=dev)
+        st = Batch(x=torch.zeros(Np, dataset.x.size(1), **f32), batch=torch.zeros(Np, dtype=torch.int64, device=dev),
+                   graph_ptr=torch.zeros(B + 2, dtype=torch.int32, device=dev), num_graphs=B + 1, real_graphs=B,
+                   y=torch.zeros(B, dataset.y[:1].numel(), dtype=dataset.y.dtype, device=dev))
+        if dataset.e_h is not None:
+            st.edge_index2 = torch.zeros(2, Ep, dtype=torch.int64, device=dev)
+            st.edge_attr2 = torch.zeros(Ep, dataset.ea.size(1), **f32)
+        if dataset.m_h is not None:
+            st.edge_index = torch.zeros(2, Mp, dtype=torch.int64, device=dev)
+        self.static = st
+        self.w = torch.zeros(B, **f32)
+        self.acc = torch.zeros(3, dtype=torch.float64, device=dev)        # metric sum | correct | graphs
+        dataset.collate_into(self._ids[0], st)
+        self.w.copy_(self._w_all[0])
+        was_training = model.training
+        model.eval()
+        try:
+            s = torch.cuda.Stream(device=dev)
+            s.wait_stream(torch.cuda.current_stream(dev))
+            with torch.cuda.stream(s), torch.no_grad():
+                for _ in range(warmup):
+                    self._step()
+            torch.cuda.current_stream(dev).wait_stream(s)
+            torch.cuda.synchronize(dev)
+            self.graph = torch.cuda.CUDAGraph()
+            with torch.no_grad(), torch.cuda.graph(self.graph):
+                self.static_out = self._step()
+        finally:
+            model.train(was_training)
+
+    def _step(self):
+        """Forward of the static batch and the metric of its real graphs, added to the accumulator."""
+        out = self.model(self.static.fresh())[:self.B]
+        if out.dim() == 1:
+            out = out.unsqueeze(1)
+        if self.metric is not None:
+            real = self.w > 0
+            term, correct = eval_terms(self.metric, out, self.static.y)
+            self.acc[0] += torch.where(real, term, torch.zeros_like(term)).double().sum()
+            if correct is not None:
+                self.acc[1] += torch.where(real, correct, torch.zeros_like(correct)).double().sum()
+        self.acc[2] += self.w.double().sum()
+        return out
+
+    def run(self, outputs=False):
+        """One pass over the split: per batch, device collation into the captured buffers, the weights and one replay."""
+        self.acc.zero_()
+        out_all = torch.empty(len(self._ids) * self.B, self.static_out.size(1), dtype=self.static_out.dtype,
+                              device=self.static_out.device) if outputs else None
+        for c, ix in enumerate(self._ids):
+            self.dataset.collate_into(ix, self.static)
+            self.w.copy_(self._w_all[c])
+            self.graph.replay()
+            if outputs:
+                out_all[c * self.B:(c + 1) * self.B].copy_(self.static_out)
+        if self.distributed:
+            dist.all_reduce(self.acc, op=dist.ReduceOp.SUM)
+        vals = self.acc.tolist()                       # the pass's one read from the device
+        res = {"graphs": int(round(vals[2]))}
+        if self.metric is not None:
+            res["sum"] = vals[0]
+            res["mean"] = vals[0] / max(res["graphs"], 1)
+            if self.metric == "bce" and self.static_out.size(1) == 1:
+                res["correct"] = int(round(vals[1]))
+                res["accuracy"] = vals[1] / max(res["graphs"], 1)
+        if outputs:
+            res["outputs"] = out_all[:self.n]
+        return res

@@ -162,6 +162,7 @@ GNNML3_API int gnnml3_ml3_act_bwd_y(const float* y, int64_t ldy, const float* au
  * without materialising the [N, K*F] aggregate (libs/spect_conv.py:70-80,93-94).  Optional self block S [N, Fs]:
  *   self_mode 1: own output columns  s[t, :] = S[t, :] Bself [Fs, Ns = 2G] (+ bias_s)  -- with epilogue 1 this is the whole
  *                ML3Layer node branch (:208-212): out[t] = [relu(main) || tanh(s[:G]) * tanh(s[G:])], aux[t] = tanh(s);
+ *                aux may be NULL (inference: nothing is saved for a backward): a forward-only kernel then stores out alone;
  *   self_mode 2: main[t, :] += S[t, :] Bself [Fs, Nc]  (SpectConv selfconn; gate gradients in the dx pass).
  * epilogue 0: out [N, Nc] = main.  X and S rows must be 16-byte aligned (ld % 4 == 0) and every column below
  * ceil4(F) / ceil4(Fs) must hold finite values.  3xTF32 arithmetic (FP32-grade).  Backward dx = the same call over the
@@ -223,7 +224,9 @@ GNNML3_API int gnnml3_fused_sddmm(const int32_t* rowptr, const int32_t* col, con
  * the point is the host cost (one call instead of ~30 small operations per layer and direction).
  *   forward : ea_s [E,K] dst-sorted edge features; w1..w4 = fc1_1..fc1_4.weight (NULL: learnedge = False, ea2 unused);
  *             wconv [K,Fi,Fo], bconv [Fo] (nullable); w11,b11,w12,b12 = fc11/fc12 (NULL iff G == 0);
- *             outputs ea2 [E,K], y [N, ldy >= Fo+G], aux [N, 2G] (tanh factors, saved for the backward).
+ *             outputs ea2 [E,K], y [N, ldy >= Fo+G], aux [N, 2G] (tanh factors, saved for the backward).  aux == NULL
+ *             (with hside == NULL: an inference forward) stores y alone, through the forward-only instantiation of the fused
+ *             kernel; the backward still requires aux.
  *   backward: gy [N, ldgy]; outputs dx [N, lddx] (if need_dx), dea [E,K] (if need_dea), dw1..dw4, dwconv [K,Fi,Fo],
  *             dbias [Fo + 2G] = (d bconv | d b11 | d b12), dw11/dw12 [G,Fi].
  *   hside   : optional [N, ldh >= (K [+1 if G > 0]) * 32] (nullable, Fi <= 32).  The forward leaves the aggregate
@@ -259,6 +262,8 @@ GNNML3_API int gnnml3_ml3layer_backward(const int32_t* rowptr, const int32_t* co
  * One fused kernel per direction: the aggregate and the four projections meet in tensor memory (tcgen05, 3xTF32, FP32-grade).
  *   forward : rowptr / col = the dst-sorted CSR of edge_index (gnnml3_csr_build); outputs y [N, ldy] and aux [N, ldaux >= 2 Fo]
  *             = [p1 | p2] (saved for the backward); hside (nullable, [N, ldh >= Fi]) receives A x.  Biases are nullable.
+ *             aux may be NULL (inference): a forward-only instantiation of the kernel then stores y alone (a third of the
+ *             sum-mode stores).  The backward requires the aux of a forward that wrote it.
  *   backward: rowptrT / colT = the transposed CSR; gy [N, ldgy]; dx [N, lddx] if need_dx (else dx may be NULL: the aggregate
  *             A^T gc is still formed for d wconv); outputs the eight parameter gradients (dw* overwritten; db* nullable).
  * Supported: 1 <= Fi <= 64, 1 <= Fo <= 64 (gnnml3_ml1layer_supported), E = 0 allowed; x rows 16-byte aligned (ldx % 4 == 0).
