@@ -82,6 +82,10 @@ SIGNATURES = {
                                      _p, _i64, _p, _sz, _p]),
     "gnnml3_ml1layer_backward": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64, _p, _i64, _i,
                                       _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "gnnml3_ml1layer_forward_precision": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _p, _i64, _p,
+                                               _i64, _p, _i64, _p, _sz, _p, _i]),
+    "gnnml3_ml1layer_backward_precision": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64, _p, _i64,
+                                                _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
     "gnnml3_segment_pool_fwd":(_i, [_p, _i64, _p, _i, _i, _i, _p, _p]),
     "gnnml3_segment_pool_bwd": (_i, [_p, _p, _i, _i, _i, _p, _i64, _p]),
     "gnnml3_segment_max_fwd": (_i, [_p, _i64, _p, _i, _i, _p, _p, _p]),
@@ -94,7 +98,7 @@ SIGNATURES = {
 
 PREC_3XTF32 = 0
 PREC_TF32 = 1
-PREC_BF16 = 2          # fused layer kernel only (GNNML3_FUSED_BF16); the stand-alone GEMMs run it as single-pass TF32
+PREC_BF16 = 2          # fused layer kernels only (GNNML3_FUSED_BF16, the GNNML1 layer); the stand-alone GEMMs run it as single-pass TF32
 FUSED_FLAGS = {0: 0, 1: 0x100, 2: 0x200}
 EPI_NONE = 0
 EPI_RELU = 1

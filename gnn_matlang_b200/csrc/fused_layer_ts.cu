@@ -201,10 +201,6 @@ __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, u
         "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// instruction descriptor of tcgen05.mma kind::f16 with BF16 A / B (K-major) and FP32 D
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
 // this thread's 16 features of a block -> 8 packed BF16 pairs (features 2j, 2j+1 of the thread's 16 in register j)
 __device__ __forceinline__ void ts_pack_bf16(const float* v, uint32_t (&r)[8]) {
 #pragma unroll

@@ -15,6 +15,14 @@
 // FP32-grade (3xTF32) products.  Two A buffers alternate, so the gather of one k-block overlaps the MMAs of the previous.
 // The accumulator D[row, column] lives in tensor memory (lane = tile row); the epilogue reads it back and applies the layer.
 //
+// Precision (template PREC = GNNML3_PREC_*; the aggregation, the epilogues and their FP32 outputs are the same in every mode):
+//   0 3xTF32 : as above (default, FP32-grade).
+//   1 TF32   : one kind::tf32 MMA per 8-wide k-step, raw A (truncated by the tensor core) x RN-TF32(w); no residual planes,
+//              so each A buffer and the resident weights are half the size.
+//   2 BF16   : A and w RN-converted to BF16 and stored in the first 64 bytes of each 128-byte swizzled row (32 values; the
+//              16-byte chunk c >> 1 of a row holds features 8 (c >> 1) .. + 7, XOR-swizzled with row & 7 as in FP32); two
+//              kind::f16 MMAs (K = 16) per k-block, FP32 accumulate.  No residual planes either.
+//
 //   forward : self = x, weights [fcA^T | fcB^T | fcC^T] -> columns [p0 | p1 | p2] (pitch Fop = ceil16(Fo));
 //             gathered = x over the CSR, weights Wc -> columns [0, Fop) (sum: adds into p0) or [3 Fop, 4 Fop) (concat).
 //   dx pass : self = [gA | gP*p2 | gP*p1] (d p0, d p1, d p2), weights [fcA ; fcB ; fcC]; gathered = gc over the transposed
@@ -22,12 +30,18 @@
 // Deterministic: every sum has a fixed order (edges in CSR order, k-blocks in list order), no atomics.  No host sync.
 #include "tc_common.cuh"
 
+#include <cuda_bf16.h>
+
 namespace gnnml3 {
 
 constexpr int ML1_THREADS = 512;
 constexpr int ML1_ROWS = 128;                      // tile rows = MMA M = tensor-memory lanes
 constexpr int ML1_APLANE = ML1_ROWS * 128;         // bytes of one 128-row x 32-float swizzled plane
-constexpr int ML1_ABUF = 2 * ML1_APLANE;           // raw plane + residual plane
+constexpr int ML1_ABUF = 2 * ML1_APLANE;           // raw plane + residual plane (3xTF32; the flagged modes use the first)
+
+// planes per k-block of an A buffer and of the weights: raw/hi + residual/lo in 3xTF32, one plane in TF32 and BF16
+__host__ __device__ constexpr int ml1_planes(int prec) { return prec == GNNML3_PREC_3XTF32 ? 2 : 1; }
+__host__ __device__ constexpr int ml1_abuf(int prec) { return ml1_planes(prec) * ML1_APLANE; }    // bytes of one A buffer
 
 struct ML1Params {
     const int* rowptr;      // [N+1] CSR of the gathered blocks (dst-sorted forward, src-sorted for dx)
@@ -70,13 +84,14 @@ __device__ __forceinline__ float4 ml1_load4(const float* __restrict__ row, int f
 __device__ __forceinline__ float ml1_lo(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
 
 // AUX = false: the forward-only instantiation of the GNNML1 epilogues (aux == NULL), which stores y and not [p1 | p2].
-template <bool AUX = true>
+// PREC: the arithmetic of the projection (GNNML3_PREC_*, see the top of this file).
+template <bool AUX = true, int PREC = GNNML3_PREC_3XTF32>
 __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_constant__ ML1Params P) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     uint8_t* wsm = smem;                                     // resident weight planes
-    uint8_t* abuf = smem + P.wbytes;                         // [2][raw plane | lo plane]
-    uint64_t* bars = reinterpret_cast<uint64_t*>(abuf + 2 * ML1_ABUF);   // [2] MMAs reading A buffer b retired
+    uint8_t* abuf = smem + P.wbytes;                         // [2][raw plane | lo plane (3xTF32 only)]
+    uint64_t* bars = reinterpret_cast<uint64_t*>(abuf + 2 * ml1_abuf(PREC));   // [2] MMAs reading A buffer b retired
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
@@ -104,7 +119,7 @@ __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_co
     bool pend0 = false, pend1 = false;
     uint32_t it = 0;
     const uint32_t wsm0 = smem_u32(wsm), abuf0 = smem_u32(abuf);
-    const uint32_t self_bytes = (uint32_t)P.nsb * 2u * (uint32_t)P.NsP * 128u;
+    const uint32_t self_bytes = (uint32_t)P.nsb * (uint32_t)ml1_planes(PREC) * (uint32_t)P.NsP * 128u;
 
     for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x) {
         const int64_t row0 = (int64_t)tile * ML1_ROWS;
@@ -115,7 +130,7 @@ __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_co
             const bool self = i < P.nsb;
             const int kb = self ? i : i - P.nsb;
             const int f = kb * 32 + 4 * c;
-            uint8_t* A = abuf + b * ML1_ABUF;
+            uint8_t* A = abuf + b * ml1_abuf(PREC);
             float4 v[2];
             int64_t r[2];
             int rs[2] = {0, 0}, re[2] = {0, 0};
@@ -162,30 +177,65 @@ __global__ void __launch_bounds__(ML1_THREADS, 1) k_ml1_agg_proj(const __grid_co
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
                 const int m = rsub + 64 * h;
-                const uint32_t off = (uint32_t)(m >> 3) * 1024u + (uint32_t)(m & 7) * 128u + (uint32_t)((c ^ (m & 7)) << 4);
-                *reinterpret_cast<float4*>(A + off) = v[h];
-                *reinterpret_cast<float4*>(A + ML1_APLANE + off) = make_float4(ml1_lo(v[h].x), ml1_lo(v[h].y), ml1_lo(v[h].z), ml1_lo(v[h].w));
+                if constexpr (PREC == GNNML3_PREC_3XTF32) {
+                    const uint32_t off = (uint32_t)(m >> 3) * 1024u + (uint32_t)(m & 7) * 128u + (uint32_t)((c ^ (m & 7)) << 4);
+                    *reinterpret_cast<float4*>(A + off) = v[h];
+                    *reinterpret_cast<float4*>(A + ML1_APLANE + off) =
+                        make_float4(ml1_lo(v[h].x), ml1_lo(v[h].y), ml1_lo(v[h].z), ml1_lo(v[h].w));
+                } else if constexpr (PREC == GNNML3_PREC_TF32) {     // raw plane alone
+                    const uint32_t off = (uint32_t)(m >> 3) * 1024u + (uint32_t)(m & 7) * 128u + (uint32_t)((c ^ (m & 7)) << 4);
+                    *reinterpret_cast<float4*>(A + off) = v[h];
+                } else {                                             // 4 BF16 = half of the 16-byte chunk c >> 1
+                    const uint32_t off = (uint32_t)(m >> 3) * 1024u + (uint32_t)(m & 7) * 128u +
+                                         (uint32_t)(((c >> 1) ^ (m & 7)) << 4) + (uint32_t)(c & 1) * 8u;
+                    const __nv_bfloat162 lo = __floats2bfloat162_rn(v[h].x, v[h].y), hi = __floats2bfloat162_rn(v[h].z, v[h].w);
+                    *reinterpret_cast<uint2*>(A + off) =
+                        make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
+                }
             }
             fence_proxy_async_smem();
             __syncthreads();
             if (tid == 0) {
                 tc_fence_after();
                 const int N = self ? P.NsP : P.NgP;
-                const uint32_t idesc = make_idesc_tf32_mn(ML1_ROWS, N);
-                const uint32_t d = tmem_base + (uint32_t)(self ? 0 : P.colG);
-                const bool fresh = self ? kb == 0 : (kb == 0 && P.colG >= P.NsP);   // first k-block into these columns
-                const uint32_t wb = wsm0 + (self ? (uint32_t)kb * 2u * (uint32_t)P.NsP * 128u
-                                                 : self_bytes + (uint32_t)kb * 2u * (uint32_t)P.NgP * 128u);
-                const uint64_t a_hi = make_kmajor_sw128_desc(abuf0 + (uint32_t)b * ML1_ABUF);
-                const uint64_t a_lo = make_kmajor_sw128_desc(abuf0 + (uint32_t)b * ML1_ABUF + ML1_APLANE);
-                const uint64_t w_hi = make_kmajor_sw128_desc(wb);
-                const uint64_t w_lo = make_kmajor_sw128_desc(wb + (uint32_t)N * 128u);
+                if constexpr (PREC == GNNML3_PREC_3XTF32) {
+                    const uint32_t idesc = make_idesc_tf32_mn(ML1_ROWS, N);
+                    const uint32_t d = tmem_base + (uint32_t)(self ? 0 : P.colG);
+                    const bool fresh = self ? kb == 0 : (kb == 0 && P.colG >= P.NsP);   // first k-block into these columns
+                    const uint32_t wb = wsm0 + (self ? (uint32_t)kb * 2u * (uint32_t)P.NsP * 128u
+                                                     : self_bytes + (uint32_t)kb * 2u * (uint32_t)P.NgP * 128u);
+                    const uint64_t a_hi = make_kmajor_sw128_desc(abuf0 + (uint32_t)b * ML1_ABUF);
+                    const uint64_t a_lo = make_kmajor_sw128_desc(abuf0 + (uint32_t)b * ML1_ABUF + ML1_APLANE);
+                    const uint64_t w_hi = make_kmajor_sw128_desc(wb);
+                    const uint64_t w_lo = make_kmajor_sw128_desc(wb + (uint32_t)N * 128u);
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const uint64_t adv = (uint64_t)((k * 32) >> 4);     // 8 TF32 = 32 bytes along K inside the swizzled row
-                    umma_tf32(d, a_hi + adv, w_hi + adv, idesc, (fresh && k == 0) ? 0u : 1u);
-                    umma_tf32(d, a_hi + adv, w_lo + adv, idesc, 1u);
-                    umma_tf32(d, a_lo + adv, w_hi + adv, idesc, 1u);
+                    for (int k = 0; k < 4; ++k) {
+                        const uint64_t adv = (uint64_t)((k * 32) >> 4);     // 8 TF32 = 32 bytes along K inside the swizzled row
+                        umma_tf32(d, a_hi + adv, w_hi + adv, idesc, (fresh && k == 0) ? 0u : 1u);
+                        umma_tf32(d, a_hi + adv, w_lo + adv, idesc, 1u);
+                        umma_tf32(d, a_lo + adv, w_hi + adv, idesc, 1u);
+                    }
+                } else {                                             // one plane each of A and w: a single product per k-step
+                    const uint32_t d = tmem_base + (uint32_t)(self ? 0 : P.colG);
+                    const bool fresh = self ? kb == 0 : (kb == 0 && P.colG >= P.NsP);
+                    const uint32_t wb = wsm0 + (self ? (uint32_t)kb * (uint32_t)P.NsP * 128u : self_bytes + (uint32_t)kb * (uint32_t)P.NgP * 128u);
+                    const uint64_t a = make_kmajor_sw128_desc(abuf0 + (uint32_t)b * ml1_abuf(PREC));
+                    const uint64_t w = make_kmajor_sw128_desc(wb);
+                    if constexpr (PREC == GNNML3_PREC_TF32) {
+                        const uint32_t idesc = make_idesc_tf32_mn(ML1_ROWS, N);
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) {
+                            const uint64_t adv = (uint64_t)((k * 32) >> 4);
+                            umma_tf32(d, a + adv, w + adv, idesc, (fresh && k == 0) ? 0u : 1u);
+                        }
+                    } else {
+                        const uint32_t idesc = make_idesc_bf16(ML1_ROWS, N);
+#pragma unroll
+                        for (int k = 0; k < 2; ++k) {
+                            const uint64_t adv = (uint64_t)((k * 32) >> 4); // 16 BF16 = 32 bytes along K
+                            umma_bf16(d, a + adv, w + adv, idesc, (fresh && k == 0) ? 0u : 1u);
+                        }
+                    }
                 }
                 umma_commit(bars + b);                                   // A buffer b reusable once these retire
             }
@@ -259,7 +309,9 @@ __device__ __forceinline__ int ml1_swz(int n, int k) {      // float index of el
 // Weight planes of one launch in the kernel's shared-memory byte layout.  dir 0 (forward): self block rows n = output
 // column (group b = n / Fop of [fcA | fcB | fcC], feature o = n % Fop), k = input feature; gathered rows n = output column of
 // Wc [Fi, Fo].  dir 1 (dx): self rows n = input feature i, k over [gA | gP p2 | gP p1] (block pitch Fo4); gathered rows
-// n = i, k = o of Wc^T.
+// n = i, k = o of Wc^T.  PREC 0: a hi plane (RN-TF32) then a lo plane (w - hi) per k-block; PREC 1: the hi plane alone;
+// PREC 2: one plane of RN-BF16 values in the first 64 bytes of each row (the kernel's BF16 A layout), the rest zero.
+template <int PREC = GNNML3_PREC_3XTF32>
 __global__ void k_ml1_prep(const float* __restrict__ wc, const float* __restrict__ wA, const float* __restrict__ wB,
                            const float* __restrict__ wC, int Fi, int Fo, int dir, int nsb, int NsP, int ngb, int NgP, int Fop,
                            int Fo4, float* __restrict__ planes) {
@@ -287,10 +339,21 @@ __global__ void k_ml1_prep(const float* __restrict__ wc, const float* __restrict
                 v = __ldg(wc + (int64_t)n * Fo + kk);
             }
         }
-        const float h = tf32_rn(v);
-        float* base = planes + (self ? (size_t)kb * 2 * NsP * 32 : (size_t)nsb * 2 * NsP * 32 + (size_t)kb * 2 * NgP * 32);
-        base[ml1_swz(n, k)] = h;
-        base[NP * 32 + ml1_swz(n, k)] = v - h;
+        if constexpr (PREC == GNNML3_PREC_3XTF32) {
+            const float h = tf32_rn(v);
+            float* base = planes + (self ? (size_t)kb * 2 * NsP * 32 : (size_t)nsb * 2 * NsP * 32 + (size_t)kb * 2 * NgP * 32);
+            base[ml1_swz(n, k)] = h;
+            base[NP * 32 + ml1_swz(n, k)] = v - h;
+        } else {
+            float* base = planes + (self ? (size_t)kb * NsP * 32 : (size_t)nsb * NsP * 32 + (size_t)kb * NgP * 32);
+            if constexpr (PREC == GNNML3_PREC_TF32) {
+                base[ml1_swz(n, k)] = tf32_rn(v);
+            } else {
+                __nv_bfloat16* row = reinterpret_cast<__nv_bfloat16*>(base) + (n >> 3) * 512 + (n & 7) * 64 + (k & 7);
+                row[((k >> 3) ^ (n & 7)) << 3] = __float2bfloat16_rn(v);
+                row[(((k >> 3) + 4) ^ (n & 7)) << 3] = __float2bfloat16_rn(0.f);
+            }
+        }
     }
 }
 
@@ -366,7 +429,7 @@ struct ML1Shape {
     size_t wbytes, smem;
 };
 
-static ML1Shape ml1_shape(int Fi, int Fo, int concat, int dir) {
+static ML1Shape ml1_shape(int Fi, int Fo, int concat, int dir, int prec = GNNML3_PREC_3XTF32) {
     ML1Shape s;
     s.Fop = ml1_c16(Fo);
     s.Fo4 = ml1_c4(Fo);
@@ -386,12 +449,12 @@ static ML1Shape ml1_shape(int Fi, int Fo, int concat, int dir) {
     const int cols = s.colG + s.NgP > s.NsP ? s.colG + s.NgP : s.NsP;
     s.tmem_cols = 32;
     while (s.tmem_cols < cols) s.tmem_cols *= 2;
-    s.wbytes = (size_t)2 * 128 * ((size_t)s.nsb * s.NsP + (size_t)s.ngb * s.NgP);
-    s.smem = 1024 + s.wbytes + 2 * ML1_ABUF + 64;
+    s.wbytes = (size_t)ml1_planes(prec) * 128 * ((size_t)s.nsb * s.NsP + (size_t)s.ngb * s.NgP);
+    s.smem = 1024 + s.wbytes + (size_t)2 * ml1_planes(prec) * ML1_APLANE + 64;
     return s;
 }
 
-// workspace layout: [planes | GG | dcat | csum | colsum scratch | gemm_tn scratch]
+// workspace layout: [planes | GG | dcat | csum | colsum scratch | gemm_tn scratch]; sized by the 3xTF32 shapes, the largest
 struct ML1Ws {
     size_t planes, gg, dcat, csum, cs, tn, total_fwd, total;
     int64_t ldgg;
@@ -414,15 +477,39 @@ static ML1Ws ml1_ws(int64_t N, int Fi, int Fo, int concat) {
     return w;
 }
 
-template <bool AUX = true>
+template <bool AUX, int PREC>
 static int ml1_launch(const ML1Params& P, size_t smem, cudaStream_t st) {
     static bool configured[64] = {};
     if (auto once = first_use_on_device(configured))
-        GNNML3_CUDA(cudaFuncSetAttribute(k_ml1_agg_proj<AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+        GNNML3_CUDA(cudaFuncSetAttribute(k_ml1_agg_proj<AUX, PREC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     const int grid = P.n_tiles < kNumSMs ? P.n_tiles : kNumSMs;
-    k_ml1_agg_proj<AUX><<<grid, ML1_THREADS, smem, st>>>(P);
+    k_ml1_agg_proj<AUX, PREC><<<grid, ML1_THREADS, smem, st>>>(P);
     GNNML3_LAUNCH_CHECK();
     return GNNML3_OK;
+}
+
+// the instantiation of (aux written, precision)
+static int ml1_launch(const ML1Params& P, size_t smem, bool aux, int prec, cudaStream_t st) {
+    if (prec == GNNML3_PREC_TF32) return aux ? ml1_launch<true, GNNML3_PREC_TF32>(P, smem, st) : ml1_launch<false, GNNML3_PREC_TF32>(P, smem, st);
+    if (prec == GNNML3_PREC_BF16) return aux ? ml1_launch<true, GNNML3_PREC_BF16>(P, smem, st) : ml1_launch<false, GNNML3_PREC_BF16>(P, smem, st);
+    return aux ? ml1_launch<true, GNNML3_PREC_3XTF32>(P, smem, st) : ml1_launch<false, GNNML3_PREC_3XTF32>(P, smem, st);
+}
+
+static int ml1_prep(const float* wc, const float* wA, const float* wB, const float* wC, int Fi, int Fo, int dir, const ML1Shape& s,
+                    int prec, float* planes, cudaStream_t st) {
+    const int grid = cdiv((int64_t)s.wbytes / (4 * ml1_planes(prec)), 256);     // one thread per weight
+    if (prec == GNNML3_PREC_TF32)
+        k_ml1_prep<GNNML3_PREC_TF32><<<grid, 256, 0, st>>>(wc, wA, wB, wC, Fi, Fo, dir, s.nsb, s.NsP, s.ngb, s.NgP, s.Fop, s.Fo4, planes);
+    else if (prec == GNNML3_PREC_BF16)
+        k_ml1_prep<GNNML3_PREC_BF16><<<grid, 256, 0, st>>>(wc, wA, wB, wC, Fi, Fo, dir, s.nsb, s.NsP, s.ngb, s.NgP, s.Fop, s.Fo4, planes);
+    else
+        k_ml1_prep<GNNML3_PREC_3XTF32><<<grid, 256, 0, st>>>(wc, wA, wB, wC, Fi, Fo, dir, s.nsb, s.NsP, s.ngb, s.NgP, s.Fop, s.Fo4, planes);
+    GNNML3_LAUNCH_CHECK();
+    return GNNML3_OK;
+}
+
+static bool ml1_prec_ok(int prec) {
+    return prec == GNNML3_PREC_3XTF32 || prec == GNNML3_PREC_TF32 || prec == GNNML3_PREC_BF16;
 }
 
 }  // namespace gnnml3
@@ -438,11 +525,12 @@ extern "C" size_t gnnml3_ml1layer_workspace_bytes(int64_t N, int Fi, int Fo, int
     return ml1_ws(N, Fi, Fo, concat).total;
 }
 
-extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x, int64_t ldx,
-                                       int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
-                                       const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat,
-                                       float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh,
-                                       void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" int gnnml3_ml1layer_forward_precision(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x,
+                                                 int64_t ldx, int Fi, const float* wconv, const float* bconv, const float* wA,
+                                                 const float* bA, const float* wB, const float* bB, const float* wC, const float* bC,
+                                                 int Fo, int concat, float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside,
+                                                 int64_t ldh, void* workspace, size_t workspace_bytes, void* stream, int precision) {
+    GNNML3_REQUIRE(ml1_prec_ok(precision), "ml1layer_forward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
     GNNML3_REQUIRE(gnnml3_ml1layer_supported(Fi, Fo, concat), "ml1layer_forward: unsupported shape Fi=%d Fo=%d", Fi, Fo);
     GNNML3_REQUIRE(N >= 0 && E >= 0 && rowptr && x && wconv && wA && wB && wC && y, "ml1layer_forward: NULL pointer");
     GNNML3_REQUIRE(E == 0 || col, "ml1layer_forward: NULL col");
@@ -454,11 +542,10 @@ extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col
     if (workspace_bytes < w.total_fwd) return set_err(GNNML3_ERR_WORKSPACE, "ml1layer_forward: workspace too small");
     if (N == 0) return GNNML3_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    const ML1Shape s = ml1_shape(Fi, Fo, concat, 0);
+    const ML1Shape s = ml1_shape(Fi, Fo, concat, 0, precision);
     float* planes = (float*)((uint8_t*)workspace + w.planes);
-    k_ml1_prep<<<cdiv((int64_t)s.wbytes / 8, 256), 256, 0, st>>>(wconv, wA, wB, wC, Fi, Fo, 0, s.nsb, s.NsP, s.ngb, s.NgP, s.Fop, s.Fo4,
-                                                                  planes);
-    GNNML3_LAUNCH_CHECK();
+    int rc;
+    if ((rc = ml1_prep(wconv, wA, wB, wC, Fi, Fo, 0, s, precision, planes, st))) return rc;
     ML1Params P = {};
     P.rowptr = rowptr; P.col = col; P.N = N; P.n_tiles = cdiv(N, ML1_ROWS);
     P.X = x; P.ldx = ldx; P.Fg = Fi; P.ngb = s.ngb;
@@ -467,15 +554,26 @@ extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col
     P.project = 1; P.epi = concat ? 2 : 1; P.Fo = Fo; P.Fop = s.Fop;
     P.bA = bA; P.bB = bB; P.bC = bC; P.bc = bconv;
     P.out = y; P.ldo = ldy; P.aux = aux; P.ldaux = ldaux; P.hout = hside; P.ldh = ldh;
-    return aux ? ml1_launch<true>(P, s.smem, st) : ml1_launch<false>(P, s.smem, st);     // no aux: the forward-only instantiation
+    return ml1_launch(P, s.smem, aux != nullptr, precision, st);     // no aux: the forward-only instantiation
 }
 
-extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
-                                        int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
-                                        const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
-                                        int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
-                                        float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
-                                        void* stream) {
+extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x, int64_t ldx,
+                                       int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
+                                       const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat,
+                                       float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh,
+                                       void* workspace, size_t workspace_bytes, void* stream) {
+    return gnnml3_ml1layer_forward_precision(rowptr, col, N, E, x, ldx, Fi, wconv, bconv, wA, bA, wB, bB, wC, bC, Fo, concat, y, ldy,
+                                             aux, ldaux, hside, ldh, workspace, workspace_bytes, stream, GNNML3_PREC_3XTF32);
+}
+
+extern "C" int gnnml3_ml1layer_backward_precision(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x,
+                                                  int64_t ldx, int Fi, const float* wconv, const float* wA, const float* wB,
+                                                  const float* wC, int Fo, int concat, const float* y, int64_t ldy, const float* aux,
+                                                  int64_t ldaux, const float* gy, int64_t ldgy, int need_dx, float* dx, int64_t lddx,
+                                                  float* dwconv, float* dbconv, float* dwA, float* dbA, float* dwB, float* dbB,
+                                                  float* dwC, float* dbC, void* workspace, size_t workspace_bytes, void* stream,
+                                                  int precision) {
+    GNNML3_REQUIRE(ml1_prec_ok(precision), "ml1layer_backward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
     GNNML3_REQUIRE(gnnml3_ml1layer_supported(Fi, Fo, concat), "ml1layer_backward: unsupported shape Fi=%d Fo=%d", Fi, Fo);
     GNNML3_REQUIRE(N > 0, "ml1layer_backward: empty batch");
     GNNML3_REQUIRE(E >= 0 && rowptrT && (E == 0 || colT) && x && wconv && wA && wB && wC && y && aux && gy && dwconv && dwA && dwB && dwC,
@@ -486,7 +584,7 @@ extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* c
     if (workspace_bytes < w.total) return set_err(GNNML3_ERR_WORKSPACE, "ml1layer_backward: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
     uint8_t* ws = (uint8_t*)workspace;
-    const ML1Shape s = ml1_shape(Fi, Fo, concat, 1);
+    const ML1Shape s = ml1_shape(Fi, Fo, concat, 1, precision);
     const int Fo4 = s.Fo4;
     float* GG = (float*)(ws + w.gg);
     k_ml1_act_bwd<<<cdiv(N * Fo4, 256) > 4 * kNumSMs * 8 ? 4 * kNumSMs * 8 : cdiv(N * Fo4, 256), 256, 0, st>>>(
@@ -494,11 +592,8 @@ extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* c
     GNNML3_LAUNCH_CHECK();
     // dx = (A^T gc) Wc^T + [gA | gP p2 | gP p1] [fcA ; fcB ; fcC]; the aggregate A^T gc lands in block 3 of GG either way
     float* planes = (float*)(ws + w.planes);
-    if (need_dx) {
-        k_ml1_prep<<<cdiv((int64_t)s.wbytes / 8, 256), 256, 0, st>>>(wconv, wA, wB, wC, Fi, Fo, 1, s.nsb, s.NsP, s.ngb, s.NgP, s.Fop,
-                                                                      Fo4, planes);
-        GNNML3_LAUNCH_CHECK();
-    }
+    int rc;
+    if (need_dx && (rc = ml1_prep(wconv, wA, wB, wC, Fi, Fo, 1, s, precision, planes, st))) return rc;
     ML1Params P = {};
     P.rowptr = rowptrT; P.col = colT; P.N = N; P.n_tiles = cdiv(N, ML1_ROWS);
     P.X = GG + 4 * Fo4; P.ldx = w.ldgg; P.Fg = Fo; P.ngb = s.ngb;
@@ -506,15 +601,27 @@ extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* c
     P.planes = planes; P.wbytes = need_dx ? (int)s.wbytes : 0; P.NsP = s.NsP; P.NgP = s.NgP; P.colG = 0; P.tmem_cols = s.tmem_cols;
     P.project = need_dx ? 1 : 0; P.epi = 0; P.out = dx; P.ldo = lddx; P.Nout = Fi;
     P.hout = GG + 3 * Fo4; P.ldh = w.ldgg;
-    int rc;
-    if ((rc = ml1_launch(P, need_dx ? s.smem : 1024 + 2 * ML1_ABUF + 64, st))) return rc;
-    // [dfcA^T | dfcB^T | dfcC^T | dWc] = x^T GG[:, 0:4 Fo4] in one contraction; bias gradients = column sums (fixed order)
+    if ((rc = ml1_launch(P, need_dx ? s.smem : 1024 + 2 * ML1_ABUF + 64, true, precision, st))) return rc;
+    // [dfcA^T | dfcB^T | dfcC^T | dWc] = x^T GG[:, 0:4 Fo4] in one contraction (single-pass TF32 in the flagged modes, as the
+    // stand-alone GEMMs run BF16); bias gradients = column sums (fixed order)
     float* dcat = (float*)(ws + w.dcat);
     float* csum = (float*)(ws + w.csum);
-    if ((rc = gnnml3_gemm_tn(x, ldx, GG, w.ldgg, dcat, 4 * Fo4, N, Fi, 4 * Fo4, GNNML3_PREC_3XTF32, ws + w.tn, w.total - w.tn, stream)))
+    const int tn_prec = precision == GNNML3_PREC_3XTF32 ? GNNML3_PREC_3XTF32 : GNNML3_PREC_TF32;
+    if ((rc = gnnml3_gemm_tn(x, ldx, GG, w.ldgg, dcat, 4 * Fo4, N, Fi, 4 * Fo4, tn_prec, ws + w.tn, w.total - w.tn, stream)))
         return rc;
     if ((rc = gnnml3_colsum(GG, w.ldgg, N, 5 * Fo4, csum, ws + w.cs, w.tn - w.cs, stream))) return rc;
     k_ml1_unpack<<<cdiv(4 * Fi * Fo + 4 * Fo, 256), 256, 0, st>>>(dcat, csum, Fi, Fo, Fo4, dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC);
     GNNML3_LAUNCH_CHECK();
     return GNNML3_OK;
+}
+
+extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
+                                        int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
+                                        const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
+                                        int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
+                                        float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
+                                        void* stream) {
+    return gnnml3_ml1layer_backward_precision(rowptrT, colT, N, E, x, ldx, Fi, wconv, wA, wB, wC, Fo, concat, y, ldy, aux, ldaux, gy,
+                                              ldgy, need_dx, dx, lddx, dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC, workspace,
+                                              workspace_bytes, stream, GNNML3_PREC_3XTF32);
 }

@@ -63,6 +63,16 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
         "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// same with BF16 inputs (kind::f16, K = 16 per instruction = 32 bytes of a K-major row), FP32 accumulate
+__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
+        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // arrive on an mbarrier once all previously issued tcgen05.mma of this thread have completed
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -124,6 +134,11 @@ __device__ __forceinline__ float tf32_rn(float v) {
 __host__ __device__ constexpr uint32_t make_idesc_tf32_mn(int M, int N, bool a_mn = false, bool b_mn = false) {
     return (1u << 4) | (2u << 7) | (2u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
            ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+
+// instruction descriptor of tcgen05.mma kind::f16 with BF16 A / B (K-major) and FP32 D
+__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
+    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
 }  // namespace gnnml3

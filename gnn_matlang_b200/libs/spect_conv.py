@@ -681,18 +681,21 @@ class _ML1LayerFn(torch.autograd.Function):
     Backward: G = [gA | gP p2 | gP p1] from the masks of y; dx = (A^T gc) Wc^T + G [WA ; WB ; WC] (one fused kernel over the
     transposed CSR); [dWA^T | dWB^T | dWC^T | dWc] = x^T [G | A^T gc] (one contraction); biases = column sums of G and gc.
 
-    ``save`` False (a forward nobody differentiates): the kernel stores y alone, without [p1 | p2], and nothing is saved."""
+    ``save`` False (a forward nobody differentiates): the kernel stores y alone, without [p1 | p2], and nothing is saved.
+    ``precision`` (PREC_*) is the arithmetic of the layer's projections in both directions."""
 
     @staticmethod
-    def forward(ctx, x, wconv, bconv, wA, bA, wB, bB, wC, bC, plan, concat, save=True):
+    def forward(ctx, x, wconv, bconv, wA, bA, wB, bB, wC, bC, plan, concat, precision=_lib.PREC_3XTF32, save=True):
         xa = ops.aligned_rows(x)
         ws = [w.contiguous() for w in (wconv, wA, wB, wC)]
         bs = [b.contiguous() if b is not None else None for b in (bconv, bA, bB, bC)]
         if save:
-            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat)
+            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat,
+                                             precision=precision)
         else:
-            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat, aux=False)
-        ctx.plan, ctx.concat = plan, concat
+            y, aux, _ = ops.ml1layer_forward(plan, xa, ws[0], bs[0], ws[1], bs[1], ws[2], bs[2], ws[3], bs[3], concat=concat, aux=False,
+                                             precision=precision)
+        ctx.plan, ctx.concat, ctx.precision = plan, concat, precision
         ctx.has_bias = tuple(b is not None for b in (bconv, bA, bB, bC))
         if save:
             ctx.save_for_backward(xa, *ws, y, aux)
@@ -706,13 +709,13 @@ class _ML1LayerFn(torch.autograd.Function):
         if N == 0:
             z = torch.zeros_like
             bz = [torch.zeros(wconv.size(2), device=xa.device) if h else None for h in ctx.has_bias]
-            return z(xa), z(wconv), bz[0], z(wA), bz[1], z(wB), bz[2], z(wC), bz[3], None, None, None
+            return z(xa), z(wconv), bz[0], z(wA), bz[1], z(wB), bz[2], z(wC), bz[3], None, None, None, None
         gy = gy if gy.stride(1) == 1 else gy.contiguous()
         dx, dwc, dbc, dwA, dbA, dwB, dbB, dwC, dbC = ops.ml1layer_backward(ctx.plan, xa, wconv, wA, wB, wC, y, aux, gy, need[0],
-                                                                          concat=ctx.concat)
+                                                                          concat=ctx.concat, precision=ctx.precision)
         hb = ctx.has_bias
         return (dx, dwc, dbc if hb[0] else None, dwA, dbA if hb[1] else None, dwB, dbB if hb[2] else None, dwC,
-                dbC if hb[3] else None, None, None, None)
+                dbC if hb[3] else None, None, None, None, None)
 
 
 class ML1Layer(torch.nn.Module):
@@ -723,11 +726,14 @@ class ML1Layer(torch.nn.Module):
     ``conv1`` is a ``SpectConv(ninp, nout, K=1, selfconn=False)`` on the graph's plain ``edge_index`` with every edge weight
     one; ``fc11``, ``fc12``, ``fc13`` are ``nn.Linear(ninp, nout)``.  ``forward(x, edge_index)`` -> [N, nout] (or [N, 3 nout]).
     Shapes with ninp, nout <= 64 run as one fused library call per direction; larger ones are composed from the aggregation
-    kernel and the tensor-core GEMMs of this library, with the same result."""
+    kernel and the tensor-core GEMMs of this library, with the same result.  ``precision`` ("fp32" = 3xTF32, "tf32", "bf16"):
+    the arithmetic of the projections, as for ML3Layer; aggregation, epilogues and outputs stay float32."""
 
-    def __init__(self, ninp, nout, concat=False):
+    def __init__(self, ninp, nout, concat=False, precision="fp32"):
         super(ML1Layer, self).__init__()
+        _check_precision(precision)
         self.concat = bool(concat)
+        self.precision = precision
         self.conv1 = SpectConv(ninp, nout, 1, selfconn=False)
         self.fc11 = torch.nn.Linear(ninp, nout)
         self.fc12 = torch.nn.Linear(ninp, nout)
@@ -738,24 +744,30 @@ class ML1Layer(torch.nn.Module):
         return self.conv1.out_channels * (3 if self.concat else 1)
 
     def forward(self, x, edge_index):
-        return ml1_layer(x, edge_index, self.conv1, self.fc11, self.fc12, self.fc13, self.concat)
+        return ml1_layer(x, edge_index, self.conv1, self.fc11, self.fc12, self.fc13, self.concat, self.precision)
 
 
-def ml1_layer(x, edge_index, conv, fcA, fcB, fcC, concat=False):
+def _check_precision(precision):
+    if precision not in _PRECISIONS:
+        raise ValueError("precision must be one of %s" % sorted(_PRECISIONS))
+
+
+def ml1_layer(x, edge_index, conv, fcA, fcB, fcC, concat=False, precision="fp32"):
     """The GNNML1 layer on given modules (``conv`` a SpectConv(K=1, selfconn=False), ``fcA``/``fcB``/``fcC`` nn.Linear):
-    what ``ML1Layer.forward`` and ``models.GNNML1`` run."""
+    what ``ML1Layer.forward`` and ``models.GNNML1`` run, in ``precision`` ("fp32", "tf32" or "bf16")."""
+    _check_precision(precision)
     if not (x.is_cuda and edge_index.is_cuda):
         raise RuntimeError("gnn_matlang_b200: x and edge_index must be CUDA tensors (the B200 hot path has no CPU fallback)")
     if x.dim() != 2 or x.dtype != torch.float32:
         raise RuntimeError("gnn_matlang_b200: x [N, F] must be float32")
     plan = get_plan(edge_index, x.size(0))
     Fi, Fo = conv.in_channels, conv.out_channels
+    prec = _PRECISIONS[precision]
     if ops.ml1layer_supported(Fi, Fo, concat):
         ML1_PATH_COUNTS["fused"] += 1
         ps = (conv.weight, conv.bias, fcA.weight, fcA.bias, fcB.weight, fcB.bias, fcC.weight, fcC.bias)
-        return _ML1LayerFn.apply(x, *ps, plan, bool(concat), _needs_save(x, *ps))
+        return _ML1LayerFn.apply(x, *ps, plan, bool(concat), prec, _needs_save(x, *ps))
     ML1_PATH_COUNTS["composed"] += 1
-    prec = _lib.PREC_3XTF32
     ones = torch.ones(plan.E, 1, dtype=torch.float32, device=x.device)
     ax = _AggregateFn.apply(x, ones, plan)
     pa = _LinearFn.apply(x, fcA.weight.t(), fcA.bias, prec)

@@ -26,7 +26,7 @@ preset (``graph8c``, ``zinc``, ``exp``, ``counting``).
 import torch
 import torch.nn as nn
 
-from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _PRECISIONS, ml1_layer
+from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _PRECISIONS, _check_precision, ml1_layer
 import torch.nn.functional as F
 
 from .pool import global_add_pool, global_max_pool, global_mean_pool
@@ -103,14 +103,17 @@ class GNNML1(nn.Module):
     form with ``concat=True``: layer width 3 * nout), then the read-out and head of ``MODEL_CONFIGS[config]``.  Parameters keep
     the reference's names: ``conv{l}1`` (SpectConv(K=1, selfconn=False)), ``fc{l}1``, ``fc{l}2``, ``fc{l}3`` (nn.Linear) for
     l = 1..nlayer, then the head (``fc1``, ``fc2``).  ``forward(data)`` reads ``data.x``, ``data.edge_index``, ``data.batch``
-    (``batch.collate(graphs, adjacency=True)`` provides ``edge_index``)."""
+    (``batch.collate(graphs, adjacency=True)`` provides ``edge_index``).  ``precision`` ("fp32" = 3xTF32, "tf32", "bf16") is
+    the arithmetic of every layer's projections and of the head, as for GNNML3; parameters are the same in every mode."""
 
-    def __init__(self, config, ninp, nlayer=3, nout=64, concat=False):
+    def __init__(self, config, ninp, nlayer=3, nout=64, concat=False, precision="fp32"):
         super().__init__()
         if isinstance(config, str) and config not in GNNML1_PRESETS:
             raise ValueError("GNNML1 presets: %s" % (GNNML1_PRESETS,))
+        _check_precision(precision)
         c = dict(MODEL_CONFIGS[config]) if isinstance(config, str) else dict(config)
         self.cfg = c
+        self.precision = precision
         self.nlayer, self.concat = int(nlayer), bool(concat)
         width = nout * (3 if concat else 1)
         for l in range(1, self.nlayer + 1):
@@ -128,12 +131,12 @@ class GNNML1(nn.Module):
         edge_index = data.edge_index
         for l in range(1, self.nlayer + 1):
             x = ml1_layer(x, edge_index, getattr(self, "conv%d1" % l), getattr(self, "fc%d1" % l), getattr(self, "fc%d2" % l),
-                          getattr(self, "fc%d3" % l), self.concat)
+                          getattr(self, "fc%d3" % l), self.concat, self.precision)
         c = self.cfg
         B = getattr(data, "num_graphs", None)
         pool = {"add": global_add_pool, "mean": global_mean_pool}[c["pool"]]
         x = pool(x, data.batch, B)
-        prec = _PRECISIONS["fp32"]
+        prec = _PRECISIONS[self.precision]
         x = _LinearFn.apply(x, self.fc1.weight.t(), self.fc1.bias, prec)
         if len(c["head"]) == 1:
             return torch.tanh(x) if c["final"] == "tanh" else x

@@ -565,11 +565,13 @@ def ml1layer_supported(Fi, Fo, concat=False):
     return bool(_lib.load().gnnml3_ml1layer_supported(int(Fi), int(Fo), int(bool(concat))))
 
 
-def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False, keep_aggregate=False, aux=True):
+def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False, keep_aggregate=False, aux=True,
+                     precision=_lib.PREC_3XTF32):
     """Whole GNNML1 layer forward in one library call (gnnml3_ml1layer_forward) over the plan of the plain ``edge_index``.
     x [N, Fi] must satisfy ``aligned_rows``; wconv [1, Fi, Fo]; wA/wB/wC [Fo, Fi].  -> (y [N, Fo] or [N, 3 Fo],
     aux [N, 2 Fo] = [p1 | p2] (None with ``aux=False``: a forward nobody differentiates stores y alone),
-    A x [N, Fi] if ``keep_aggregate`` else None)"""
+    A x [N, Fi] if ``keep_aggregate`` else None).  ``precision`` (PREC_3XTF32 | PREC_TF32 | PREC_BF16): the arithmetic of the
+    projection (gnnml3_ml1layer_forward_precision for the flagged modes)."""
     lib = _lib.load()
     N, Fi = x.shape
     Fo = wconv.size(2)
@@ -580,17 +582,20 @@ def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False
     hside = _padded_rows(N, Fi, dev) if keep_aggregate else None
     ws = _ws(dev, lib.gnnml3_ml1layer_workspace_bytes(N, Fi, Fo, int(bool(concat))), tag="ml1")
     p = _lib.ptr
+    args = (p(plan.rowptr), p(plan.col), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(bconv), p(wA), p(bA), p(wB), p(bB), p(wC), p(bC), Fo,
+            int(bool(concat)), p(y), _ld(y) if N > 1 else (W + 3) // 4 * 4, p(aux), 2 * Fo, p(hside), (Fi + 3) // 4 * 4, p(ws), ws.numel(),
+            _lib.stream_ptr())
     with _on(dev):
-        _lib.check(lib.gnnml3_ml1layer_forward(p(plan.rowptr), p(plan.col), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(bconv), p(wA), p(bA),
-                                               p(wB), p(bB), p(wC), p(bC), Fo, int(bool(concat)), p(y), _ld(y) if N > 1 else (W + 3) // 4 * 4,
-                                               p(aux), 2 * Fo, p(hside), (Fi + 3) // 4 * 4, p(ws), ws.numel(), _lib.stream_ptr()),
-                   "gnnml3_ml1layer_forward")
+        if precision == _lib.PREC_3XTF32:
+            _lib.check(lib.gnnml3_ml1layer_forward(*args), "gnnml3_ml1layer_forward")
+        else:
+            _lib.check(lib.gnnml3_ml1layer_forward_precision(*args, int(precision)), "gnnml3_ml1layer_forward_precision")
     return y, aux, hside
 
 
-def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=False):
-    """Whole GNNML1 layer backward in one library call (gnnml3_ml1layer_backward).
-    -> dx (None unless need_dx), dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC"""
+def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=False, precision=_lib.PREC_3XTF32):
+    """Whole GNNML1 layer backward in one library call (gnnml3_ml1layer_backward, or its _precision form for a flagged
+    ``precision``).  -> dx (None unless need_dx), dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC"""
     lib = _lib.load()
     N, Fi = x.shape
     Fo = wconv.size(2)
@@ -603,11 +608,14 @@ def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=Fa
     dbs = torch.empty(4, Fo, **f32)                      # conv | fcA | fcB | fcC
     ws = _ws(dev, lib.gnnml3_ml1layer_workspace_bytes(N, Fi, Fo, int(bool(concat))), tag="ml1")
     p = _lib.ptr
-    with _on(dev):
-        _lib.check(lib.gnnml3_ml1layer_backward(
-            p(plan.rowptrT), p(plan.colT), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(wA), p(wB), p(wC), Fo, int(bool(concat)),
+    args = (p(plan.rowptrT), p(plan.colT), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(wA), p(wB), p(wC), Fo, int(bool(concat)),
             p(y), _ld(y) if N > 1 else y.size(1), p(aux), 2 * Fo, p(gy), _ld(gy), int(bool(need_dx)), p(dx), lddx, p(dwc), p(dbs[0]),
-            p(dwA), p(dbs[1]), p(dwB), p(dbs[2]), p(dwC), p(dbs[3]), p(ws), ws.numel(), _lib.stream_ptr()), "gnnml3_ml1layer_backward")
+            p(dwA), p(dbs[1]), p(dwB), p(dbs[2]), p(dwC), p(dbs[3]), p(ws), ws.numel(), _lib.stream_ptr())
+    with _on(dev):
+        if precision == _lib.PREC_3XTF32:
+            _lib.check(lib.gnnml3_ml1layer_backward(*args), "gnnml3_ml1layer_backward")
+        else:
+            _lib.check(lib.gnnml3_ml1layer_backward_precision(*args, int(precision)), "gnnml3_ml1layer_backward_precision")
     return (dx[:, :Fi] if need_dx else None), dwc, dbs[0], dwA, dbs[1], dwB, dbs[2], dwC, dbs[3]
 
 

@@ -43,9 +43,11 @@ extern "C" {
 #define GNNML3_ERR_CUDA 2        /* a CUDA runtime call or kernel launch failed */
 #define GNNML3_ERR_WORKSPACE 3   /* workspace too small */
 
-/* GEMM arithmetic: FP32-grade error-compensated 3xTF32 (default, meets rtol 1e-5), single-pass TF32. */
+/* GEMM arithmetic: FP32-grade error-compensated 3xTF32 (default, meets rtol 1e-5), single-pass TF32.  BF16 inputs with FP32
+ * accumulation: the GNNML1 layer (gnnml3_ml1layer_*_precision); the stand-alone GEMMs take it as single-pass TF32. */
 #define GNNML3_PREC_3XTF32 0
 #define GNNML3_PREC_TF32 1
+#define GNNML3_PREC_BF16 2
 
 /* precision flags OR-ed into the `epilogue` argument of gnnml3_fused_agg_proj (tensor-memory kernel only): one tensor-core
  * product per k-step on TF32-truncated / BF16-rounded inputs instead of the FP32-grade 3xTF32 triple; FP32 accumulation.
@@ -260,14 +262,21 @@ GNNML3_API int gnnml3_ml3layer_backward(const int32_t* rowptr, const int32_t* co
  *   concat = 0: y = relu(p0 + p1 * p2)                                                        [N, Fo]
  *   concat = 1: y = [relu(x wA^T + bA) | relu((A x) wconv[0] + bconv) | relu(p1 * p2)]         [N, 3 Fo]
  * One fused kernel per direction: the aggregate and the four projections meet in tensor memory (tcgen05, 3xTF32, FP32-grade).
+ * The *_precision entry points take the same arguments plus the projection's arithmetic: GNNML3_PREC_3XTF32 (what the plain
+ * entry points run), GNNML3_PREC_TF32 (one MMA per k-step on the raw FP32 operand, truncated by the tensor core, and RN-TF32
+ * weights) or GNNML3_PREC_BF16 (RN-BF16 operands and weights); anything else is GNNML3_ERR_INVALID.  In every mode the
+ * aggregation (FP32 sums in CSR order), the epilogues, y / aux / dx (float32) and determinism are unchanged; the weight
+ * gradient contraction runs at GNNML3_PREC_TF32 in both flagged modes.  Stated tolerances (tests/test_gpu_gnnml1_precision.py):
+ * TF32 2e-3, BF16 2e-2 of the result's scale.
  *   forward : rowptr / col = the dst-sorted CSR of edge_index (gnnml3_csr_build); outputs y [N, ldy] and aux [N, ldaux >= 2 Fo]
  *             = [p1 | p2] (saved for the backward); hside (nullable, [N, ldh >= Fi]) receives A x.  Biases are nullable.
  *             aux may be NULL (inference): a forward-only instantiation of the kernel then stores y alone (a third of the
  *             sum-mode stores).  The backward requires the aux of a forward that wrote it.
  *   backward: rowptrT / colT = the transposed CSR; gy [N, ldgy]; dx [N, lddx] if need_dx (else dx may be NULL: the aggregate
  *             A^T gc is still formed for d wconv); outputs the eight parameter gradients (dw* overwritten; db* nullable).
- * Supported: 1 <= Fi <= 64, 1 <= Fo <= 64 (gnnml3_ml1layer_supported), E = 0 allowed; x rows 16-byte aligned (ldx % 4 == 0).
- * Deterministic (fixed summation order, no atomics), no host sync; caller-provided workspace.
+ * Supported: 1 <= Fi <= 64, 1 <= Fo <= 64 (gnnml3_ml1layer_supported) in every precision, E = 0 allowed; x rows 16-byte
+ * aligned (ldx % 4 == 0).  Deterministic (fixed summation order, no atomics), no host sync; caller-provided workspace
+ * (gnnml3_ml1layer_workspace_bytes covers every precision).
  * --------------------------------------------------------------------------------------------------- */
 GNNML3_API int gnnml3_ml1layer_supported(int Fi, int Fo, int concat);
 GNNML3_API size_t gnnml3_ml1layer_workspace_bytes(int64_t N, int Fi, int Fo, int concat);
@@ -282,6 +291,17 @@ GNNML3_API int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* c
                              int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
                              float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
                              void* stream);
+GNNML3_API int gnnml3_ml1layer_forward_precision(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x,
+                            int64_t ldx, int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
+                            const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat, float* y,
+                            int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh, void* workspace,
+                            size_t workspace_bytes, void* stream, int precision);
+GNNML3_API int gnnml3_ml1layer_backward_precision(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x,
+                             int64_t ldx, int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo,
+                             int concat, const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy,
+                             int64_t ldgy, int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA,
+                             float* dbA, float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
+                             void* stream, int precision);
 
 /* ---------------------------------------------------------------------------------------------------
  * Readout: PyG global_add_pool (mean = 0) / global_mean_pool (mean = 1) over contiguous node ranges

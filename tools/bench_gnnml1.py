@@ -16,6 +16,10 @@
   eager step on fresh batches (so that both arms build the CSR); captured against eager at batch 64; the host's
   ``collate(adjacency=True)`` (the feed without this data path) at both batch sizes; one ``gnnml3_collate_graphs`` call at the
   bench batch with its algorithmic bytes;
+* the precision modes (key ``precision``): for each of ``fp32`` (3xTF32), ``tf32`` and ``bf16`` the captured ``zinc`` training
+  step at the bench batch from the resident ``DeviceDataset``, the ``no_grad`` forward of the bench batch, one layer call and
+  the fused kernel at 64 -> 64 (forward and dx), and the largest deviation of loss, outputs and gradients from the fp32 run on
+  the same batch and weights; the arms alternate within every round;
 * the card's name and power limit, read in the same run.
 
     python tools/bench_gnnml1.py [--batch 8192] [--steps 20] [--warmup 5] [--rounds 3] [--pool 65536] [--out FILE]
@@ -114,6 +118,118 @@ def _events(fn, steps):
 
 def _strip(hb):
     return hb.__class__(**{k: v for k, v in hb.__dict__.items() if k not in ("edge_index2", "edge_attr2")})
+
+
+def kernel_us(fn, reps=20):
+    """Device time per call of each ml1 kernel that ``fn`` launches (torch.profiler), microseconds."""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    out = {}
+    for evt in prof.key_averages():
+        if evt.device_type.name == "CUDA" and "ml1" in evt.key:
+            t = getattr(evt, "device_time_total", None) or getattr(evt, "cuda_time_total", 0)
+            out[evt.key.split("(")[0].split("<")[0]] = t / max(evt.count, 1)
+    return out
+
+
+def precision_path(a, d, b):
+    """GNNML1 in its three precisions on the same batch ``b``, weights and id lists; arms alternate within every round."""
+    from gnn_matlang_b200 import ops
+    from gnn_matlang_b200.graph import get_plan
+    from gnn_matlang_b200.libs.spect_conv import _PRECISIONS
+    from gnn_matlang_b200.models import GNNML1
+    from gnn_matlang_b200.synthetic import DeviceDataset, GraphPool
+    from gnn_matlang_b200.train import GraphedTrainer, pad_batch, padded_shapes
+    precs = ("fp32", "tf32", "bf16")
+    out = {"modes": {p: {} for p in precs}}
+    # deviation from fp32: one forward + L1-sum loss + backward per mode, identical weights, before any update
+    ref = {}
+    for p in precs:
+        torch.manual_seed(0)
+        m = GNNML1("zinc", ninp=25, precision=p).to(d)
+        o = m(b)
+        loss = (o.view(-1) - b.y.view(-1)).abs().sum()
+        loss.backward()
+        r = dict(loss=loss.detach().double(), out=o.detach().double(), grads={k: v.grad.double() for k, v in m.named_parameters()})
+        if p == "fp32":
+            ref = r
+        dev_g = {k: float((g - ref["grads"][k]).abs().max() / ref["grads"][k].abs().max().clamp_min(1e-30)) for k, g in r["grads"].items()}
+        out["modes"][p].update(
+            loss=float(r["loss"]), loss_rel_dev_vs_fp32=float((r["loss"] - ref["loss"]).abs() / ref["loss"].abs()),
+            out_max_rel_dev_vs_fp32=float((r["out"] - ref["out"]).abs().max() / ref["out"].abs().max()),
+            grad_max_rel_dev_vs_fp32=max(dev_g.values()), grad_max_rel_dev_param=max(dev_g, key=dev_g.get))
+    pool = GraphPool("zinc", a.pool, seed=11)
+    dds = DeviceDataset(pool, d, adjacency=True, supports=False)
+    rng = np.random.default_rng(2)
+    ids = [rng.integers(0, a.pool, a.batch) for _ in range(8)]
+    host = [_strip(pool.collate(i, adjacency=True)) for i in ids[:2]]
+    Np, _, Mp = padded_shapes([_strip(pool.collate(i, adjacency=True)) for i in ids], adjacency=True)
+    pinned = [torch.from_numpy(i).pin_memory() for i in ids]
+    N = int(b.x.shape[0])
+    plan = get_plan(b.edge_index, N)
+    g = torch.Generator().manual_seed(1)
+    x = torch.randn(N, 64, generator=g).to(d)
+    gy = torch.randn(N, 64, generator=g).to(d)
+    arms, calls = {}, {}
+    for p in precs:
+        torch.manual_seed(0)
+        gt = GraphedTrainer(GNNML1("zinc", ninp=25, precision=p).to(d), pad_batch(host[0], Np, None, Mp), loss="l1")
+        arms["captured_step_" + p] = lambda i, gt=gt: (gt.load_from_dataset(dds, pinned[i % len(pinned)]), gt.step())
+        torch.manual_seed(0)
+        m = GNNML1("zinc", ninp=25, precision=p).to(d)
+
+        def fwd_nograd(i, m=m):
+            with torch.no_grad():
+                m(b)
+        arms["no_grad_forward_" + p] = fwd_nograd
+        L = m.conv21, m.fc21, m.fc22, m.fc23
+        w = [l.weight.detach() for l in L]
+        bs = [l.bias.detach() for l in L]
+        pr = _PRECISIONS[p]
+        y, aux, _ = ops.ml1layer_forward(plan, x, w[0], bs[0], w[1], bs[1], w[2], bs[2], w[3], bs[3], precision=pr)
+        calls["fwd_" + p] = lambda w=w, bs=bs, pr=pr: ops.ml1layer_forward(plan, x, w[0], bs[0], w[1], bs[1], w[2], bs[2], w[3], bs[3],
+                                                                           precision=pr)
+        calls["bwd_" + p] = lambda w=w, y=y, aux=aux, pr=pr: ops.ml1layer_backward(plan, x, w[0], w[1], w[2], w[3], y, aux, gy, True,
+                                                                                   precision=pr)
+        arms["layer_forward_call_" + p] = lambda i, f=calls["fwd_" + p]: f()
+        arms["layer_backward_call_" + p] = lambda i, f=calls["bwd_" + p]: f()
+    for name, fn in arms.items():
+        for i in range(a.warmup):
+            fn(i)
+    torch.cuda.synchronize()
+    times = {k: [] for k in arms}
+    for _ in range(a.rounds):
+        for name, fn in arms.items():
+            times[name].append(_events(fn, a.steps))
+    for p in precs:
+        r = out["modes"][p]
+        r["ms_per_step"] = {k[:-len(p) - 1]: v for k, v in times.items() if k.endswith("_" + p)}
+        best = {k: min(v) for k, v in r["ms_per_step"].items()}
+        r["graphs_per_s_captured"] = a.batch / (best["captured_step"] * 1e-3)
+        r["graphs_per_s_no_grad_forward"] = a.batch / (best["no_grad_forward"] * 1e-3)
+        r["layer_forward_call_ms"], r["layer_backward_call_ms"] = best["layer_forward_call"], best["layer_backward_call"]
+        kf, kb = kernel_us(calls["fwd_" + p]), kernel_us(calls["bwd_" + p])
+        r["forward_kernel_us"] = next(v for k, v in kf.items() if "agg_proj" in k)
+        r["dx_kernel_us"] = next(v for k, v in kb.items() if "agg_proj" in k)
+        r["forward_call_kernels_us"], r["backward_call_kernels_us"] = kf, kb
+    f32 = out["modes"]["fp32"]
+    for p in ("tf32", "bf16"):
+        r = out["modes"][p]
+        r["captured_step_speedup_vs_fp32"] = min(f32["ms_per_step"]["captured_step"]) / min(r["ms_per_step"]["captured_step"])
+        r["no_grad_forward_speedup_vs_fp32"] = min(f32["ms_per_step"]["no_grad_forward"]) / min(r["ms_per_step"]["no_grad_forward"])
+        r["forward_kernel_speedup_vs_fp32"] = f32["forward_kernel_us"] / r["forward_kernel_us"]
+        r["dx_kernel_speedup_vs_fp32"] = f32["dx_kernel_us"] / r["dx_kernel_us"]
+    out.update(batch_graphs=a.batch, nodes=N, edges=int(b.edge_index.shape[1]), pool_graphs=a.pool, layer_shape="64 -> 64, sum mode",
+               note=("captured_step: load_from_dataset + graph replay of the zinc preset (L1 loss, Adam); no_grad_forward: the bench "
+                     "batch; ms_per_step and layer_*_call: CUDA events around the timed calls; *_kernel_us and *_call_kernels_us: "
+                     "k_ml1_agg_proj (and the call's other ml1 kernels) device time per launch from a separate torch.profiler pass, "
+                     "not CUDA events; deviations: one forward + backward per mode on the bench batch, same weights"))
+    return out
 
 
 def train_path(a, d):
@@ -303,21 +419,6 @@ def main():
     res["layer_forward_call_ms"] = ev(fwd)
     res["layer_backward_call_ms"] = ev(bwd)
 
-    def kernel_us(fn, reps=20):
-        from torch.profiler import ProfilerActivity, profile
-        fn()
-        torch.cuda.synchronize()
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(reps):
-                fn()
-            torch.cuda.synchronize()
-        out = {}
-        for evt in prof.key_averages():
-            if evt.device_type.name == "CUDA" and "ml1" in evt.key:
-                t = getattr(evt, "device_time_total", None) or getattr(evt, "cuda_time_total", 0)
-                out[evt.key.split("(")[0].split("<")[0]] = t / max(evt.count, 1)
-        return out
-
     kf, kb = kernel_us(fwd), kernel_us(bwd)
     fk = next(v for k, v in kf.items() if "agg_proj" in k)
     bk = next(v for k, v in kb.items() if "agg_proj" in k)
@@ -339,6 +440,7 @@ def main():
         res["graph8c_graphs"] = len(gs)
         res["graph8c_embed_ms"] = ev(lambda: m8(g8), reps=20)
     res["train"] = train_path(a, d)
+    res["precision"] = precision_path(a, d, b)
     line = json.dumps(res)
     print(line)
     if a.out:
