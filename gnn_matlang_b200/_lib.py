@@ -94,6 +94,8 @@ SIGNATURES = {
     "gnnml3_spectral_count": (_i, [_p, _i64, _p, _p, _i, _i, _i, _p, _p]),
     "gnnml3_spectral_design": (_i, [_p, _i64, _p, _p, _i, _i, ctypes.c_double, _i, _i, _i, _i, ctypes.c_double, _i, _p, _i, _p,
                                     _i64, _p, _p, _p, _p]),
+    "gnnml3_pairs_mark": (_i, [_p, _i64, _i64, _i, _p, _i64, ctypes.c_float, _p, _i64, _p]),
+    "gnnml3_pairs_count": (_i, [_p, _i64, _i64, _i64, _p, _p]),
 }
 
 PREC_3XTF32 = 0

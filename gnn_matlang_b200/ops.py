@@ -742,6 +742,26 @@ def segment_max_bwd(gout, arg, graph_ptr, N):
     return gx
 
 
+def pairs_mark(emb, bits, wpr, threshold, pairs=None):
+    """OR one seed's embeddings emb [n, d] (float32 CUDA, unit-stride rows) into the pair bitmap ``bits`` (int32 words read as
+    uint32): all pairs i < j (``pairs`` None, ``wpr`` words per row) or the listed pairs ``pairs`` [P, 2] int64."""
+    lib = _lib.load()
+    emb = _rows(emb, "emb")
+    n, d = emb.shape
+    P = 0 if pairs is None else pairs.size(0)
+    with _on(emb.device):
+        _lib.check(lib.gnnml3_pairs_mark(_lib.ptr(emb), _ld(emb), n, d, _lib.ptr(pairs), P, float(threshold), _lib.ptr(bits), wpr,
+                                         _lib.stream_ptr()), "gnnml3_pairs_mark")
+
+
+def pairs_count(bits, n, wpr, P, out):
+    """out (int64 CUDA scalar) = the pairs of the bitmap whose bit is still 0 (P == 0: all pairs of n rows; P > 0: P listed pairs)."""
+    lib = _lib.load()
+    with _on(bits.device):
+        _lib.check(lib.gnnml3_pairs_count(_lib.ptr(bits), n, wpr, P, _lib.ptr(out), _lib.stream_ptr()), "gnnml3_pairs_count")
+    return out
+
+
 # --------------------------------------------------------------------------------------------------
 # optional per-call device timing (CUDA events on the launching stream) used by bench.py
 # --------------------------------------------------------------------------------------------------

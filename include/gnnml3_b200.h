@@ -384,6 +384,26 @@ GNNML3_API int gnnml3_collate_graphs(const int64_t* idx, const int32_t* n, const
                    int64_t* out_edge_index2, float* out_edge_attr2, int64_t* out_edge_index, int64_t* out_batch,
                    int32_t* out_graph_ptr, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Isomorphism test (pairs.cu; graph8c.py:281-302, sr25.py, exp_iso.py): a pair of graphs is distinguished once the L1 distance
+ * of its embeddings, dist = sum_{k=0..d-1} |a_k - b_k| (FP32, summed in dimension order: deterministic), exceeds `threshold`
+ * under any seed.  NaN compares false: a pair whose distance is NaN stays undistinguished, as with the reference's cdist > thr.
+ * Each call ORs one seed's embeddings emb [n, d] (row stride ld >= d) into a bitmap of uint32 words.
+ *   gnnml3_pairs_mark, pairs == NULL (P = 0): every pair i < j < n; bit j of row i is bit (j % 32) of bits[i * wpr + j / 32],
+ *       wpr >= ceil(n / 32).  128 x 128 pair tiles; a tile whose pairs are all marked already does no arithmetic.
+ *   gnnml3_pairs_mark, pairs != NULL: the P listed pairs pairs [P, 2] int64 (row ids in [0, n); a pair with an id outside is
+ *       never marked); bit p is bit (p % 32) of bits[p / 32], bits of ceil(P / 32) words (wpr unused).
+ *   gnnml3_pairs_count: *out (device int64) = the number of pairs whose bit is still 0 -- the undistinguished pairs.  P == 0: the
+ *       all-pairs bitmap of n rows; P > 0: the listed-pairs bitmap of P bits (n and wpr unused).  Fixed-order integer reduction
+ *       in one thread-block cluster.
+ * Returns GNNML3_ERR_INVALID for d < 1, ld < d, a negative n or P, a non-finite or negative threshold, or wpr < ceil(n / 32) in
+ * all-pairs mode.  Bits that stand for no valid pair are ignored and never set.  No host sync; both calls are CUDA-graph
+ * capturable.
+ * --------------------------------------------------------------------------------------------------- */
+GNNML3_API int gnnml3_pairs_mark(const float* emb, int64_t ld, int64_t n, int d, const int64_t* pairs, int64_t P,
+                                 float threshold, uint32_t* bits, int64_t wpr, void* stream);
+GNNML3_API int gnnml3_pairs_count(const uint32_t* bits, int64_t n, int64_t wpr, int64_t P, int64_t* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
