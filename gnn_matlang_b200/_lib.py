@@ -60,7 +60,7 @@ SIGNATURES = {
     "gnnml3_fused_supported": (_i, [_i, _i, _i, _i, _i, _i, _i]),
     "gnnml3_fused_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "gnnml3_fused_agg_proj": (_i, [_p, _p, _p, _p, _i, _i, _p, _i64, _i, _p, _i64, _i, _i, _p, _i64, _p, _i64, _i, _p, _p,
-                                   _i64, _i, _p, _i64, _p, _i64, _i, _i, _p, _i64, _p, _p, _sz, _p]),
+                                   _i64, _i, _p, _i64, _p, _i64, _i, _i, _i, _p, _i64, _p, _p, _sz, _p]),
     "gnnml3_tile_rows": (_i, []),
     "gnnml3_tile_windows": (_i, [_p, _p, _i64, _p, _p]),
     "gnnml3_fused_ts_supported": (_i, [_i, _i, _i, _i, _i, _i, _i]),
@@ -79,13 +79,9 @@ SIGNATURES = {
     "gnnml3_ml1layer_supported": (_i, [_i, _i, _i]),
     "gnnml3_ml1layer_workspace_bytes": (_sz, [_i64, _i, _i, _i]),
     "gnnml3_ml1layer_forward": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64,
-                                     _p, _i64, _p, _sz, _p]),
+                                     _p, _i64, _p, _sz, _p, _i]),
     "gnnml3_ml1layer_backward": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64, _p, _i64, _i,
-                                      _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
-    "gnnml3_ml1layer_forward_precision": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _p, _i64, _p,
-                                               _i64, _p, _i64, _p, _sz, _p, _i]),
-    "gnnml3_ml1layer_backward_precision": (_i, [_p, _p, _i64, _i64, _p, _i64, _i, _p, _p, _p, _p, _i, _i, _p, _i64, _p, _i64, _p, _i64,
-                                                _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
+                                      _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
     "gnnml3_segment_pool_fwd":(_i, [_p, _i64, _p, _i, _i, _i, _p, _p]),
     "gnnml3_segment_pool_bwd": (_i, [_p, _p, _i, _i, _i, _p, _i64, _p]),
     "gnnml3_segment_max_fwd": (_i, [_p, _i64, _p, _i, _i, _p, _p, _p]),
@@ -100,8 +96,7 @@ SIGNATURES = {
 
 PREC_3XTF32 = 0
 PREC_TF32 = 1
-PREC_BF16 = 2          # fused layer kernels only (GNNML3_FUSED_BF16, the GNNML1 layer); the stand-alone GEMMs run it as single-pass TF32
-FUSED_FLAGS = {0: 0, 1: 0x100, 2: 0x200}
+PREC_BF16 = 2          # BF16 in the fused layer kernels; the stand-alone GEMMs run it as single-pass TF32
 EPI_NONE = 0
 EPI_RELU = 1
 

@@ -41,6 +41,9 @@ void count_launch(int n);
 
 static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+static inline bool prec_valid(int prec) {
+    return prec == GNNML3_PREC_3XTF32 || prec == GNNML3_PREC_TF32 || prec == GNNML3_PREC_BF16;
+}
 
 constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 

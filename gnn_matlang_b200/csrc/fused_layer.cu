@@ -944,8 +944,8 @@ namespace gnnml3 {
 int fused_ts_run(const int32_t* rowptr, const int32_t* col, const int32_t* eperm, const float* ea, int Kstride, int K, const float* X,
                  int64_t ldx, int F, const float* S, int64_t lds, int Fs, int self_mode, const float* Bmain, int64_t ldb,
                  const float* Bself, int64_t ldbs, int Ns, const float* bias, const float* bias_s, int64_t N, int Nc, float* out,
-                 int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, float* hout, int64_t ldh, const int32_t* tilewin,
-                 void* workspace, size_t workspace_bytes, unsigned long long* dbg, cudaStream_t st);
+                 int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, int precision, float* hout, int64_t ldh,
+                 const int32_t* tilewin, void* workspace, size_t workspace_bytes, unsigned long long* dbg, cudaStream_t st);
 void fused_path_count(int which);
 }
 extern "C" int gnnml3_fused_ts_supported(int K, int Kstride, int F, int Nc, int Fs, int self_mode, int Ns);
@@ -1048,7 +1048,7 @@ extern "C" int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
                                      int Kstride, int K, const float* X, int64_t ldx, int F, const float* S, int64_t lds,
                                      int Fs, int self_mode, const float* Bmain, int64_t ldb, const float* Bself,
                                      int64_t ldbs, int Ns, const float* bias, const float* bias_s, int64_t N, int Nc,
-                                     float* out, int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue,
+                                     float* out, int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, int precision,
                                      float* hout, int64_t ldh, const int32_t* tilewin, void* workspace, size_t workspace_bytes,
                                      void* stream_) {
     GNNML3_REQUIRE(N > 0 && N < (1ll << 31) - 256, "fused_agg_proj: bad N");
@@ -1059,11 +1059,9 @@ extern "C" int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
     GNNML3_REQUIRE((uintptr_t)ea % 16 == 0, "fused_agg_proj: ea must be 16-byte aligned");
     GNNML3_REQUIRE(self_mode == 0 || (S && Bself && lds % 4 == 0 && (uintptr_t)S % 16 == 0),
                    "fused_agg_proj: self block needs S, Bself and 16-byte aligned rows");
-    const int prec_bits = epilogue & 0x300;                  // GNNML3_FUSED_TF32 / GNNML3_FUSED_BF16 (tensor-memory kernel only)
-    epilogue &= 0xff;
     GNNML3_REQUIRE(epilogue == 0 || epilogue == 1, "fused_agg_proj: unknown epilogue");
-    GNNML3_REQUIRE(prec_bits == 0 || prec_bits == 0x100 || prec_bits == 0x200, "fused_agg_proj: unknown precision flag");
-    GNNML3_REQUIRE(prec_bits == 0 || (gnnml3_fused_ts_supported(K, Kstride, F, Nc, Fs, self_mode, Ns) && g_fl_slot_mode == 0),
+    GNNML3_REQUIRE(prec_valid(precision), "fused_agg_proj: unknown precision %d", precision);
+    GNNML3_REQUIRE(precision == GNNML3_PREC_3XTF32 || (gnnml3_fused_ts_supported(K, Kstride, F, Nc, Fs, self_mode, Ns) && g_fl_slot_mode == 0),
                    "fused_agg_proj: the single-pass TF32 / BF16 modes exist in the tensor-memory kernel only (F <= 32, even K)");
     GNNML3_REQUIRE(self_mode != 1 || (epilogue == 1 && G >= 1 && G <= 16 && Ns == 2 * G),
                    "fused_agg_proj: gate columns need the ML3 epilogue and Ns == 2G <= 32");
@@ -1090,7 +1088,7 @@ extern "C" int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
             cudaEventRecord(rec.a, st);
         }
         const int rc = fused_ts_run(rowptr, col, eperm, ea, Kstride, K, X, ldx, F, S, lds, Fs, self_mode, Bmain, ldb, Bself, ldbs, Ns, bias,
-                                    bias_s, N, Nc, out, ldo, aux, ldaux, G, epilogue | prec_bits, hout, ldh, tilewin, workspace, workspace_bytes,
+                                    bias_s, N, Nc, out, ldo, aux, ldaux, G, epilogue, precision, hout, ldh, tilewin, workspace, workspace_bytes,
                                     g_fl_dbg, st);
         if (g_fl_prof_on) {
             cudaEventRecord(rec.b, st);

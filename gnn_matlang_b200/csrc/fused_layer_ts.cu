@@ -1026,10 +1026,8 @@ int ts_make_xmap(CUtensorMap* map, const float* base, int64_t rows, int F, int64
 int fused_ts_run(const int32_t* rowptr, const int32_t* col, const int32_t* eperm, const float* ea, int Kstride, int K, const float* X,
                  int64_t ldx, int F, const float* S, int64_t lds, int Fs, int self_mode, const float* Bmain, int64_t ldb,
                  const float* Bself, int64_t ldbs, int Ns, const float* bias, const float* bias_s, int64_t N, int Nc, float* out,
-                 int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, float* hout, int64_t ldh, const int32_t* tilewin,
-                 void* workspace, size_t workspace_bytes, unsigned long long* dbg, cudaStream_t st) {
-    const int prec = (epilogue >> 8) & 3;
-    epilogue &= 0xff;
+                 int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, int precision, float* hout, int64_t ldh,
+                 const int32_t* tilewin, void* workspace, size_t workspace_bytes, unsigned long long* dbg, cudaStream_t st) {
     if (workspace_bytes < gnnml3_fused_ts_workspace_bytes(K, Nc, self_mode))
         return set_err(GNNML3_ERR_WORKSPACE, "fused_agg_proj: workspace too small");
     const int BNH = Nc <= 32 ? 32 : 64;
@@ -1039,7 +1037,7 @@ int fused_ts_run(const int32_t* rowptr, const int32_t* col, const int32_t* eperm
     {
         const int total = nkb_total * 2 * BNH * 32;
         const int blocks = cdiv(total, 256) > 592 ? 592 : cdiv(total, 256);
-        k_ts_prep_weights<<<blocks, 256, 0, st>>>(Bmain, ldb, K, F, Nc, BNH, Bself, ldbs, Fs, Ns, self_mode, prec, planes);
+        k_ts_prep_weights<<<blocks, 256, 0, st>>>(Bmain, ldb, K, F, Nc, BNH, Bself, ldbs, Fs, Ns, self_mode, precision, planes);
         GNNML3_LAUNCH_CHECK();
     }
     CUtensorMap mW, mX;
@@ -1051,7 +1049,7 @@ int fused_ts_run(const int32_t* rowptr, const int32_t* col, const int32_t* eperm
     P.rowptr = rowptr; P.col = col; P.eperm = eperm; P.ea = ea; P.Kstride = Kstride; P.K = K;
     P.X = X; P.ldx = ldx; P.F = F; P.S = S; P.lds = lds; P.Fs = Fs; P.self_mode = self_mode;
     P.N = N; P.n_tiles = cdiv(N, TS_ROWS); P.nkb_main = K; P.tilewin = reinterpret_cast<const int2*>(tilewin); P.win_rows = win_rows;
-    P.bias = bias; P.bias_s = bias_s; P.out = out; P.ldo = ldo; P.Nc = Nc; P.aux = aux; P.ldaux = ldaux; P.G = G; P.epi = epilogue; P.prec = prec;
+    P.bias = bias; P.bias_s = bias_s; P.out = out; P.ldo = ldo; P.Nc = Nc; P.aux = aux; P.ldaux = ldaux; P.G = G; P.epi = epilogue; P.prec = precision;
     P.hout = hout; P.ldh = ldh; P.dbg = dbg;
     P.edge_cap = tilewin ? ts_edge_cap(K, Kstride, Nc, self_mode) : 0;
     const size_t smem = ts_smem_bytes(K, Kstride, Nc, self_mode, P.edge_cap);

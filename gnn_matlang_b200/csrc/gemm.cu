@@ -9,7 +9,7 @@
 // M (nodes) is 1e3..1e6+, Nc/Ka/Nb/Kc are 2..2560, so the kernels are bound by streaming the tall operand from
 // HBM once; the math runs on the tensor cores as TF32 m16n8k8 with FP32 accumulation.  Default arithmetic is
 // the error-compensated 3xTF32 split (a = hi + lo, a*b ~= lo*hi + hi*lo + hi*hi), which restores FP32-grade
-// accuracy (needed for the rtol 1e-5 parity bar); GNNML3_PREC_TF32 runs the single-pass variant.
+// accuracy (needed for the rtol 1e-5 parity bar); GNNML3_PREC_TF32 and GNNML3_PREC_BF16 run the single-pass variant.
 #include "common.cuh"
 
 namespace gnnml3 {
@@ -515,7 +515,7 @@ extern "C" int gnnml3_gemm_nn(const float* A, int64_t lda, const float* B, int64
     GNNML3_REQUIRE(M > 0 && Nc > 0 && Kc > 0, "gemm_nn: bad shape M=%lld Nc=%d Kc=%d", (long long)M, Nc, Kc);
     GNNML3_REQUIRE(A && B && C, "gemm_nn: NULL pointer");
     GNNML3_REQUIRE(lda >= Kc && ldb >= Nc && ldc >= Nc, "gemm_nn: leading dimensions too small");
-    GNNML3_REQUIRE(precision == GNNML3_PREC_3XTF32 || precision == GNNML3_PREC_TF32, "gemm_nn: unknown precision %d", precision);
+    GNNML3_REQUIRE(prec_valid(precision), "gemm_nn: unknown precision %d", precision);
     GNNML3_REQUIRE(epilogue == GNNML3_EPI_NONE || epilogue == GNNML3_EPI_RELU, "gemm_nn: unknown epilogue %d", epilogue);
     GNNML3_REQUIRE(cdiv(M, NN_BM) > 0 && cdiv(Nc, 32) < 65536, "gemm_nn: grid too large");
     cudaStream_t st = (cudaStream_t)stream_;
@@ -567,7 +567,7 @@ extern "C" int gnnml3_gemm_tn(const float* A, int64_t lda, const float* B, int64
     GNNML3_REQUIRE(M > 0 && Ka > 0 && Nb > 0, "gemm_tn: bad shape");
     GNNML3_REQUIRE(A && B && C && workspace, "gemm_tn: NULL pointer");
     GNNML3_REQUIRE(lda >= Ka && ldb >= Nb && ldc >= Nb, "gemm_tn: leading dimensions too small");
-    GNNML3_REQUIRE(precision == GNNML3_PREC_3XTF32 || precision == GNNML3_PREC_TF32, "gemm_tn: unknown precision %d", precision);
+    GNNML3_REQUIRE(prec_valid(precision), "gemm_tn: unknown precision %d", precision);
     GNNML3_REQUIRE(cdiv(Nb, 64) < 65536, "gemm_tn: grid too large");
     if (workspace_bytes < gnnml3_gemm_tn_workspace_bytes(M, Ka, Nb))
         return set_err(GNNML3_ERR_WORKSPACE, "gemm_tn: workspace %zu < %zu bytes", workspace_bytes,
@@ -580,7 +580,7 @@ extern "C" int gnnml3_gemm_tn(const float* A, int64_t lda, const float* B, int64
     const bool vb = (ldb % 4 == 0 || M == 1) && (uintptr_t)B % 16 == 0;
     float* P = (float*)workspace;
     int rc;
-    if (tn_narrow(Ka, Nb)) {   // exact FP32 FMAs: at least as accurate as either requested precision
+    if (tn_narrow(Ka, Nb)) {   // exact FP32 FMAs: at least as accurate as any requested precision
         const int64_t nblk = cdiv(M, (int64_t)TNN_ROWS);
         GNNML3_REQUIRE(nblk < (int64_t)1 << 31, "gemm_tn: too many rows");
         k_gemm_tn_narrow<<<(unsigned)nblk, TNN_WARPS * 32, 0, st>>>(A, lda, B, ldb, P, M, Ka, Nb);

@@ -183,7 +183,7 @@ extern "C" int gnnml3_ml3layer_forward(const int32_t* rowptr, const int32_t* col
         GNNML3_LAUNCH_CHECK();
     }
     return gnnml3_fused_agg_proj(rowptr, col, nullptr, eaw, K, K, x, ldx, Fi, G > 0 ? x : nullptr, ldx, G > 0 ? Fi : 0, G > 0 ? 1 : 0, wconv,
-                                 Fo, wg, 2 * G, 2 * G, bconv, bg, N, Fo, y, ldy, aux, 2 * G, G, 1, hside, hside ? ldh : 0, win, ws + w.fused,
+                                 Fo, wg, 2 * G, 2 * G, bconv, bg, N, Fo, y, ldy, aux, 2 * G, G, 1, GNNML3_PREC_3XTF32, hside, hside ? ldh : 0, win, ws + w.fused,
                                  w.wg - w.fused, stream);
 }
 
@@ -242,13 +242,13 @@ extern "C" int gnnml3_ml3layer_backward(const int32_t* rowptr, const int32_t* co
         ldG = (int64_t)(K + (G > 0 ? 1 : 0)) * 32;
         if ((rc = gnnml3_fused_agg_proj(rowptrT, colT, permT, eaw, K, K, gpre, w.ldg, Fo, G > 0 ? gpre + Fo4 : nullptr, w.ldg, 2 * G,
                                         G > 0 ? 2 : 0, wT, Fi, G > 0 ? ws2 : nullptr, Fi, 0, nullptr, nullptr, N, Fi, dx, lddx, nullptr, 0, 0,
-                                        0, Gp, ldG, winT, ws + w.fused, w.wg - w.fused, stream)))
+                                        0, GNNML3_PREC_3XTF32, Gp, ldG, winT, ws + w.fused, w.wg - w.fused, stream)))
             return rc;
     } else {
         if (need_dx) {
             if ((rc = gnnml3_fused_agg_proj(rowptrT, colT, permT, eaw, K, K, gpre, w.ldg, Fo, G > 0 ? gpre + Fo4 : nullptr, w.ldg, 2 * G,
                                             G > 0 ? 2 : 0, wT, Fi, G > 0 ? ws2 : nullptr, Fi, 0, nullptr, nullptr, N, Fi, dx, lddx, nullptr, 0,
-                                            0, 0, nullptr, 0, winT, ws + w.fused, w.wg - w.fused, stream)))
+                                            0, 0, GNNML3_PREC_3XTF32, nullptr, 0, winT, ws + w.fused, w.wg - w.fused, stream)))
                 return rc;
         }
         pitch = Fo;

@@ -508,10 +508,6 @@ static int ml1_prep(const float* wc, const float* wA, const float* wB, const flo
     return GNNML3_OK;
 }
 
-static bool ml1_prec_ok(int prec) {
-    return prec == GNNML3_PREC_3XTF32 || prec == GNNML3_PREC_TF32 || prec == GNNML3_PREC_BF16;
-}
-
 }  // namespace gnnml3
 
 using namespace gnnml3;
@@ -525,12 +521,12 @@ extern "C" size_t gnnml3_ml1layer_workspace_bytes(int64_t N, int Fi, int Fo, int
     return ml1_ws(N, Fi, Fo, concat).total;
 }
 
-extern "C" int gnnml3_ml1layer_forward_precision(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x,
-                                                 int64_t ldx, int Fi, const float* wconv, const float* bconv, const float* wA,
-                                                 const float* bA, const float* wB, const float* bB, const float* wC, const float* bC,
-                                                 int Fo, int concat, float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside,
-                                                 int64_t ldh, void* workspace, size_t workspace_bytes, void* stream, int precision) {
-    GNNML3_REQUIRE(ml1_prec_ok(precision), "ml1layer_forward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
+extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x, int64_t ldx,
+                                       int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
+                                       const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat,
+                                       float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh,
+                                       void* workspace, size_t workspace_bytes, void* stream, int precision) {
+    GNNML3_REQUIRE(prec_valid(precision), "ml1layer_forward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
     GNNML3_REQUIRE(gnnml3_ml1layer_supported(Fi, Fo, concat), "ml1layer_forward: unsupported shape Fi=%d Fo=%d", Fi, Fo);
     GNNML3_REQUIRE(N >= 0 && E >= 0 && rowptr && x && wconv && wA && wB && wC && y, "ml1layer_forward: NULL pointer");
     GNNML3_REQUIRE(E == 0 || col, "ml1layer_forward: NULL col");
@@ -557,23 +553,13 @@ extern "C" int gnnml3_ml1layer_forward_precision(const int32_t* rowptr, const in
     return ml1_launch(P, s.smem, aux != nullptr, precision, st);     // no aux: the forward-only instantiation
 }
 
-extern "C" int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x, int64_t ldx,
-                                       int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
-                                       const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat,
-                                       float* y, int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh,
-                                       void* workspace, size_t workspace_bytes, void* stream) {
-    return gnnml3_ml1layer_forward_precision(rowptr, col, N, E, x, ldx, Fi, wconv, bconv, wA, bA, wB, bB, wC, bC, Fo, concat, y, ldy,
-                                             aux, ldaux, hside, ldh, workspace, workspace_bytes, stream, GNNML3_PREC_3XTF32);
-}
-
-extern "C" int gnnml3_ml1layer_backward_precision(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x,
-                                                  int64_t ldx, int Fi, const float* wconv, const float* wA, const float* wB,
-                                                  const float* wC, int Fo, int concat, const float* y, int64_t ldy, const float* aux,
-                                                  int64_t ldaux, const float* gy, int64_t ldgy, int need_dx, float* dx, int64_t lddx,
-                                                  float* dwconv, float* dbconv, float* dwA, float* dbA, float* dwB, float* dbB,
-                                                  float* dwC, float* dbC, void* workspace, size_t workspace_bytes, void* stream,
-                                                  int precision) {
-    GNNML3_REQUIRE(ml1_prec_ok(precision), "ml1layer_backward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
+extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
+                                        int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
+                                        const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
+                                        int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
+                                        float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
+                                        void* stream, int precision) {
+    GNNML3_REQUIRE(prec_valid(precision), "ml1layer_backward: unknown precision %d (GNNML3_PREC_3XTF32, _TF32 or _BF16)", precision);
     GNNML3_REQUIRE(gnnml3_ml1layer_supported(Fi, Fo, concat), "ml1layer_backward: unsupported shape Fi=%d Fo=%d", Fi, Fo);
     GNNML3_REQUIRE(N > 0, "ml1layer_backward: empty batch");
     GNNML3_REQUIRE(E >= 0 && rowptrT && (E == 0 || colT) && x && wconv && wA && wB && wC && y && aux && gy && dwconv && dwA && dwB && dwC,
@@ -602,26 +588,14 @@ extern "C" int gnnml3_ml1layer_backward_precision(const int32_t* rowptrT, const 
     P.project = need_dx ? 1 : 0; P.epi = 0; P.out = dx; P.ldo = lddx; P.Nout = Fi;
     P.hout = GG + 3 * Fo4; P.ldh = w.ldgg;
     if ((rc = ml1_launch(P, need_dx ? s.smem : 1024 + 2 * ML1_ABUF + 64, true, precision, st))) return rc;
-    // [dfcA^T | dfcB^T | dfcC^T | dWc] = x^T GG[:, 0:4 Fo4] in one contraction (single-pass TF32 in the flagged modes, as the
-    // stand-alone GEMMs run BF16); bias gradients = column sums (fixed order)
+    // [dfcA^T | dfcB^T | dfcC^T | dWc] = x^T GG[:, 0:4 Fo4] in one contraction (the GEMM runs BF16 as single-pass TF32);
+    // bias gradients = column sums (fixed order)
     float* dcat = (float*)(ws + w.dcat);
     float* csum = (float*)(ws + w.csum);
-    const int tn_prec = precision == GNNML3_PREC_3XTF32 ? GNNML3_PREC_3XTF32 : GNNML3_PREC_TF32;
-    if ((rc = gnnml3_gemm_tn(x, ldx, GG, w.ldgg, dcat, 4 * Fo4, N, Fi, 4 * Fo4, tn_prec, ws + w.tn, w.total - w.tn, stream)))
+    if ((rc = gnnml3_gemm_tn(x, ldx, GG, w.ldgg, dcat, 4 * Fo4, N, Fi, 4 * Fo4, precision, ws + w.tn, w.total - w.tn, stream)))
         return rc;
     if ((rc = gnnml3_colsum(GG, w.ldgg, N, 5 * Fo4, csum, ws + w.cs, w.tn - w.cs, stream))) return rc;
     k_ml1_unpack<<<cdiv(4 * Fi * Fo + 4 * Fo, 256), 256, 0, st>>>(dcat, csum, Fi, Fo, Fo4, dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC);
     GNNML3_LAUNCH_CHECK();
     return GNNML3_OK;
-}
-
-extern "C" int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
-                                        int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
-                                        const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
-                                        int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
-                                        float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
-                                        void* stream) {
-    return gnnml3_ml1layer_backward_precision(rowptrT, colT, N, E, x, ldx, Fi, wconv, wA, wB, wC, Fo, concat, y, ldy, aux, ldaux, gy,
-                                              ldgy, need_dx, dx, lddx, dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC, workspace,
-                                              workspace_bytes, stream, GNNML3_PREC_3XTF32);
 }

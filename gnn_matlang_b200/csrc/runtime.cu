@@ -30,6 +30,6 @@ std::mutex& config_mutex() {
 extern "C" {
 
 const char* gnnml3_last_error(void) { return gnnml3::err_buf(); }
-int gnnml3_version(void) { return 100; }
+int gnnml3_version(void) { return 101; }
 int64_t gnnml3_launch_count(void) { return gnnml3::g_launches.load(); }
 }

@@ -34,13 +34,16 @@ USE_LAYER_API = os.environ.get("GNNML3_NO_LAYER_API", "0") != "1"
 KEEP_FIRST_LAYER_AGGREGATE = os.environ.get("GNNML3_KEEP_AGGREGATE", "1") != "0"
 
 
-def _use_fused(precision):
-    """The fused tcgen05 layer kernels exist for every precision: FP32-grade 3xTF32 in both generations, the flagged
-    single-pass TF32 and BF16 modes in the tensor-memory generation (``_fused_ok`` checks the shape)."""
-    return USE_FUSED
+def _precision_code(precision):
+    """The library's PREC_* code of a precision name ("fp32" = "3xtf32", "tf32", "bf16"); ValueError for any other value."""
+    if precision not in _PRECISIONS:
+        raise ValueError("precision must be one of %s" % sorted(_PRECISIONS))
+    return _PRECISIONS[precision]
 
 
 def _fused_ok(precision, K, Kstride, F, Nc, Fs=0, self_mode=0, Ns=0):
+    """The fused layer kernels cover this shape in ``precision``: 3xTF32 in both generations, the flagged single-pass TF32 and
+    BF16 modes in the tensor-memory generation only."""
     if precision == _lib.PREC_3XTF32:
         return ops.fused_supported(K, Kstride, F, Nc, Fs, self_mode, Ns)
     return ops.fused_ts_supported(K, Kstride, F, Nc, Fs, self_mode, Ns)
@@ -89,7 +92,7 @@ class _SpectConvFn(torch.autograd.Function):
         N, Fi = x.shape
         Kw, _, Fo = weight.shape
         K = ea_s.size(1)
-        fused = (_use_fused(precision) and N > 0 and plan.E > 0 and (not selfconn or Fi <= 32)
+        fused = (USE_FUSED and N > 0 and plan.E > 0 and (not selfconn or Fi <= 32)
                  and _fused_ok(precision, K, K, Fi, Fo, Fi if selfconn else 0, 2 if selfconn else 0, 0))
         ctx.plan, ctx.selfconn, ctx.precision, ctx.has_bias = plan, selfconn, precision, bias is not None
         ctx.fused = fused
@@ -316,7 +319,7 @@ class _ML3LayerFn(torch.autograd.Function):
         K, _, Fo = wconv.shape
         G = 0 if w11 is None else w11.size(0)
         ctx.composite = False
-        if (_use_fused(precision) and precision == _lib.PREC_3XTF32 and USE_LAYER_API and N > 0 and plan.E > 0
+        if (USE_FUSED and precision == _lib.PREC_3XTF32 and USE_LAYER_API and N > 0 and plan.E > 0
                 and (fused_edge or w1 is None) and ops.ml3layer_supported(K, Fi, Fo, G, fused_edge)):
             # the whole layer in ONE library call (layer_api.cu): same kernels as below, a fraction of the host time
             xa = ops.aligned_rows(x)
@@ -341,7 +344,7 @@ class _ML3LayerFn(torch.autograd.Function):
             ea2 = ops.edge_mlp_fwd(ea_s, None, w1, w2, w3, w4)
         else:
             ea2 = ea_s
-        fused = (_use_fused(precision) and N > 0 and plan.E > 0 and (G == 0 or Fi <= 32)
+        fused = (USE_FUSED and N > 0 and plan.E > 0 and (G == 0 or Fi <= 32)
                  and _fused_ok(precision, K, K, Fi, Fo, Fi if G else 0, 1 if G else 0, 2 * G)
                  and _fused_ok(precision, K, K, Fo, Fi, 2 * G, 2 if G else 0, 0))
         ctx.plan, ctx.fused_edge, ctx.precision, ctx.G = plan, fused_edge, precision, G
@@ -481,8 +484,7 @@ class SpectConv(nn.Module):
         if kwargs.pop('aggr') != 'add':
             raise ValueError("SpectConv only implements aggr='add' (the reference's default, :27)")
         self.precision = kwargs.pop('precision', 'fp32')
-        if self.precision not in _PRECISIONS:
-            raise ValueError("precision must be one of %s" % sorted(_PRECISIONS))
+        _precision_code(self.precision)
         # 'auto' (default): the fused aggregate-first kernels where they apply, else whichever order moves fewer HBM words
         # (project_first_pays); 'aggregate_first' / 'project_first' force one order (measurements, DESIGN.md section 4.5)
         self.order = kwargs.pop('order', 'auto')
@@ -520,7 +522,7 @@ class SpectConv(nn.Module):
 
     def forward_sorted(self, x, plan, ea_s):
         """Same as ``forward`` with the graph plan and the dst-sorted edge features already at hand."""
-        prec = _PRECISIONS[self.precision]
+        prec = _precision_code(self.precision)
         if not self.depthwise:
             nk = self.weight.size(0) - (1 if self.selfconn else 0)
             if ea_s.size(1) < nk:
@@ -531,7 +533,7 @@ class SpectConv(nn.Module):
             order = self.order
             if order == 'auto':
                 Fi, Fo = self.in_channels, self.out_channels
-                fused = _use_fused(prec) and _fused_ok(prec, nk, nk, Fi, Fo, Fi if self.selfconn else 0, 2 if self.selfconn else 0, 0)
+                fused = USE_FUSED and _fused_ok(prec, nk, nk, Fi, Fo, Fi if self.selfconn else 0, 2 if self.selfconn else 0, 0)
                 order = 'project_first' if (not fused and Fo <= 256 and project_first_pays(plan.N, plan.E, nk, Fi, Fo)) else 'aggregate_first'
             if order == 'project_first' and self.out_channels <= 256:
                 out = _SpectConvProjectFirstFn.apply(x, ea_s, self.weight[:nk], None if self.selfconn else self.bias, plan, prec)
@@ -564,8 +566,7 @@ class SpectConCatConv(nn.Module):
         if kwargs.pop('aggr') != 'add':
             raise ValueError("SpectConCatConv only implements aggr='add' (the reference's default, :109)")
         self.precision = kwargs.pop('precision', 'fp32')
-        if self.precision not in _PRECISIONS:
-            raise ValueError("precision must be one of %s" % sorted(_PRECISIONS))
+        _precision_code(self.precision)
         super(SpectConCatConv, self).__init__()
         assert K > 0
         self.in_channels = in_channels
@@ -588,7 +589,7 @@ class SpectConCatConv(nn.Module):
         _check_inputs(x, edge_index, edge_attr)
         plan = get_plan(edge_index, x.size(0))
         ea_s = sorted_edge_attr(edge_attr, plan)
-        prec = _PRECISIONS[self.precision]
+        prec = _precision_code(self.precision)
         nk = self.weight.size(0) - (1 if self.selfconn else 0)
         if ea_s.size(1) < nk:
             raise RuntimeError("SpectConCatConv: edge_attr has %d channels but the layer was built with K=%d" % (ea_s.size(1), nk))
@@ -627,6 +628,7 @@ class ML3Layer(torch.nn.Module):
 
     def __init__(self, learnedge, nedgeinput, nedgeoutput, ninp, nout1, nout2, precision='fp32'):
         super(ML3Layer, self).__init__()
+        _precision_code(precision)
         self.learnedge = learnedge
         self.nout2 = nout2
         self.precision = precision
@@ -646,7 +648,7 @@ class ML3Layer(torch.nn.Module):
         _check_inputs(x, edge_index, edge_attr)
         plan = get_plan(edge_index, x.size(0))
         ea = sorted_edge_attr(edge_attr, plan)
-        prec = _PRECISIONS[self.precision]
+        prec = _precision_code(self.precision)
         c = self.conv1
         if not self.learnedge and ea.size(1) > c.weight.size(0):
             # the reference's SpectConv reads edge_attr[:, i] for i < K only (libs/spect_conv.py:76-80): extra channels are ignored
@@ -731,7 +733,7 @@ class ML1Layer(torch.nn.Module):
 
     def __init__(self, ninp, nout, concat=False, precision="fp32"):
         super(ML1Layer, self).__init__()
-        _check_precision(precision)
+        _precision_code(precision)
         self.concat = bool(concat)
         self.precision = precision
         self.conv1 = SpectConv(ninp, nout, 1, selfconn=False)
@@ -747,22 +749,16 @@ class ML1Layer(torch.nn.Module):
         return ml1_layer(x, edge_index, self.conv1, self.fc11, self.fc12, self.fc13, self.concat, self.precision)
 
 
-def _check_precision(precision):
-    if precision not in _PRECISIONS:
-        raise ValueError("precision must be one of %s" % sorted(_PRECISIONS))
-
-
 def ml1_layer(x, edge_index, conv, fcA, fcB, fcC, concat=False, precision="fp32"):
     """The GNNML1 layer on given modules (``conv`` a SpectConv(K=1, selfconn=False), ``fcA``/``fcB``/``fcC`` nn.Linear):
     what ``ML1Layer.forward`` and ``models.GNNML1`` run, in ``precision`` ("fp32", "tf32" or "bf16")."""
-    _check_precision(precision)
+    prec = _precision_code(precision)
     if not (x.is_cuda and edge_index.is_cuda):
         raise RuntimeError("gnn_matlang_b200: x and edge_index must be CUDA tensors (the B200 hot path has no CPU fallback)")
     if x.dim() != 2 or x.dtype != torch.float32:
         raise RuntimeError("gnn_matlang_b200: x [N, F] must be float32")
     plan = get_plan(edge_index, x.size(0))
     Fi, Fo = conv.in_channels, conv.out_channels
-    prec = _PRECISIONS[precision]
     if ops.ml1layer_supported(Fi, Fo, concat):
         ML1_PATH_COUNTS["fused"] += 1
         ps = (conv.weight, conv.bias, fcA.weight, fcA.bias, fcB.weight, fcB.bias, fcC.weight, fcC.bias)

@@ -26,7 +26,7 @@ preset (``graph8c``, ``zinc``, ``exp``, ``counting``).
 import torch
 import torch.nn as nn
 
-from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _PRECISIONS, _check_precision, ml1_layer
+from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _precision_code, ml1_layer
 import torch.nn.functional as F
 
 from .pool import global_add_pool, global_max_pool, global_mean_pool
@@ -46,6 +46,7 @@ MODEL_CONFIGS = {
 class GNNML3(nn.Module):
     def __init__(self, config, ne, ninp, precision="fp32"):
         super().__init__()
+        _precision_code(precision)
         c = dict(MODEL_CONFIGS[config]) if isinstance(config, str) else dict(config)
         self.cfg = c
         self.precision = precision
@@ -84,7 +85,7 @@ class GNNML3(nn.Module):
             x = torch.cat([pools[k](x, data.batch, B) for k in c["pool"].split("_")], 1)
         if c.get("bn") == "readout":
             x = getattr(self, "bn%d" % c["nlayer"])(x)
-        prec = _PRECISIONS[self.precision]
+        prec = _precision_code(self.precision)
         if len(c["head"]) == 1:
             fc = self.fc2 if c.get("fc_name") == "fc2" else self.fc1
             x = _LinearFn.apply(x, fc.weight.t(), fc.bias, prec)
@@ -110,7 +111,7 @@ class GNNML1(nn.Module):
         super().__init__()
         if isinstance(config, str) and config not in GNNML1_PRESETS:
             raise ValueError("GNNML1 presets: %s" % (GNNML1_PRESETS,))
-        _check_precision(precision)
+        _precision_code(precision)
         c = dict(MODEL_CONFIGS[config]) if isinstance(config, str) else dict(config)
         self.cfg = c
         self.precision = precision
@@ -136,7 +137,7 @@ class GNNML1(nn.Module):
         B = getattr(data, "num_graphs", None)
         pool = {"add": global_add_pool, "mean": global_mean_pool}[c["pool"]]
         x = pool(x, data.batch, B)
-        prec = _PRECISIONS[self.precision]
+        prec = _precision_code(self.precision)
         x = _LinearFn.apply(x, self.fc1.weight.t(), self.fc1.bias, prec)
         if len(c["head"]) == 1:
             return torch.tanh(x) if c["final"] == "tanh" else x

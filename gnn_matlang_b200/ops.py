@@ -221,7 +221,6 @@ def gemm_nn(A, B, bias=None, precision=_lib.PREC_3XTF32, epilogue=_lib.EPI_NONE,
     """C = A @ B (+ bias) (+ relu) on the tensor cores; A [M,Kc], B [Kc,Nc].  FP32-grade (3xTF32) requests with
     16-byte aligned rows run on tcgen05/TMEM; everything else on the mma.sync kernel."""
     lib = _lib.load()
-    precision = min(int(precision), _lib.PREC_TF32)
     A = _rows(A, "A")
     B = _f32c(B, "B")
     M, Kc = A.shape
@@ -246,7 +245,6 @@ def gemm_nn(A, B, bias=None, precision=_lib.PREC_3XTF32, epilogue=_lib.EPI_NONE,
 def gemm_tn(A, B, precision=_lib.PREC_3XTF32):
     """C = A^T @ B; A [M,Ka], B [M,Nb] -> [Ka,Nb]; deterministic split over M."""
     lib = _lib.load()
-    precision = min(int(precision), _lib.PREC_TF32)
     A = _rows(A, "A")
     B = _rows(B, "B")
     M, Ka = A.shape
@@ -422,7 +420,7 @@ def fused_agg_proj(rowptr, col, eperm, ea, x, Bmain, bias=None, S=None, self_mod
             _lib.ptr(rowptr), _lib.ptr(col), _lib.ptr(eperm), _lib.ptr(ea), K, K, _lib.ptr(x), _ld(x), F,
             _lib.ptr(S) if self_mode else None, _ld(S) if self_mode else 0, Fs, self_mode, _lib.ptr(Bmain), _ld(Bmain),
             _lib.ptr(Bself) if self_mode else None, _ld(Bself) if self_mode else 0, Ns, _lib.ptr(bias), _lib.ptr(bias_s),
-            N, Nc, _lib.ptr(out), (W + 3) // 4 * 4, _lib.ptr(aux), 2 * G, G, epilogue | _lib.FUSED_FLAGS[precision], _lib.ptr(hout), _ld(hout) if hout is not None else 0,
+            N, Nc, _lib.ptr(out), (W + 3) // 4 * 4, _lib.ptr(aux), 2 * G, G, epilogue, precision, _lib.ptr(hout), _ld(hout) if hout is not None else 0,
             _lib.ptr(win), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
             "gnnml3_fused_agg_proj")
     return out, aux
@@ -571,7 +569,7 @@ def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False
     x [N, Fi] must satisfy ``aligned_rows``; wconv [1, Fi, Fo]; wA/wB/wC [Fo, Fi].  -> (y [N, Fo] or [N, 3 Fo],
     aux [N, 2 Fo] = [p1 | p2] (None with ``aux=False``: a forward nobody differentiates stores y alone),
     A x [N, Fi] if ``keep_aggregate`` else None).  ``precision`` (PREC_3XTF32 | PREC_TF32 | PREC_BF16): the arithmetic of the
-    projection (gnnml3_ml1layer_forward_precision for the flagged modes)."""
+    projection."""
     lib = _lib.load()
     N, Fi = x.shape
     Fo = wconv.size(2)
@@ -584,18 +582,15 @@ def ml1layer_forward(plan, x, wconv, bconv, wA, bA, wB, bB, wC, bC, concat=False
     p = _lib.ptr
     args = (p(plan.rowptr), p(plan.col), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(bconv), p(wA), p(bA), p(wB), p(bB), p(wC), p(bC), Fo,
             int(bool(concat)), p(y), _ld(y) if N > 1 else (W + 3) // 4 * 4, p(aux), 2 * Fo, p(hside), (Fi + 3) // 4 * 4, p(ws), ws.numel(),
-            _lib.stream_ptr())
+            _lib.stream_ptr(), precision)
     with _on(dev):
-        if precision == _lib.PREC_3XTF32:
-            _lib.check(lib.gnnml3_ml1layer_forward(*args), "gnnml3_ml1layer_forward")
-        else:
-            _lib.check(lib.gnnml3_ml1layer_forward_precision(*args, int(precision)), "gnnml3_ml1layer_forward_precision")
+        _lib.check(lib.gnnml3_ml1layer_forward(*args), "gnnml3_ml1layer_forward")
     return y, aux, hside
 
 
 def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=False, precision=_lib.PREC_3XTF32):
-    """Whole GNNML1 layer backward in one library call (gnnml3_ml1layer_backward, or its _precision form for a flagged
-    ``precision``).  -> dx (None unless need_dx), dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC"""
+    """Whole GNNML1 layer backward in one library call (gnnml3_ml1layer_backward) in ``precision``.
+    -> dx (None unless need_dx), dwconv, dbconv, dwA, dbA, dwB, dbB, dwC, dbC"""
     lib = _lib.load()
     N, Fi = x.shape
     Fo = wconv.size(2)
@@ -610,12 +605,9 @@ def ml1layer_backward(plan, x, wconv, wA, wB, wC, y, aux, gy, need_dx, concat=Fa
     p = _lib.ptr
     args = (p(plan.rowptrT), p(plan.colT), N, plan.E, p(x), _ld(x), Fi, p(wconv), p(wA), p(wB), p(wC), Fo, int(bool(concat)),
             p(y), _ld(y) if N > 1 else y.size(1), p(aux), 2 * Fo, p(gy), _ld(gy), int(bool(need_dx)), p(dx), lddx, p(dwc), p(dbs[0]),
-            p(dwA), p(dbs[1]), p(dwB), p(dbs[2]), p(dwC), p(dbs[3]), p(ws), ws.numel(), _lib.stream_ptr())
+            p(dwA), p(dbs[1]), p(dwB), p(dbs[2]), p(dwC), p(dbs[3]), p(ws), ws.numel(), _lib.stream_ptr(), precision)
     with _on(dev):
-        if precision == _lib.PREC_3XTF32:
-            _lib.check(lib.gnnml3_ml1layer_backward(*args), "gnnml3_ml1layer_backward")
-        else:
-            _lib.check(lib.gnnml3_ml1layer_backward_precision(*args, int(precision)), "gnnml3_ml1layer_backward_precision")
+        _lib.check(lib.gnnml3_ml1layer_backward(*args), "gnnml3_ml1layer_backward")
     return (dx[:, :Fi] if need_dx else None), dwc, dbs[0], dwA, dbs[1], dwB, dbs[2], dwC, dbs[3]
 
 

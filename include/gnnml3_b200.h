@@ -43,17 +43,13 @@ extern "C" {
 #define GNNML3_ERR_CUDA 2        /* a CUDA runtime call or kernel launch failed */
 #define GNNML3_ERR_WORKSPACE 3   /* workspace too small */
 
-/* GEMM arithmetic: FP32-grade error-compensated 3xTF32 (default, meets rtol 1e-5), single-pass TF32.  BF16 inputs with FP32
- * accumulation: the GNNML1 layer (gnnml3_ml1layer_*_precision); the stand-alone GEMMs take it as single-pass TF32. */
+/* The `precision` argument of every entry point that takes one: FP32-grade error-compensated 3xTF32 (default, meets rtol 1e-5),
+ * single-pass TF32, or BF16 inputs with FP32 accumulation.  The fused layer kernels (gnnml3_fused_agg_proj, gnnml3_ml1layer_*)
+ * run BF16 as such; the stand-alone GEMMs (gnnml3_gemm_nn / _tn) run it as single-pass TF32.  Any other value is
+ * GNNML3_ERR_INVALID. */
 #define GNNML3_PREC_3XTF32 0
 #define GNNML3_PREC_TF32 1
 #define GNNML3_PREC_BF16 2
-
-/* precision flags OR-ed into the `epilogue` argument of gnnml3_fused_agg_proj (tensor-memory kernel only): one tensor-core
- * product per k-step on TF32-truncated / BF16-rounded inputs instead of the FP32-grade 3xTF32 triple; FP32 accumulation.
- * Stated tolerances (tests/test_gpu_fused.py): TF32 2e-3, BF16 2e-2 of the result's scale. */
-#define GNNML3_FUSED_TF32 0x100
-#define GNNML3_FUSED_BF16 0x200
 
 /* epilogues of gnnml3_gemm_nn */
 #define GNNML3_EPI_NONE 0
@@ -167,7 +163,10 @@ GNNML3_API int gnnml3_ml3_act_bwd_y(const float* y, int64_t ldy, const float* au
  *                aux may be NULL (inference: nothing is saved for a backward): a forward-only kernel then stores out alone;
  *   self_mode 2: main[t, :] += S[t, :] Bself [Fs, Nc]  (SpectConv selfconn; gate gradients in the dx pass).
  * epilogue 0: out [N, Nc] = main.  X and S rows must be 16-byte aligned (ld % 4 == 0) and every column below
- * ceil4(F) / ceil4(Fs) must hold finite values.  3xTF32 arithmetic (FP32-grade).  Backward dx = the same call over the
+ * ceil4(F) / ceil4(Fs) must hold finite values.  precision (GNNML3_PREC_*): 3xTF32 is FP32-grade; TF32 and BF16 issue one
+ * tensor-core product per k-step on TF32-truncated / BF16-rounded inputs, with FP32 accumulation, and exist in the
+ * tensor-memory kernel only (gnnml3_fused_ts_supported shapes, aggregator mode 0).  Stated tolerances
+ * (tests/test_gpu_fused.py): TF32 2e-3, BF16 2e-2 of the result's scale.  Backward dx = the same call over the
  * transposed CSR with X = d pre, Bmain = W_k^T.  hout (nullable, [N, ldh]) receives a copy of the aggregate: support k in
  * columns [k * Fp, k * Fp + F) with Fp = 32 * ceil(F / 32) (zero padded), the self block S behind them at K * Fp (32 columns) --
  * the operand of the weight-gradient contraction x^T [S_0^T g .. S_{K-1}^T g | g1 g2], so the backward needs no separate SpMM.
@@ -187,7 +186,7 @@ GNNML3_API int gnnml3_fused_agg_proj(const int32_t* rowptr, const int32_t* col, 
                           int Kstride, int K, const float* X, int64_t ldx, int F, const float* S, int64_t lds,
                           int Fs, int self_mode, const float* Bmain, int64_t ldb, const float* Bself,
                           int64_t ldbs, int Ns, const float* bias, const float* bias_s, int64_t N, int Nc,
-                          float* out, int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue,
+                          float* out, int64_t ldo, float* aux, int64_t ldaux, int G, int epilogue, int precision,
                           float* hout, int64_t ldh, const int32_t* tilewin, void* workspace, size_t workspace_bytes,
                           void* stream);
 /* Second generation of the same kernel (fused_layer_ts.cu), taken automatically when the shape allows (F <= 32, even K):
@@ -261,10 +260,10 @@ GNNML3_API int gnnml3_ml3layer_backward(const int32_t* rowptr, const int32_t* co
  *   p0 = x wA^T + bA + (A x) wconv[0] + bconv,   p1 = x wB^T + bB,   p2 = x wC^T + bC
  *   concat = 0: y = relu(p0 + p1 * p2)                                                        [N, Fo]
  *   concat = 1: y = [relu(x wA^T + bA) | relu((A x) wconv[0] + bconv) | relu(p1 * p2)]         [N, 3 Fo]
- * One fused kernel per direction: the aggregate and the four projections meet in tensor memory (tcgen05, 3xTF32, FP32-grade).
- * The *_precision entry points take the same arguments plus the projection's arithmetic: GNNML3_PREC_3XTF32 (what the plain
- * entry points run), GNNML3_PREC_TF32 (one MMA per k-step on the raw FP32 operand, truncated by the tensor core, and RN-TF32
- * weights) or GNNML3_PREC_BF16 (RN-BF16 operands and weights); anything else is GNNML3_ERR_INVALID.  In every mode the
+ * One fused kernel per direction: the aggregate and the four projections meet in tensor memory (tcgen05).
+ * The trailing `precision` is the projection's arithmetic: GNNML3_PREC_3XTF32 (FP32-grade), GNNML3_PREC_TF32 (one MMA per
+ * k-step on the raw FP32 operand, truncated by the tensor core, and RN-TF32 weights) or GNNML3_PREC_BF16 (RN-BF16 operands
+ * and weights); anything else is GNNML3_ERR_INVALID.  In every mode the
  * aggregation (FP32 sums in CSR order), the epilogues, y / aux / dx (float32) and determinism are unchanged; the weight
  * gradient contraction runs at GNNML3_PREC_TF32 in both flagged modes.  Stated tolerances (tests/test_gpu_gnnml1_precision.py):
  * TF32 2e-3, BF16 2e-2 of the result's scale.
@@ -284,23 +283,12 @@ GNNML3_API int gnnml3_ml1layer_forward(const int32_t* rowptr, const int32_t* col
                             int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA, const float* wB,
                             const float* bB, const float* wC, const float* bC, int Fo, int concat, float* y, int64_t ldy,
                             float* aux, int64_t ldaux, float* hside, int64_t ldh, void* workspace, size_t workspace_bytes,
-                            void* stream);
+                            void* stream, int precision);
 GNNML3_API int gnnml3_ml1layer_backward(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x, int64_t ldx,
                              int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo, int concat,
                              const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy, int64_t ldgy,
                              int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA, float* dbA,
                              float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
-                             void* stream);
-GNNML3_API int gnnml3_ml1layer_forward_precision(const int32_t* rowptr, const int32_t* col, int64_t N, int64_t E, const float* x,
-                            int64_t ldx, int Fi, const float* wconv, const float* bconv, const float* wA, const float* bA,
-                            const float* wB, const float* bB, const float* wC, const float* bC, int Fo, int concat, float* y,
-                            int64_t ldy, float* aux, int64_t ldaux, float* hside, int64_t ldh, void* workspace,
-                            size_t workspace_bytes, void* stream, int precision);
-GNNML3_API int gnnml3_ml1layer_backward_precision(const int32_t* rowptrT, const int32_t* colT, int64_t N, int64_t E, const float* x,
-                             int64_t ldx, int Fi, const float* wconv, const float* wA, const float* wB, const float* wC, int Fo,
-                             int concat, const float* y, int64_t ldy, const float* aux, int64_t ldaux, const float* gy,
-                             int64_t ldgy, int need_dx, float* dx, int64_t lddx, float* dwconv, float* dbconv, float* dwA,
-                             float* dbA, float* dwB, float* dbB, float* dwC, float* dbC, void* workspace, size_t workspace_bytes,
                              void* stream, int precision);
 
 /* ---------------------------------------------------------------------------------------------------

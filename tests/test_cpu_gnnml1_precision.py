@@ -1,17 +1,21 @@
-"""GNNML1 precision modes on the CPU: an unknown precision is rejected before any device work, and the precision changes no
-parameter.  No GPU needed."""
+"""GNNML1 precision modes on the CPU: an unknown precision is rejected before any device work (by the GNNML3 modules too),
+and the precision changes no parameter.  No GPU needed."""
 import pytest
 import torch
 
 
 @pytest.mark.parametrize("bad", ["fp16", "FP32", "", None, 1])
 def test_bad_precision_is_rejected(bad):
-    from gnn_matlang_b200.libs.spect_conv import ML1Layer, ml1_layer
-    from gnn_matlang_b200.models import GNNML1
+    from gnn_matlang_b200.libs.spect_conv import ML1Layer, ML3Layer, ml1_layer
+    from gnn_matlang_b200.models import GNNML1, GNNML3
     with pytest.raises(ValueError, match="precision must be one of"):
         ML1Layer(8, 16, precision=bad)
     with pytest.raises(ValueError, match="precision must be one of"):
         GNNML1("zinc", 25, precision=bad)
+    with pytest.raises(ValueError, match="precision must be one of"):
+        ML3Layer(True, 4, 4, 8, 16, 2, precision=bad)
+    with pytest.raises(ValueError, match="precision must be one of"):
+        GNNML3("zinc", 4, 25, precision=bad)
     lay = ML1Layer(8, 16)
     # CPU tensors: the precision is checked before the device check (and before any library call)
     with pytest.raises(ValueError, match="precision must be one of"):

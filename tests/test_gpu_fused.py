@@ -342,6 +342,11 @@ def test_fused_flagged_precisions(N, deg, K, F, Nc, G, precision, rtol):
     assert ops.fused_path_counts()[0] == before[0] + 1
     # the flagged modes must really be reduced precision (a silent fall-through to 3xTF32 would sit at ~1e-7)
     assert float(err) > 1e-5, "suspiciously exact for %s: %.2e" % (precision, float(err))
+    # an unknown precision, and anything but 0 or 1 as the epilogue, is GNNML3_ERR_INVALID
+    with pytest.raises(RuntimeError, match=r"code 1\).*unknown precision"):
+        ops.fused_agg_proj(plan["rowptr"], plan["col"], None, ea_s, xa, W.view(K * F, Nc).to(d), epilogue=0, precision=3)
+    with pytest.raises(RuntimeError, match=r"code 1\).*unknown epilogue"):
+        ops.fused_agg_proj(plan["rowptr"], plan["col"], None, ea_s, xa, W.view(K * F, Nc).to(d), epilogue=0x101, precision=prec)
 
 
 @pytest.mark.parametrize("precision,rtol", [("tf32", 5e-3), ("bf16", 5e-2)])

@@ -1,6 +1,6 @@
 """GNNML1 in its reduced-precision modes on the B200: ``precision="tf32"`` (one tensor-core product per k-step on the raw FP32
 operand, truncated by the tensor core, against RN-TF32 weights) and ``precision="bf16"`` (RN-BF16 operands and weights, FP32
-accumulation) of the fused layer kernel (ml1_layer.cu), the C ABI's *_precision entry points, the composed path, the whole
+accumulation) of the fused layer kernel (ml1_layer.cu), the C ABI's precision argument, the composed path, the whole
 model, forward-only inference and the captured training step and evaluation pass.
 
 Bars, relative to the result's scale (test_gpu_kernels.assert_close: |a - ref| <= rtol |ref| + rtol max|ref|), the ones
@@ -260,7 +260,8 @@ def test_layer_is_deterministic(concat, precision):
 
 
 def _abi_args(plan, x, layer, concat):
-    """Arguments of gnnml3_ml1layer_forward / _backward (fresh outputs each call) for the layer's parameters."""
+    """Arguments of gnnml3_ml1layer_forward / _backward but the trailing precision (fresh outputs each call) for the layer's
+    parameters."""
     from gnn_matlang_b200 import _lib
     lib = _lib.load()
     N, Fi = x.shape
@@ -290,9 +291,8 @@ def _abi_bwd(plan, x, out, gy, concat, Fo):
 
 
 @pytest.mark.parametrize("concat", [False, True], ids=["sum", "concat"])
-def test_abi_precision_entry_points(concat):
-    """*_precision(..., GNNML3_PREC_3XTF32) is bit-identical to the plain entry points; an unknown precision is
-    GNNML3_ERR_INVALID (1) with a message, and writes nothing."""
+def test_abi_rejects_unknown_precision(concat):
+    """An unknown precision is GNNML3_ERR_INVALID (1) with a message, and writes nothing."""
     from gnn_matlang_b200 import _lib
     from gnn_matlang_b200.graph import get_plan
     lib = _lib.load()
@@ -302,24 +302,12 @@ def test_abi_precision_entry_points(concat):
     layer = _layer(Fi, Fo, concat, "fp32", seed=6)
     plan = get_plan(ei, N)
     gy = torch.randn(N, 3 * Fo if concat else Fo, generator=torch.Generator().manual_seed(8)).to(dev())
-    res = {}
-    for name in ("plain", "precision"):
-        out, fwd = _abi_args(plan, x, layer, concat)
-        rc = lib.gnnml3_ml1layer_forward(*fwd) if name == "plain" else lib.gnnml3_ml1layer_forward_precision(*fwd, _lib.PREC_3XTF32)
-        assert rc == 0
-        g, bwd = _abi_bwd(plan, x, out, gy, concat, Fo)
-        rc = lib.gnnml3_ml1layer_backward(*bwd) if name == "plain" else lib.gnnml3_ml1layer_backward_precision(*bwd, _lib.PREC_3XTF32)
-        assert rc == 0
-        torch.cuda.synchronize()
-        res[name] = [out["y"], out["aux"]] + [g[k] for k in ("dx", "dwc", "dwA", "dwB", "dwC", "dbs")]
-    for a, b in zip(res["plain"], res["precision"]):
-        assert torch.equal(a, b)
     for bad in (3, -1, 0x100):
         out, fwd = _abi_args(plan, x, layer, concat)
-        assert lib.gnnml3_ml1layer_forward_precision(*fwd, bad) == 1
+        assert lib.gnnml3_ml1layer_forward(*fwd, bad) == 1
         assert b"precision" in lib.gnnml3_last_error()
         g, bwd = _abi_bwd(plan, x, out, gy, concat, Fo)
-        assert lib.gnnml3_ml1layer_backward_precision(*bwd, bad) == 1
+        assert lib.gnnml3_ml1layer_backward(*bwd, bad) == 1
         assert b"precision" in lib.gnnml3_last_error()
         torch.cuda.synchronize()
         assert float(out["y"].abs().max()) == 0.0 and float(g["dx"].abs().max()) == 0.0

@@ -173,6 +173,11 @@ def test_gemm_nn(M, Kc, Nc):
     assert torch.equal(out_relu, out.clamp(min=0))
     out_fast = ops.gemm_nn(A.to(dev()), B.to(dev()), None, precision=_lib.PREC_TF32)
     assert_close(out_fast, A.double() @ B.double(), rtol=2e-3, name="gemm_nn TF32")      # 10-bit mantissa mode
+    # the C GEMM runs GNNML3_PREC_BF16 as single-pass TF32
+    Ad, Bd, out_bf16 = A.to(dev()), B.to(dev()), torch.empty(M, Nc, device=dev())
+    _lib.check(_lib.load().gnnml3_gemm_nn(Ad.data_ptr(), Kc, Bd.data_ptr(), Nc, None, out_bf16.data_ptr(), Nc, M, Nc, Kc,
+                                          _lib.PREC_BF16, _lib.EPI_NONE, _lib.stream_ptr()), "gnnml3_gemm_nn")
+    assert torch.equal(out_bf16, out_fast)
 
 
 @pytest.mark.parametrize("M,Ka,Nb", [(1, 1, 1), (7, 3, 5), (1000, 25, 240), (5000, 64, 640), (333, 130, 70), (100000, 32, 30),
@@ -182,13 +187,20 @@ def test_gemm_nn(M, Kc, Nc):
                                      (30000, 32, 320), (12000, 16, 384), (9000, 8, 260),  # tcgen05 path (last three: several 256-column launches)
                                      (20000, 64, 640), (10000, 100, 300), (9000, 130, 70)])  # wide A: 32-column blocks of A x 256-column blocks of B
 def test_gemm_tn_and_colsum(M, Ka, Nb):
-    from gnn_matlang_b200 import ops
+    from gnn_matlang_b200 import ops, _lib
     g = torch.Generator().manual_seed(M + Ka + Nb)
     A = torch.randn(M, Ka, generator=g)
     B = torch.randn(M, Nb, generator=g)
     out = ops.gemm_tn(A.to(dev()), B.to(dev()))
     assert_close(out, A.double().t() @ B.double(), name="gemm_tn")
     assert torch.equal(out, ops.gemm_tn(A.to(dev()), B.to(dev())))              # deterministic
+    # the C GEMM runs GNNML3_PREC_BF16 as single-pass TF32
+    lib = _lib.load()
+    Ad, Bd, out_bf16 = A.to(dev()), B.to(dev()), torch.empty(Ka, Nb, device=dev())
+    ws = torch.empty(lib.gnnml3_gemm_tn_workspace_bytes(M, Ka, Nb), dtype=torch.uint8, device=dev())
+    _lib.check(lib.gnnml3_gemm_tn(Ad.data_ptr(), Ka, Bd.data_ptr(), Nb, out_bf16.data_ptr(), Nb, M, Ka, Nb, _lib.PREC_BF16,
+                                  ws.data_ptr(), ws.numel(), _lib.stream_ptr()), "gnnml3_gemm_tn")
+    assert torch.equal(out_bf16, ops.gemm_tn(Ad, Bd, precision=_lib.PREC_TF32))
     assert_close(ops.colsum(B.to(dev())), B.double().sum(0), name="colsum")
 
 
