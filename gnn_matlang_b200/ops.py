@@ -378,8 +378,12 @@ def fused_supported(K, Kstride, F, Nc, Fs=0, self_mode=0, Ns=0):
 
 
 def fused_ts_supported(K, Kstride, F, Nc, Fs=0, self_mode=0, Ns=0):
-    """Shape covered by the tensor-memory generation of the fused kernel (the only one with the TF32 / BF16 modes)."""
-    return bool(_lib.load().gnnml3_fused_ts_supported(int(K), int(Kstride), int(F), int(Nc), int(Fs), int(self_mode), int(Ns)))
+    """gnnml3_fused_agg_proj runs the tensor-memory generation of the fused kernel (the only one with the TF32 / BF16 modes)
+    for this shape: the shape is covered (gnnml3_fused_ts_supported) and the aggregator mode is the default one -- the slot
+    mode (gnnml3_fused_set_mode(1)) always runs the shared-memory-plane kernel."""
+    lib = _lib.load()
+    return bool(lib.gnnml3_fused_ts_supported(int(K), int(Kstride), int(F), int(Nc), int(Fs), int(self_mode), int(Ns))
+                and lib.gnnml3_fused_set_mode(-1) == 0)
 
 
 def fused_agg_proj(rowptr, col, eperm, ea, x, Bmain, bias=None, S=None, self_mode=0, Bself=None, bias_s=None, G=0,
