@@ -86,6 +86,10 @@ SIGNATURES = {
     "gnnml3_segment_pool_bwd": (_i, [_p, _p, _i, _i, _i, _p, _i64, _p]),
     "gnnml3_segment_max_fwd": (_i, [_p, _i64, _p, _i, _i, _p, _p, _p]),
     "gnnml3_segment_max_bwd": (_i, [_p, _p, _p, _i, _i, _p, _i64, _p]),
+    "gnnml3_bn_rows_workspace_bytes": (_sz, [_i64, _i]),
+    "gnnml3_bn_rows_fwd": (_i, [_p, _i64, _i64, _i, _p, _p, _p, ctypes.c_double, ctypes.c_double, _p, _p, _p, _p, _i64, _p, _p, _p,
+                                _sz, _p]),
+    "gnnml3_bn_rows_bwd": (_i, [_p, _i64, _p, _i64, _i64, _i, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _sz, _p]),
     "gnnml3_spectral_max_nodes": (_i, [_i]),
     "gnnml3_spectral_count": (_i, [_p, _i64, _p, _p, _i, _i, _i, _p, _p]),
     "gnnml3_spectral_design": (_i, [_p, _i64, _p, _p, _i, _i, ctypes.c_double, _i, _i, _i, _i, ctypes.c_double, _i, _p, _i, _p,

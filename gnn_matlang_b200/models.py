@@ -18,6 +18,9 @@ concatenated read-outs, log-softmax heads:
 
 The same (unlearned) ``edge_attr2`` feeds every layer; the graph plan (CSR) is built once per batch.  BatchNorm, dropout and
 log-softmax are torch modules (statistics / elementwise work on [N, F] and [B, F], outside the hot path of SURVEY.md 8a).
+On a padded batch in training mode (``train.pad_batch``, ``real_graphs < num_graphs``) the BatchNorm statistics leave the dummy
+graph out: ``bn="layers"`` runs the node BatchNorm kernels of ``norm.batch_norm_rows`` over the first ``graph_ptr[real_graphs]``
+rows, ``bn="readout"`` applies the module to the first ``real_graphs`` pooled rows and passes the dummy row through.
 
 ``GNNML1`` is the paper's 1-WL model, defined next to GNNML3 in every experiment script of the reference: ``nlayer`` GNNML1
 layers (``libs.spect_conv.ML1Layer``) on the graph's plain ``edge_index``, then the pool and head of the same-named GNNML3
@@ -29,6 +32,7 @@ import torch.nn as nn
 from .libs.spect_conv import ML3Layer, SpectConv, _LinearFn, _precision_code, ml1_layer
 import torch.nn.functional as F
 
+from .norm import batch_norm_rows
 from .pool import global_add_pool, global_max_pool, global_mean_pool
 
 MODEL_CONFIGS = {
@@ -73,18 +77,24 @@ class GNNML3(nn.Module):
         edge_index = data.edge_index2
         edge_attr = data.edge_attr2
         c = self.cfg
+        B = getattr(data, "num_graphs", None)
+        # a padded batch (train.pad_batch: one dummy graph behind the real ones) in training mode: BatchNorm statistics over the
+        # real rows only, so that the captured step trains the model the eager step trains on the same graphs
+        real = getattr(data, "real_graphs", None)
+        padded = self.training and c.get("bn") is not None and real is not None and B is not None and real < B
         for l in range(c["nlayer"]):
             if c.get("dropout"):
                 x = F.dropout(x, p=c["dropout"], training=self.training)
             x = getattr(self, "conv%d" % (l + 1))(x, edge_index, edge_attr)
             if c.get("bn") == "layers":
-                x = getattr(self, "bn%d" % (l + 1))(x)
-        B = getattr(data, "num_graphs", None)
+                bn = getattr(self, "bn%d" % (l + 1))
+                x = batch_norm_rows(x, data.graph_ptr[real:real + 1], bn) if padded else bn(x)
         pools = {"add": global_add_pool, "mean": global_mean_pool, "max": global_max_pool}
         if c["pool"] != "none":                          # "none": node-level output (filtering.py:281)
             x = torch.cat([pools[k](x, data.batch, B) for k in c["pool"].split("_")], 1)
         if c.get("bn") == "readout":
-            x = getattr(self, "bn%d" % c["nlayer"])(x)
+            bn = getattr(self, "bn%d" % c["nlayer"])
+            x = torch.cat([bn(x[:real]), x[real:]], 0) if padded else bn(x)
         prec = _precision_code(self.precision)
         if len(c["head"]) == 1:
             fc = self.fc2 if c.get("fc_name") == "fc2" else self.fc1

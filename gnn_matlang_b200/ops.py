@@ -738,6 +738,55 @@ def segment_max_bwd(gout, arg, graph_ptr, N):
     return gx
 
 
+def _bn_cnt(cnt, device):
+    if cnt.dtype != torch.int32 or cnt.numel() != 1 or cnt.device != device:
+        raise RuntimeError("cnt must be a one-element int32 tensor on %s" % device)
+    return cnt
+
+
+def bn_rows_fwd(x, cnt, weight, bias, running_mean, running_var, num_batches_tracked, eps, momentum):
+    """Training-mode BatchNorm over the first ``cnt`` rows of x [N, F] (``cnt``: one-element int32 CUDA tensor, read on the
+    device); running buffers updated in place.  -> (y [N, F], save_mean [F], save_invstd [F])."""
+    lib = _lib.load()
+    x = _rows(x, "x")
+    N, F = x.shape
+    cnt = _bn_cnt(cnt, x.device)
+    for t, name in ((weight, "weight"), (bias, "bias"), (running_mean, "running_mean"), (running_var, "running_var")):
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != F or t.device != x.device:
+            raise RuntimeError("%s must be a contiguous float32 [%d] tensor on %s" % (name, F, x.device))
+    if num_batches_tracked.dtype != torch.int64 or num_batches_tracked.numel() != 1 or num_batches_tracked.device != x.device:
+        raise RuntimeError("num_batches_tracked must be a one-element int64 tensor on %s" % x.device)
+    y = torch.empty(N, F, dtype=torch.float32, device=x.device)
+    mean = torch.empty(F, dtype=torch.float32, device=x.device)
+    invstd = torch.empty(F, dtype=torch.float32, device=x.device)
+    with _on(x.device):
+        nb = lib.gnnml3_bn_rows_workspace_bytes(N, F)
+        ws = _ws(x.device, nb, "bn")
+        _lib.check(lib.gnnml3_bn_rows_fwd(_lib.ptr(x), _ld(x), N, F, _lib.ptr(cnt), _lib.ptr(weight), _lib.ptr(bias), float(eps),
+                                          float(momentum), _lib.ptr(running_mean), _lib.ptr(running_var),
+                                          _lib.ptr(num_batches_tracked), _lib.ptr(y), F, _lib.ptr(mean), _lib.ptr(invstd),
+                                          _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "gnnml3_bn_rows_fwd")
+    return y, mean, invstd
+
+
+def bn_rows_bwd(x, gy, cnt, weight, save_mean, save_invstd):
+    """Backward of ``bn_rows_fwd``: -> (dx [N, F] with zero rows from ``cnt`` on, dweight [F], dbias [F])."""
+    lib = _lib.load()
+    x, gy = _rows(x, "x"), _rows(gy, "gy")
+    N, F = x.shape
+    cnt = _bn_cnt(cnt, x.device)
+    dx = torch.empty(N, F, dtype=torch.float32, device=x.device)
+    dw = torch.empty(F, dtype=torch.float32, device=x.device)
+    db = torch.empty(F, dtype=torch.float32, device=x.device)
+    with _on(x.device):
+        nb = lib.gnnml3_bn_rows_workspace_bytes(N, F)
+        ws = _ws(x.device, nb, "bn")
+        _lib.check(lib.gnnml3_bn_rows_bwd(_lib.ptr(x), _ld(x), _lib.ptr(gy), _ld(gy), N, F, _lib.ptr(cnt), _lib.ptr(weight),
+                                          _lib.ptr(save_mean), _lib.ptr(save_invstd), _lib.ptr(dx), F, _lib.ptr(dw), _lib.ptr(db),
+                                          _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "gnnml3_bn_rows_bwd")
+    return dx, dw, db
+
+
 def pairs_mark(emb, bits, wpr, threshold, pairs=None):
     """OR one seed's embeddings emb [n, d] (float32 CUDA, unit-stride rows) into the pair bitmap ``bits`` (int32 words read as
     uint32): all pairs i < j (``pairs`` None, ``wpr`` words per row) or the listed pairs ``pairs`` [P, 2] int64."""
@@ -797,5 +846,5 @@ def _instrument(name, fn):
 
 for _n in ("csr_build", "gather_rows", "scatter_rows", "spmm_k", "spmm_projected", "sddmm_k", "gemm_nn_tc", "gemm_nn", "gemm_tn", "colsum", "edge_mlp_fwd",
            "edge_mlp_bwd", "ml3_act_fwd", "ml3_act_bwd", "ml3_act_bwd_y", "fused_agg_proj", "fused_sddmm", "ml3layer_forward", "ml3layer_backward", "segment_pool_fwd",
-           "segment_pool_bwd"):
+           "segment_pool_bwd", "bn_rows_fwd", "bn_rows_bwd"):
     globals()[_n] = _instrument(_n, globals()[_n])

@@ -87,6 +87,54 @@ def sweep_graph(rng, nfeat):
     return n, ei, rng.standard_normal((n, nfeat)).astype(np.float32)
 
 
+def _local_graph(rng, n, extra, window):
+    """Connected graph of n nodes: a random tree whose edges join nodes at most ``window`` apart, plus ``extra`` distinct chords
+    of the same reach (molecule / protein-contact like, no hubs)."""
+    have = set()
+    for v in range(1, n):
+        have.add((int(rng.integers(max(0, v - window), v)), v))
+    for _ in range(extra):
+        u = int(rng.integers(0, n))
+        v = int(min(n - 1, u + rng.integers(2, window + 1)))
+        if u < v:
+            have.add((u, v))
+    if not have:
+        return np.zeros((2, 0), np.int64)
+    u, v = (np.array(a, dtype=np.int64) for a in zip(*sorted(have)))
+    return _sym_sorted(u, v)
+
+
+def tu_records(kind, count, seed=0):
+    """Reader-shaped records (``datasets.read_mat``: ``dict(x, edge_index, y)``) of synthetic graphs shaped like two TU datasets
+    the ``enzymes`` / ``mutag`` presets train on (their ``.mat`` files are not part of this repository):
+
+    * ``enzymes`` -- n ~ Gamma(4.5, 7.3) clipped to [2, 126] (ENZYMES: 2-126 nodes, mean ~33), every 50th graph 120-126 nodes
+                     (beyond the one-block eigensolver's envelope), ~1.9 edges per node; x = one-hot of 3 node labels (the three
+                     feature columns ``read_mat`` keeps); y = int64 [1] class in 0..5, a function of the dominant node label and
+                     the size (learnable, so that a short training run shows a falling loss)
+    * ``mutag``   -- n ~ N(18, 4.6) clipped to [10, 28], tree plus 1-3 ring chords; x = one-hot of 7 atom types; y = float32 [1]
+                     in {0, 1} (whether the graph holds at least two atoms of type 1)"""
+    rng = np.random.default_rng(seed)
+    out = []
+    for i in range(count):
+        if kind == "enzymes":
+            n = int(rng.integers(120, 127)) if i % 50 == 49 else int(np.clip(round(rng.gamma(4.5, 7.3)), 2, 126))
+            ei = _local_graph(rng, n, int(round(0.9 * n)), 6)
+            lab = rng.choice(3, size=n, p=rng.dirichlet([1.0, 1.0, 1.0]))
+            x = np.eye(3, dtype=np.float32)[lab]
+            y = np.array([(int(np.bincount(lab, minlength=3).argmax()) * 2 + int(n > 30)) % 6], np.int64)
+        elif kind == "mutag":
+            n = int(np.clip(round(rng.normal(18.0, 4.6)), 10, 28))
+            ei = _local_graph(rng, n, int(rng.integers(1, 4)), 4)
+            lab = rng.choice(7, size=n, p=[0.7, 0.1, 0.1, 0.04, 0.03, 0.02, 0.01])
+            x = np.eye(7, dtype=np.float32)[lab]
+            y = np.array([float((lab == 1).sum() >= 2)], np.float32)
+        else:
+            raise ValueError("tu_records: kind must be 'enzymes' or 'mutag', got %r" % (kind,))
+        out.append(dict(x=x, edge_index=ei, y=y))
+    return out
+
+
 def mask_edges(n, ei, recfield):
     """Row-major coordinates of the receptive-field mask (libs/utils.py:566-573, :608): recfield 0 -> A,
     r >= 1 -> (A + I)^(2^(r-1)) > 0."""
@@ -345,6 +393,72 @@ class DeviceDataset(object):
         ys = [torch.as_tensor(get(g, "y")) for g in records]         # batch.collate's label layout: one row per graph
         self.y = t(torch.cat([y.reshape(1, -1) if y.dim() < 2 else y for y in ys], 0))
         self.e_h = self.e = self.e32 = self.edge_off = self.el = self.ea = None
+        return self
+
+    @classmethod
+    def from_records(cls, records, sd, device):
+        """Resident GNNML3 dataset straight from reader records ``dict(x [n, F], edge_index [2, m] graph-local, y)`` (what
+        ``datasets.read_mat``, ``read_graph6`` and ``read_exp_pickle`` return): the supports of ``sd`` (a ``SpectralDesign``) are
+        designed on the device -- every graph within ``sd.max_kernel_nodes()`` in ONE ``design_batch`` launch, larger ones one by
+        one on the dense path, as ``design_list`` routes them -- ``x`` gets the degree column when ``sd.adddegree`` is set, and
+        features, supports and labels stay resident.  Batches carry ``x``, ``edge_index2``, ``edge_attr2``, ``batch``,
+        ``graph_ptr`` and ``y`` as per-record ``sd(data)`` + ``batch.collate`` give them."""
+        def get(g, k):
+            return g.get(k) if isinstance(g, dict) else getattr(g, k, None)
+        if len(records) == 0:
+            raise ValueError("DeviceDataset.from_records: no records")
+        xs = [np.asarray(get(g, "x"), dtype=np.float32).reshape(np.shape(get(g, "x"))[0], -1) for g in records]
+        if len({x.shape[1] for x in xs}) != 1:
+            raise ValueError("DeviceDataset.from_records: the records' x differ in width")
+        eis = [np.asarray(get(g, "edge_index"), dtype=np.int64).reshape(2, -1) for g in records]
+        n_h = np.array([x.shape[0] for x in xs], dtype=np.int64)
+        for ei, n in zip(eis, n_h):
+            if ei.size and (ei.min() < 0 or ei.max() >= n):
+                raise ValueError("DeviceDataset.from_records: edge_index holds ids outside its graph")
+        if any(get(g, "y") is None for g in records):
+            raise ValueError("DeviceDataset.from_records: every record needs a label y")
+        limit = sd.max_kernel_nodes()
+        small = np.flatnonzero(n_h <= limit)
+        large = np.flatnonzero(n_h > limit)
+        # per-record blocks laid out as [all kernel-designed graphs | the large graphs one by one]; the collation reads every
+        # record through its own node / entry offset, so the layout need not follow record order
+        order = np.concatenate([small, large])
+        els, eas, degs, counts = [], [], [], np.zeros(len(records), dtype=np.int64)
+        if len(small):
+            ns, ms = n_h[small], np.array([eis[i].shape[1] for i in small], dtype=np.int64)
+            ei = np.concatenate([eis[i] for i in small], 1)
+            out = sd.design_batch(torch.from_numpy(ei).to(device), torch.from_numpy(np.concatenate([[0], np.cumsum(ms)])).to(device),
+                                  torch.from_numpy(np.concatenate([[0], np.cumsum(ns)])), device=device)
+            els.append(out["edge_index2"])
+            eas.append(out["edge_attr2"])
+            degs.append(out["degree"])
+            counts[small] = out["counts"].cpu().numpy()
+        for i in large:
+            o = sd._design_large(eis[i], int(n_h[i]), device=device)
+            els.append(o["edge_index2"])
+            eas.append(o["edge_attr2"])
+            degs.append(o["degree"])
+            counts[i] = o["edge_index2"].size(1)
+        self = cls.__new__(cls)
+        self.device = device
+        self.n_h, self.e_h = n_h, counts
+        node_off, edge_off = np.zeros(len(records) + 1, dtype=np.int64), np.zeros(len(records) + 1, dtype=np.int64)
+        node_off[order] = np.concatenate([[0], np.cumsum(n_h[order])])[:-1]
+        edge_off[order] = np.concatenate([[0], np.cumsum(counts[order])])[:-1]
+        node_off[-1], edge_off[-1] = n_h.sum(), counts.sum()
+        t = lambda a: torch.as_tensor(a).to(device)
+        self.n, self.e = t(n_h), t(counts)
+        self.n32, self.e32 = self.n.to(torch.int32), self.e.to(torch.int32)
+        self.node_off, self.edge_off = t(node_off), t(edge_off)
+        x = t(np.concatenate([xs[i] for i in order], 0))
+        if sd.adddegree:
+            x = torch.cat([x, torch.cat(degs).unsqueeze(-1)], 1)
+        self.x = x.contiguous()
+        self.el = torch.cat(els, 1).contiguous()
+        self.ea = torch.cat(eas, 0).contiguous()
+        ys = [torch.as_tensor(get(g, "y")) for g in records]         # batch.collate's label layout: one row per graph
+        self.y = t(torch.cat([y.reshape(1, -1) if y.dim() < 2 else y for y in ys], 0))
+        self.m_h = self.m32 = self.adj_off = self.al = None
         return self
 
     @classmethod

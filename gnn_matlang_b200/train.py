@@ -11,6 +11,17 @@ import torch.distributed as dist
 import torch.nn.functional as F
 
 
+LOSSES = ("l1", "mse", "bce", "nll")
+
+
+def class_labels(out, y):
+    """Class ids of a ``log_softmax`` head: integer labels with one per row of out [B, C] (``read_mat``'s int64 [B, 1]) -> [B]."""
+    if y.dtype.is_floating_point or y.dtype == torch.bool or y.numel() != out.size(0):
+        raise ValueError("nll: labels must be integer class ids, one per graph (got %s of %d elements for %d graphs)"
+                         % (y.dtype, y.numel(), out.size(0)))
+    return y.reshape(-1).long()
+
+
 def loss_fn(kind, out, y):
     if kind == "l1":                                   # Zinc12k.py:365
         return F.l1_loss(out, y.to(out.dtype).reshape(out.shape), reduction="sum")
@@ -18,6 +29,11 @@ def loss_fn(kind, out, y):
         return torch.square(out - y.to(out.dtype).reshape(out.shape)).sum()
     if kind == "bce":                                  # exp_classify.py:327-329
         return F.binary_cross_entropy(torch.sigmoid(out), y.to(out.dtype).reshape(out.shape), reduction="sum")
+    if kind == "nll":
+        # -sum_b log p[b, y_b] over the log-probabilities of a log_softmax head (the enzymes preset).  SUM, like every loss
+        # here, so that the data-parallel all-reduce stays a SUM; the reduction of the reference's TU scripts is not restated,
+        # their training loops are not part of this repository.
+        return F.nll_loss(out, class_labels(out, y), reduction="sum")
     raise ValueError(kind)
 
 
@@ -42,6 +58,8 @@ def shard_graphs(sizes, world, rank=None):
 
 class Trainer(object):
     def __init__(self, model, loss="l1", lr=1e-3, distributed=False):
+        if loss not in LOSSES:
+            raise ValueError("Trainer: loss must be one of %s, got %r" % (LOSSES, loss))
         self.model = model
         self.loss_kind = loss
         self.distributed = distributed and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
@@ -272,6 +290,8 @@ class GraphedTrainer(object):
 
     def __init__(self, model, example, loss="l1", lr=1e-3, distributed=False, warmup=3):
         from .graph import set_range_check
+        if loss not in LOSSES:
+            raise ValueError("GraphedTrainer: loss must be one of %s, got %r" % (LOSSES, loss))
         set_range_check(False)                         # the range check reads a flag back from the device
         self.model, self.loss_kind = model, loss
         self.distributed = distributed and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
@@ -411,13 +431,17 @@ class GraphedTrainer(object):
         return self.static_loss
 
 
-EVAL_METRICS = ("l1", "mse", "bce", None)
+EVAL_METRICS = ("l1", "mse", "bce", "nll", None)
 
 
 def eval_terms(metric, out, y):
     """Per-graph terms of ``loss_fn(metric, out, y)`` (its SUM over graphs is the loss): out [B, d], labels y (any shape with
-    B * d elements) -> (term [B], correct [B] or None).  ``correct`` = [(o > 0) == (y > 0.5)] for a single-output "bce" head (the
-    accuracy of exp_classify.py's test loop); None for the other metrics and for wider heads."""
+    B * d elements; for "nll" B integer class ids) -> (term [B], correct [B] or None).  ``correct`` = [(o > 0) == (y > 0.5)] for a
+    single-output "bce" head (the accuracy of exp_classify.py's test loop), [argmax o == y] for "nll"; None for the other metrics
+    and for wider "bce" heads."""
+    if metric == "nll":
+        c = class_labels(out, y)
+        return -out.gather(1, c.unsqueeze(1))[:, 0], (out.argmax(1) == c).to(out.dtype)
     y = y.to(out.dtype).reshape(out.shape)
     if metric == "l1":
         return (out - y).abs().sum(1), None
@@ -466,7 +490,7 @@ class GraphedEvaluator(object):
     for a backward) and the metric accumulated on the device in float64.
 
         ev = GraphedEvaluator(model, dataset, ids, batch_size, metric="l1")
-        res = ev.run()                  # {"graphs": n, "sum": s, "mean": s / n} (+ "correct", "accuracy" for "bce")
+        res = ev.run()                  # {"graphs": n, "sum": s, "mean": s / n} (+ "correct", "accuracy" for "bce", "nll")
         res = ev.run(outputs=True)      # also res["outputs"]: [len(ids), out] device tensor in id order
 
     Batches are consecutive chunks of ``ids`` (``eval_chunks``); a short last chunk is filled with copies of the split's smallest
@@ -475,7 +499,7 @@ class GraphedEvaluator(object):
     no dropout) during warm-up and capture; its previous mode is restored afterwards.  The graph reads parameters and buffers in
     place: a trainer stepping the same model between two ``run()`` calls is seen by the second.  ``run()`` reads the device once,
     at the end.  ``distributed=True``: every rank passes its own ids and ``run()`` SUM-all-reduces the metric once (outputs stay per
-    rank).  ``metric``: "l1", "mse", "bce" (the per-graph terms of ``loss_fn``) or None (outputs only)."""
+    rank).  ``metric``: "l1", "mse", "bce", "nll" (the per-graph terms of ``loss_fn``) or None (outputs only)."""
 
     def __init__(self, model, dataset, ids, batch_size, metric="l1", max_pad_degree=8, distributed=False, warmup=2):
         import numpy as np
@@ -483,6 +507,9 @@ class GraphedEvaluator(object):
         from .graph import set_range_check
         if metric not in EVAL_METRICS:
             raise ValueError("GraphedEvaluator: metric must be one of %s, got %r" % (EVAL_METRICS, metric))
+        if metric == "nll" and getattr(model, "cfg", {}).get("final") != "log_softmax":
+            # the term -log p[y] and the argmax accuracy are those of log-probabilities
+            raise ValueError("GraphedEvaluator: metric 'nll' needs a model with a log_softmax head (cfg['final'])")
         ids = np.asarray(ids, dtype=np.int64).reshape(-1)
         if len(ids) == 0:
             raise ValueError("GraphedEvaluator: ids is empty")
@@ -563,7 +590,7 @@ class GraphedEvaluator(object):
         if self.metric is not None:
             res["sum"] = vals[0]
             res["mean"] = vals[0] / max(res["graphs"], 1)
-            if self.metric == "bce" and self.static_out.size(1) == 1:
+            if (self.metric == "bce" and self.static_out.size(1) == 1) or self.metric == "nll":
                 res["correct"] = int(round(vals[1]))
                 res["accuracy"] = vals[1] / max(res["graphs"], 1)
         if outputs:

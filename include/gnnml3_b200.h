@@ -307,6 +307,28 @@ GNNML3_API int gnnml3_segment_max_bwd(const float* gout, const int32_t* arg, con
                            int64_t ldx, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
+ * Node BatchNorm of a padded batch (batchnorm.cu; mutag.py:283-285): training-mode nn.BatchNorm1d over the first *cnt rows of
+ * x [N, F] (row stride ldx), *cnt read on the device (int32, clamped to [0, N]) -- graph_ptr[real_graphs] of a padded batch, so
+ * a captured step replays with the node count of every new batch.
+ *   fwd: y = (x - mean) invstd weight + bias on EVERY row, mean / biased variance over rows < cnt only (rows >= cnt, NaN or
+ *        inf included, reach no statistic and no real row); save_mean / save_invstd [F] for the backward; running_mean /
+ *        running_var = (1 - momentum) old + momentum new with the unbiased variance; *num_batches_tracked += 1.
+ *        cnt = 1: the output is the bias and running_var is left unchanged (nn.BatchNorm1d refuses one row); cnt = 0: the
+ *        running buffers are left unchanged.
+ *   bwd: dx (rows >= cnt get 0), dweight, dbias [F] summed over rows < cnt, from the forward's x and saved statistics.
+ * Two launches per direction, FP64 partial sums in a fixed order (no atomics, bit-identical reruns), workspace of
+ * gnnml3_bn_rows_workspace_bytes(N, F) used by both directions (N >= 1, F >= 1).  No host sync; CUDA-graph capturable.
+ * --------------------------------------------------------------------------------------------------- */
+GNNML3_API size_t gnnml3_bn_rows_workspace_bytes(int64_t N, int F);
+GNNML3_API int gnnml3_bn_rows_fwd(const float* x, int64_t ldx, int64_t N, int F, const int32_t* cnt, const float* weight,
+                                  const float* bias, double eps, double momentum, float* running_mean, float* running_var,
+                                  int64_t* num_batches_tracked, float* y, int64_t ldy, float* save_mean, float* save_invstd,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+GNNML3_API int gnnml3_bn_rows_bwd(const float* x, int64_t ldx, const float* gy, int64_t ldgy, int64_t N, int F, const int32_t* cnt,
+                                  const float* weight, const float* save_mean, const float* save_invstd, float* dx, int64_t lddx,
+                                  float* dweight, float* dbias, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------
  * SpectralDesign (libs/utils.py:525-610), batched: one thread block per graph, FP64 Jacobi eigensolver.
  * Input graphs are given as concatenated LOCAL edge lists: edge_index [2, Etot] int64 (row 0 = src, row 1 = dst,
  * node ids local to their graph), edge_ptr [B+1], node_ptr [B+1] (int32).  nmax = largest node count.
